@@ -23,6 +23,8 @@ headline line is quoted on (default 3 = configs[2], the one the metric names); t
   stream_object the drop-in ParamBase object (MfccCuda) on 10 s files: one handle, and several handles from host threads
 
 `--impl reference` times that CPU path alone (no CUDA) and prints the same line with "impl": "reference".
+`--dump-outputs DIR` writes the features of the last timed step (a fixed sample of utterances) to DIR/features.npy, so that
+two builds can be compared output for output on identical inputs.
 torch is used for device memory, streams, events and torch.distributed only; all compute is libafe_cuda.so.
 """
 import argparse
@@ -200,6 +202,12 @@ def cpu_arm(n_utts, steps, warmup, threads, pcm=None, g=CFG16):
                        f"fresh MfccCpu per utterance sized to it (Q3/Q5), FFT = oracle/fftw_shim.c (FFTW not installed)")
 
 
+def cpu_arm_threads(ol):
+    """Cores the CPU arm runs on, which its sample is sized for: every host core for the reference's build, one for the C port
+    (single-threaded), which stands in when oracle/_ref was not built."""
+    return (os.cpu_count() or 1) if ol.available("ref") else 1
+
+
 def cpu_denominators(p, sample):
     return {"fft_shim_us_per_512pt": shim_us_per_transform(512), "fft_shim_us_per_256pt": shim_us_per_transform(256),
             "stage_split_1core": cpu_stage_split(p, sample)}
@@ -209,8 +217,8 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    threads = os.cpu_count() or 1
     import oracle_lib as ol
+    threads = cpu_arm_threads(ol)
     lib = ol.RefLib("ref" if ol.available("ref") else "port")
     cal = synth_host(8, 99)
     _, s = lib.extract(params_dict(), [cal[i] for i in range(8)], sample_limit=0, n_threads=1)
@@ -336,6 +344,22 @@ def leg_config3(cx, args, pcm, out, offs, lens, n_utts):
                launches=launches, t_begin=t_begin, t_end=t_end, tiles=b.num_tiles, kernel=b.kernel_name)
     b.close()
     return res
+
+
+DUMP_UTTS = 256     # 256 utterances x 998 frames x 39 x 4 B = 39.9 MB, under the 64 MB a dump may take
+
+
+def dump_outputs(dirname, out, n_utts, T):
+    """--dump-outputs: the rows the last timed step wrote for a fixed sample of whole utterances (seed 0, ascending utterance
+    index) -> DIR/features.npy, float32 [k, T, 39]. The PCM is generated from fixed seeds, so the same arguments give the
+    same inputs on every run."""
+    import torch
+    k = min(DUMP_UTTS, n_utts)
+    pick = np.sort(np.random.default_rng(0).choice(n_utts, k, replace=False))
+    feats = out.view(n_utts, T, WIDTH)[torch.from_numpy(pick).to(out.device)].cpu().numpy()
+    assert feats.dtype == np.float32 and feats.nbytes <= 64 << 20
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, "features.npy"), feats)
 
 
 def parity_gate(cx, pcm, out, n_utts, g=CFG16, n_check=64):
@@ -695,10 +719,14 @@ def run_b200(args):
         offs = np.arange(n_utts, dtype=np.int64) * n
         lens = np.full(n_utts, n, np.int64)
         r3 = leg_config3(cx, args, pcm, out, offs, lens, n_utts)
+        if args.dump_outputs and cx.rank == 0:
+            dump_outputs(args.dump_outputs, out, n_utts, T)      # before the corpus leg reuses `out`
         parity = parity_gate(cx, pcm, out, n_utts) if cx.rank == 0 and not args.no_cpu else None
         clocks = sampler.stop(r3["t_begin"], r3["t_end"]) if cx.rank == 0 else None
         try:
-            corpus = leg_corpus(cx, args, pcm, out, offs, lens, n_utts, steps=max(2, min(args.steps, 10)))
+            # the headline of --config 4 times exactly --steps steps; as a side block of --config 3, 2 to 10
+            corpus_steps = args.steps if config == 4 else max(2, min(args.steps, 10))
+            corpus = leg_corpus(cx, args, pcm, out, offs, lens, n_utts, steps=corpus_steps)
         except Exception as e:  # NCCL missing etc.: the headline number does not depend on it
             corpus = {"unavailable": str(e)[:300]}
         e2e = None if args.no_e2e else leg_e2e(cx, args, pcm, out, offs, lens, n_utts)
@@ -712,9 +740,9 @@ def run_b200(args):
         if cx.rank == 0 and not args.no_cpu:
             if _FULL_AFFINITY:
                 os.sched_setaffinity(0, _FULL_AFFINITY)   # the CPU baseline uses every host core, not one NUMA node
-            threads = os.cpu_count() or 1
-            sample = pcm[:64 * n].cpu().numpy().reshape(64, n)
             import oracle_lib as ol
+            threads = cpu_arm_threads(ol)
+            sample = pcm[:64 * n].cpu().numpy().reshape(64, n)
             lib1 = ol.RefLib("ref" if ol.available("ref") else "port")
             _, s1 = lib1.extract(params_dict(), [sample[i] for i in range(16)], sample_limit=0, n_threads=1)
             rate1 = 16 * T / s1
@@ -770,7 +798,7 @@ def run_b200(args):
                 roof = dict(corpus.get("roofline", {}), kernel="k_fused_mfcc + k_reduce_partials(_level1) + ncclAllReduce + k_finalize_stats + k_normalize_tiles",
                             peak_source="measured" if cx.peaks else "fallback", traffic=None)
                 value, ms_per_step = corpus.get("value"), corpus.get("ms_per_step")
-                launches, scaling = corpus.get("launches_per_step", 0) * max(2, min(args.steps, 10)), "strong" if cx.world >= 2 else "weak"
+                launches, scaling = corpus.get("launches_per_step", 0) * args.steps, "strong" if cx.world >= 2 else "weak"
                 extra["config3_on_this_shard"] = {"value": r3["value"], "ms_per_step": r3["ms_per_step"]}
             line = {"metric": METRIC, "value": value, "unit": UNIT, "n_gpus": cx.world, "steps": args.steps, "warmup": args.warmup,
                     "ms_per_step": ms_per_step, "higher_is_better": True, "scaling": scaling, "vs_baseline": None,
@@ -780,7 +808,7 @@ def run_b200(args):
                     "extra": extra, "kernels_per_step": [r3["kernel"]], "tiles_per_gpu": r3["tiles"],
                     "flags": {"tma": not args.no_tma, "devtools": bool(afe.lib().afe_build_flags() & 1), "abi": afe.lib().afe_abi_version()}}
     else:
-        r5 = leg_config5(cx, args, steps=max(5, args.steps))
+        r5 = leg_config5(cx, args, steps=args.steps)
         clocks = sampler.stop() if cx.rank == 0 else None
         if cx.rank == 0:
             g8 = CFG8
@@ -795,7 +823,7 @@ def run_b200(args):
                     "warmup": args.warmup, "ms_per_step": ms, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
                     "dtype": "f32", "data": "synthetic", "config": workload_config(5, 1, cx.world),
                     "audio_hours_per_s": r5["no_norm"]["frames_per_s"] * g8["S"] / g8["sr"] / 3600.0, "roofline": roof,
-                    "cpu_baseline": None, "e2e": None, "gpu_launches": r5["no_norm"]["kernel_launches"] * max(5, args.steps), "clocks": clocks,
+                    "cpu_baseline": None, "e2e": None, "gpu_launches": r5["no_norm"]["kernel_launches"] * args.steps, "clocks": clocks,
                     "extra": {"config5": r5}, "flags": {"devtools": bool(afe.lib().afe_build_flags() & 1)}}
     if cx.rank == 0:
         print(json.dumps(line), flush=True)
@@ -819,7 +847,13 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the config-4 / config-5 / stream-object extra blocks")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the features of the last timed step (256 utterances, fixed "
+                    "sample) to DIR/features.npy (--config 3)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.config != 3):
+        ap.error("--dump-outputs writes the features of the --config 3 headline of the b200 implementation")
     if args.impl == "reference":
         run_reference(args)
     else:
