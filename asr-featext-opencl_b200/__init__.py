@@ -12,12 +12,12 @@ import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libafe_cuda.so")
-ABI_VERSION = 2
+ABI_VERSION = 3
 
 NORM_NONE, NORM_CMN, NORM_CVN, NORM_MINMAX = 0, 1, 2, 3
 DYN_NONE, DYN_DELTA, DYN_ACC = 0, 1, 2
 STATS_REFERENCE_BLOCK, STATS_UTTERANCE, STATS_CORPUS = 0, 1, 2
-BATCH_Q1_EXACT, BATCH_NO_TMA, BATCH_UNFUSED_NORM, BATCH_NO_CLUSTER, BATCH_MMA_PHASE2 = 1, 2, 8, 32, 64
+BATCH_Q1_EXACT, BATCH_NO_TMA, BATCH_UNFUSED_NORM, BATCH_NO_CLUSTER = 1, 2, 8, 32
 OPT_FIX_FLUSH_STATICS, OPT_STAGED_KERNELS = 1, 2
 
 # every symbol include/afe_cuda.h declares (tests/test_abi.py checks the header against this list and the .so)

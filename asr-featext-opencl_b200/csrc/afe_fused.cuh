@@ -29,6 +29,7 @@
 #include <cfloat>
 
 #include "afe_fft.cuh"
+#include "afe_internal.h"
 #include "afe_mel.cuh"
 
 namespace afe {
@@ -65,10 +66,6 @@ struct MelConst {
     float4 dct4[kMaxBanks][4];   // [nb][16]
     int desc[kMaxBanks];         // fchunk[b] (first 4-bin chunk = edges[b] / 4; leading weights are zero) | n8[b] << 16
     short wstart[8];             // first float4 of warp class w (8 warps per CTA)
-    // tensor-core variant of phase 2 (template parameter MMA): work units of warp w, -1 = none. A unit = (half round m: frames
-    // 16m .. 16m+15) x (filter tile j: filters 8j .. 8j+7), its band of the mel matrix in steps of 8 bins
-    int mma_unit[8][2];          // m | j << 4 | first step << 8 | steps << 16
-    int mma_boff[8][2];          // first fragment row of the unit's filter tile in FusedArgs::mma_bfrag
 };
 
 struct FusedArgs {
@@ -107,9 +104,6 @@ struct FusedArgs {
     // output frames, the last one shorter) and, with blk_spec, one more tile holding the D rows a flush() right after this
     // block would return (right edge replicated, no statistics): see dev::load_tile.
     int blk_ntiles, blk_T, blk_t_first, blk_n_out, blk_nout, blk_spec, blk_spec_q1;
-    // MMA variant: the mel matrix band and the DCT matrix as mma.sync m16n8k8 B fragments, split into TF32 (hi, lo) terms:
-    // [fragment row][lane] = (b0.hi, b1.hi, b0.lo, b1.lo); see dev::mma_phase2_unit
-    const float4 *mma_bfrag, *mma_dfrag;
     int stats_kind;      // 0: none, 1: sums (CMN), 2: + sums of squares (CVN), 3: + min/max (MINMAX)
     int tc_max;          // capacity (frames) of the cepstra tile
     float rden1, rden2;  // 1 / (2*sum(l^2))
@@ -229,6 +223,22 @@ __device__ __forceinline__ double ld_peer_f64(const double *local, uint32_t rank
 }
 
 __device__ __forceinline__ int clampi(int v, int lo, int hi) { return v < lo ? lo : (v > hi ? hi : v); }
+
+// The tile's record of column c: its rp row-group records rec[g][width][4] (sum, sumsq, min, max) summed in group order,
+// stored to dst(). The destination address is formed after the loop: computed by the caller and held across it, it changed
+// ptxas' register allocation and schedule of the whole epilogue.
+template <class Dst>
+__device__ __forceinline__ void sum_row_groups(const double *rec, int rp, int width, int c, Dst dst)
+{
+    double s0 = 0.0, s1 = 0.0, lo = (double)FLT_MAX, hi = -(double)FLT_MAX;
+    for (int g = 0; g < rp; g++) {
+        const double *p = rec + (g * width + c) * 4;
+        s0 += p[0]; s1 += p[1];
+        lo = fmin(lo, p[2]); hi = fmax(hi, p[3]);
+    }
+    double *d = dst();
+    d[0] = s0; d[1] = s1; d[2] = lo; d[3] = hi;
+}
 
 } // namespace dev
 
@@ -354,32 +364,6 @@ __device__ __forceinline__ void phase3_l3(const int KIND, const FusedArgs &a, co
     }
 }
 
-} // namespace dev
-
-namespace dev {
-// ---- phase 2 on the tensor cores (mma.sync m16n8k8, TF32 operands, FP32 accumulate), 3xTF32: x = hi + lo,
-// a*b ~ a.lo*b.hi + a.hi*b.lo + a.hi*b.hi (the lo*lo term is below 2^-20 relative). The constant B operands are split with
-// round-to-nearest on the host; the A operands here by truncation - hi = the upper 19 bits, lo = x - hi (exact), of which the
-// tensor core again reads the upper 19 bits: two instructions per value (cvt.rna.tf32 is emulated with four on sm_100a).
-__device__ __forceinline__ void mma_tf32(float (&c)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1)
-{
-    asm volatile("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, {%0, %1, %2, %3};"
-                 : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-                 : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-// c += A * B with A given as fp32 values (split here) and B as a pre-split fragment (b0.hi, b1.hi, b0.lo, b1.lo)
-__device__ __forceinline__ void mma_3xtf32(float (&c)[4], const float (&av)[4], const float4 b)
-{
-    uint32_t ah[4], al[4];
-#pragma unroll
-    for (int i = 0; i < 4; i++) {
-        ah[i] = __float_as_uint(av[i]) & 0xffffe000u;
-        al[i] = __float_as_uint(av[i] - __uint_as_float(ah[i]));
-    }
-    mma_tf32(c, al, __float_as_uint(b.x), __float_as_uint(b.y));
-    mma_tf32(c, ah, __float_as_uint(b.z), __float_as_uint(b.w));
-    mma_tf32(c, ah, __float_as_uint(b.x), __float_as_uint(b.y));
-}
 } // namespace dev
 
 namespace dev {
@@ -558,7 +542,7 @@ __device__ __forceinline__ void normalise_role(const FusedArgs &a, const Tile tl
 
 // KF = filters per warp in phase 2 (ceil(num_banks / WARPS), rounded up to 3, 5 or 8): the phase is unrolled KF times,
 // so a tight bound keeps the round loop inside the instruction cache.
-template <int N2, int NZ, int kFusedWarps, int KF, bool PRE, bool MMA = false>
+template <int N2, int NZ, int kFusedWarps, int KF, bool PRE>
 __global__ void __launch_bounds__(32 * kFusedWarps, 2)
 k_fused_mfcc(const FusedArgs a, const FusedSmem L, const __grid_constant__ MelConst mc)
 {
@@ -675,54 +659,7 @@ k_fused_mfcc(const FusedArgs a, const FusedSmem L, const __grid_constant__ MelCo
         // ---- phase 2: lane = frame of the round, warp = filter class (filters warp, warp + WARPS, ...).
         //      Three unrolled passes over the warp's <= KF filters - sums, logs, DCT - so that the independent filters'
         //      long dependency chains (accumulation, logf) interleave instead of running back to back.
-        if constexpr (MMA) {
-            // ---- phase 2 on the tensor cores: a warp takes up to two units (half round m, filter tile j). Mel sums: the
-            // magnitudes of 16 frames x 8 bins are an A fragment read straight from the magnitude rows (conflict free: the 8 rows
-            // of a half round are 4 banks apart), the band of the mel matrix comes as pre-split B fragments from global memory
-            // (L1 resident, 19 KB). The accumulator fragment holds E[frame g / g+8][filter 2t / 2t+1]: after the log it IS the A
-            // fragment of the DCT product (the DCT fragments are built with the rows in that order), no data movement.
-            const int g = lane >> 2, t = lane & 3;
-#pragma unroll 1
-            for (int ui = 0; ui < 2; ui++) {
-                const int ud = mc.mma_unit[warp][ui];
-                if (ud < 0) break;
-                const int m = ud & 1, j = (ud >> 4) & 15, s0 = (ud >> 8) & 255, ns = (ud >> 16) & 255;
-                const float4 *bf = a.mma_bfrag + (size_t)mc.mma_boff[warp][ui] * 32 + lane;
-                const int row = 16 * m + (g >> 1) + 4 * (g & 1);                     // mag_row(16 m + g); + 8 for frame g + 8
-                const float *r0 = s_mags + row * kMagStride + 8 * s0 + t, *r1 = r0 + 8 * kMagStride;
-                float e[4] = {0.f, 0.f, 0.f, 0.f};
-#pragma unroll 2
-                for (int s = 0; s < ns; s++, r0 += 8, r1 += 8, bf += 32) {
-                    const float4 b = __ldg(bf);
-                    const float av[4] = {r0[0], r1[0], r0[4], r1[4]};
-                    dev::mma_3xtf32(e, av, b);
-                }
-                const float2 l01 = dev::mel_log2<FAST>(make_float2(e[0], e[1])), l23 = dev::mel_log2<FAST>(make_float2(e[2], e[3]));
-                if (a.dct_len > 0) {
-                    const float lv[4] = {l01.x, l23.x, l01.y, l23.y};                // a0 (g, 2t) a1 (g+8, 2t) a2 (g, 2t+1) a3 (g+8, 2t+1)
-#pragma unroll
-                    for (int ct = 0; ct < 2; ct++) {
-                        float dd[4] = {0.f, 0.f, 0.f, 0.f};
-                        dev::mma_3xtf32(dd, lv, __ldg(a.mma_dfrag + (j * 2 + ct) * 32 + lane));
-                        // partial cepstra of (m, j), columns 8 ct .. 8 ct + 7 -> the exchange tile of the warp 2 m + ct that sums them
-                        float *part = reinterpret_cast<float *>(smem + L.off_part + (2 * m + ct) * L.w_scratch) + (j * 16 + g) * 8 + 2 * t;
-                        *reinterpret_cast<float2 *>(part) = make_float2(dd[0], dd[1]);
-                        *reinterpret_cast<float2 *>(part + 64) = make_float2(dd[2], dd[3]);
-                    }
-                } else {
-                    const int fa = 16 * m + g, fb = fa + 8, b0 = 8 * j + 2 * t;
-                    if (fa < nfr) {
-                        if (b0 < a.nb) s_cep[(f0 + fa) * cols + b0] = l01.x;
-                        if (b0 + 1 < a.nb) s_cep[(f0 + fa) * cols + b0 + 1] = l01.y;
-                    }
-                    if (fb < nfr) {
-                        if (b0 < a.nb) s_cep[(f0 + fb) * cols + b0] = l23.x;
-                        if (b0 + 1 < a.nb) s_cep[(f0 + fb) * cols + b0 + 1] = l23.y;
-                    }
-                }
-            }
-        } else
-        #ifdef AFE_DEVTOOLS
+#ifdef AFE_DEVTOOLS
         if (lane < nfr && !(a.debug_skip & 2)) {
 #else
         if (lane < nfr) {
@@ -802,27 +739,7 @@ k_fused_mfcc(const FusedArgs a, const FusedSmem L, const __grid_constant__ MelCo
             }
         }
         __syncthreads(); // B: partial cepstra are complete; the magnitudes may be overwritten
-        if (MMA) {
-            // warp q < 4 sums, over the filter tiles j, the partial cepstra of half round q / 2, columns 8 (q % 2) .. + 7: they sit
-            // in ITS OWN exchange tile as [j][16 frames][8 columns]; lane = (frame, 4 columns)
-            if (a.dct_len > 0 && warp < 4) {
-                const int nt = (a.nb + 7) >> 3, fr = 16 * (warp >> 1) + (lane >> 1), c0 = 8 * (warp & 1) + 4 * (lane & 1);
-                const float4 *part = reinterpret_cast<const float4 *>(w_scratch) + (lane >> 1) * 2 + (lane & 1);
-                float4 tsum = part[0];
-                for (int j = 1; j < nt; j++) {
-                    const float4 u = part[j * 32];
-                    tsum.x += u.x; tsum.y += u.y; tsum.z += u.z; tsum.w += u.w;
-                }
-                if (fr < nfr) {
-                    float *crow = s_cep + (f0 + fr) * cols + c0;
-                    if (c0 + 0 < a.dct_len) crow[0] = tsum.x;
-                    if (c0 + 1 < a.dct_len) crow[1] = tsum.y;
-                    if (c0 + 2 < a.dct_len) crow[2] = tsum.z;
-                    if (c0 + 3 < a.dct_len) crow[3] = tsum.w;
-                }
-                __syncwarp();
-            }
-        } else if (a.dct_len > 0 && warp < 4) {
+        if (a.dct_len > 0 && warp < 4) {
             // warp w (< 4) sums columns 4w..4w+3 of every frame over the filter classes, in a fixed order. The partials
             // sit in ITS OWN exchange tile, so no CTA barrier is needed before the next round's FFTs reuse that memory.
             // (Spreading this sum over all 8 warps was measured 6 % SLOWER, tools/gpu_ab.sh: warps 4-7 running ahead
@@ -883,17 +800,7 @@ k_fused_mfcc(const FusedArgs a, const FusedSmem L, const __grid_constant__ MelCo
         float *s_mean = reinterpret_cast<float *>(smem + L.off_mags + 30 * 1024), *s_scale = s_mean + width;
         dev::phase3_l3<1>(a.stats_kind, a, tl, s_cep, c0f, c1f, s_red3, tid, kFusedThreads, rs);
         __syncthreads();
-        if (tid < width) {
-            const int rp = kFusedThreads / cols;
-            double s0 = 0.0, s1 = 0.0, lo = (double)FLT_MAX, hi = -(double)FLT_MAX;
-            for (int g = 0; g < rp; g++) {
-                const double *p = s_red3 + (g * width + tid) * 4;
-                s0 += p[0]; s1 += p[1];
-                lo = fmin(lo, p[2]); hi = fmax(hi, p[3]);
-            }
-            double *rec = s_rec + tid * 4;
-            rec[0] = s0; rec[1] = s1; rec[2] = lo; rec[3] = hi;
-        }
+        if (tid < width) dev::sum_row_groups(s_red3, kFusedThreads / cols, width, tid, [&] { return s_rec + tid * 4; });
         dev::cluster_sync(); // every tile's record is in its CTA's shared memory
         if (tid < width) {   // normalizercpu.cpp:31-66
             const double *rec = s_rec + (a.norm_after_dyn ? tid : tid % cols) * 4;
@@ -903,10 +810,8 @@ k_fused_mfcc(const FusedArgs a, const FusedSmem L, const __grid_constant__ MelCo
                 s0 += dev::ld_peer_f64(rec, t); s1 += dev::ld_peer_f64(rec + 1, t);
                 lo = fmin(lo, dev::ld_peer_f64(rec + 2, t)); hi = fmax(hi, dev::ld_peer_f64(rec + 3, t));
             }
-            const double n = (double)n_stats;
-            float m = (float)(s0 / n), sc = 1.f;
-            if (a.norm_type == AFE_NORM_CVN) sc = (float)sqrt((n - 1.0) / (s1 - s0 * (s0 / n)));
-            else if (a.norm_type == AFE_NORM_MINMAX) sc = 1.f / fmaxf(fabsf((float)lo - m), fabsf((float)hi - m));
+            float m, sc;
+            finalize_column(a.norm_type, (double)n_stats, s0, s1, (float)lo, (float)hi, m, sc);
             if (!a.norm_after_dyn && tid >= cols) m = 0.f;
             s_mean[tid] = m; s_scale[tid] = sc;
             if (a.g_mean && tile_idx == tl.tile0) { // every tile holds the same values: the group's first tile exports them
@@ -928,17 +833,8 @@ k_fused_mfcc(const FusedArgs a, const FusedSmem L, const __grid_constant__ MelCo
         dev::phase3_l3<0>(a.stats_kind, a, tl, s_cep, c0f, c1f, s_red3, tid, kFusedThreads, rs);
         if (a.partials) {
             __syncthreads();
-            if (tid < width) {
-                const int rp = kFusedThreads / cols;
-                double s0 = 0.0, s1 = 0.0, lo = (double)FLT_MAX, hi = -(double)FLT_MAX;
-                for (int g = 0; g < rp; g++) {
-                    const double *p = s_red3 + (g * width + tid) * 4;
-                    s0 += p[0]; s1 += p[1];
-                    lo = fmin(lo, p[2]); hi = fmax(hi, p[3]);
-                }
-                double *dst = a.partials + ((long long)tile_idx * width + tid) * 4;
-                dst[0] = s0; dst[1] = s1; dst[2] = lo; dst[3] = hi;
-            }
+            if (tid < width)
+                dev::sum_row_groups(s_red3, kFusedThreads / cols, width, tid, [&] { return a.partials + ((long long)tile_idx * width + tid) * 4; });
         }
     } else {
         if (a.nstreams >= 2) {
@@ -989,16 +885,8 @@ k_fused_mfcc(const FusedArgs a, const FusedSmem L, const __grid_constant__ MelCo
             s_red[tid * 4 + 2] = (double)mn;
             s_red[tid * 4 + 3] = (double)mx;
             __syncthreads();
-            if (tid < width) {
-                double s0 = 0.0, s1 = 0.0, lo = (double)FLT_MAX, hi = -(double)FLT_MAX;
-                for (int g = 0; g < rpp; g++) {
-                    const double *p = s_red + (g * width + tid) * 4;
-                    s0 += p[0]; s1 += p[1];
-                    lo = fmin(lo, p[2]); hi = fmax(hi, p[3]);
-                }
-                double *dst = a.partials + ((long long)tile_idx * width + tid) * 4;
-                dst[0] = s0; dst[1] = s1; dst[2] = lo; dst[3] = hi;
-            }
+            if (tid < width)
+                dev::sum_row_groups(s_red, rpp, width, tid, [&] { return a.partials + ((long long)tile_idx * width + tid) * 4; });
         }
         if (a.use_last) {
             // flush block of the streaming object, generic regression: the rows just written are normalised in place with
@@ -1033,10 +921,8 @@ k_fused_mfcc(const FusedArgs a, const FusedSmem L, const __grid_constant__ MelCo
                 dev::group_total(a.partials, width, tl.tile0, tl.ntiles, tid, kFusedThreads, s_seg, tid < width ? src_col : 0, s0, s1, lo, hi);
             }
             if (tid < width) {
-                const double n = (double)n_stats;
-                float m = (float)(s0 / n), sc = 1.f;
-                if (a.norm_type == AFE_NORM_CVN) sc = (float)sqrt((n - 1.0) / (s1 - s0 * (s0 / n)));
-                else if (a.norm_type == AFE_NORM_MINMAX) sc = 1.f / fmaxf(fabsf((float)lo - m), fabsf((float)hi - m));
+                float m, sc;
+                finalize_column(a.norm_type, (double)n_stats, s0, s1, (float)lo, (float)hi, m, sc);
                 if (!a.norm_after_dyn && tid >= cols) m = 0.f;
                 s_mean[tid] = m; s_scale[tid] = sc;
                 if (a.g_mean) {

@@ -21,13 +21,6 @@ struct FusedEngine {
     bool pruned = false;         // zero-padded window tail: the first FFT layer is pruned (NZ = 13)
     bool window_set = false;
     float pre = 0.f;             // pre-emphasis coefficient
-    // phase 2 on the tensor cores (k_fused_mfcc<..., MMA = true>): opt-in, tables rebuilt with the mel tables
-    bool want_mma = false;
-    float4 *d_bfrag = nullptr, *d_dfrag = nullptr;
-    size_t bfrag_rows = 0;
-    float mma_alpha = -1.f;
-    bool mma_active() const { return want_mma && pruned && pre == 0.f; }
-    void ensure_mma(cudaStream_t st); // (re)builds and uploads the fragment tables for mc_alpha
     FusedSmem L{};
     int tc_max = 0, nout_max = 0, key = 0;
     int cluster_probe[5] = {-1, -1, -1, -1, -1}; // max active clusters per cluster size (lazy; 0 = not schedulable)

@@ -1,23 +1,21 @@
-// One instantiation of the fused kernel per translation unit: nvcc -DAFE_INST_KEY=<0..25> (see the Makefile).
+// One instantiation of the fused kernel per translation unit: nvcc -DAFE_INST_KEY=<0..23> (see the Makefile).
 #include <atomic>
 
 #include "afe_internal.h"
 #include "afe_fused_launch.h"
 
 #ifndef AFE_INST_KEY
-#error "compile with -DAFE_INST_KEY=0..25"
+#error "compile with -DAFE_INST_KEY=0..23"
 #endif
 
 namespace afe {
 
 namespace {
-// keys 24, 25: phase 2 on the tensor cores (mma.sync, 3xTF32) for 512 / 256 points, pruned first FFT layer, no pre-emphasis
-constexpr bool kMma = AFE_INST_KEY >= 24;
 constexpr int kKey = AFE_INST_KEY % 12;
-constexpr bool kPre = !kMma && AFE_INST_KEY >= 12;   // keys 12..23: the same shapes with per-frame pre-emphasis in the load
-constexpr int kN2 = kMma ? (AFE_INST_KEY == 24 ? 512 : 256) : kKey < 6 ? 512 : 256;
-constexpr int kNZ = kMma ? 13 : (kKey % 6) < 3 ? 13 : 16;
-constexpr int kKF = kMma ? 5 : (kKey % 3) == 0 ? 3 : (kKey % 3) == 1 ? 5 : 8;
+constexpr bool kPre = AFE_INST_KEY >= 12;   // keys 12..23: the same shapes with per-frame pre-emphasis in the load
+constexpr int kN2 = kKey < 6 ? 512 : 256;
+constexpr int kNZ = (kKey % 6) < 3 ? 13 : 16;
+constexpr int kKF = (kKey % 3) == 0 ? 3 : (kKey % 3) == 1 ? 5 : 8;
 
 void fill(cudaLaunchConfig_t &cfg, cudaLaunchAttribute &attr, const FusedLaunch &fl)
 {
@@ -41,14 +39,14 @@ static cudaError_t ensure_smem_attr(int bytes)
     if (e != cudaSuccess) return e;
     if (dev < 0 || dev >= 64) dev = 63;
     if (done[dev].load(std::memory_order_acquire) >= bytes) return cudaSuccess;
-    e = cudaFuncSetAttribute(k_fused_mfcc<kN2, kNZ, 8, kKF, kPre, kMma>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+    e = cudaFuncSetAttribute(k_fused_mfcc<kN2, kNZ, 8, kKF, kPre>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
     if (e == cudaSuccess) done[dev].store(bytes, std::memory_order_release);
     return e;
 }
 
 cudaError_t AFE_CAT(fused_launch_, AFE_INST_KEY)(const FusedLaunch &fl)
 {
-    auto kern = k_fused_mfcc<kN2, kNZ, 8, kKF, kPre, kMma>;
+    auto kern = k_fused_mfcc<kN2, kNZ, 8, kKF, kPre>;
     cudaError_t e = ensure_smem_attr(fl.L.total);
     if (e != cudaSuccess) return e;
     cudaLaunchConfig_t cfg; cudaLaunchAttribute attr;
@@ -58,7 +56,7 @@ cudaError_t AFE_CAT(fused_launch_, AFE_INST_KEY)(const FusedLaunch &fl)
 
 int AFE_CAT(fused_max_clusters_, AFE_INST_KEY)(const FusedLaunch &fl)
 {
-    auto kern = k_fused_mfcc<kN2, kNZ, 8, kKF, kPre, kMma>;
+    auto kern = k_fused_mfcc<kN2, kNZ, 8, kKF, kPre>;
     if (ensure_smem_attr(fl.L.total) != cudaSuccess) return -1;
     cudaLaunchConfig_t cfg; cudaLaunchAttribute attr;
     fill(cfg, attr, fl);

@@ -15,8 +15,7 @@ struct FusedLaunch {
 };
 
 // key = (N2 == 512 ? 0 : 6) + (pruned first layer, NZ = 13 ? 0 : 3) + (KF: 3 -> 0, 5 -> 1, 8 -> 2) + (pre-emphasis ? 12 : 0)
-// keys 24 (512 points) and 25 (256 points): phase 2 on the tensor cores (template parameter MMA), pruned first layer, no pre-emphasis
-constexpr int kFusedVariants = 26;
+constexpr int kFusedVariants = 24;
 cudaError_t launch_fused_variant(int key, const FusedLaunch &fl);
 // occupancy probe for the cluster path (cudaOccupancyMaxActiveClusters); < 0 on error
 int fused_variant_max_clusters(int key, const FusedLaunch &fl);

@@ -158,14 +158,9 @@ int afe_cmvn_finalize_host(int norm_type, int width, const double *stats, float 
         const int w = width;
         const double n = stats[2 * (size_t)w];
         if (!(n >= 1)) throw Error("cmvn finalize: empty statistics");
-        for (int c = 0; c < w; c++) {
-            const double s = stats[c], s2 = stats[w + c];
-            const float mn = (float)stats[2 * w + 1 + c], mx = (float)stats[3 * w + 1 + c];
-            mean[c] = (float)(s / n);
-            if (norm_type == AFE_NORM_CVN) scale[c] = (float)sqrt((n - 1) / (s2 - s * (s / n)));
-            else if (norm_type == AFE_NORM_MINMAX) scale[c] = 1.f / std::fmax(std::fabs(mn - mean[c]), std::fabs(mx - mean[c]));
-            else scale[c] = 1.f;
-        }
+        for (int c = 0; c < w; c++)
+            finalize_column(norm_type, n, stats[c], stats[w + c], (float)stats[2 * w + 1 + c], (float)stats[3 * w + 1 + c],
+                            mean[c], scale[c]);
     });
 }
 

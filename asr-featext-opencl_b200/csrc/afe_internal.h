@@ -57,6 +57,20 @@ struct Derived {
     explicit Derived(const afe_params &p);
 };
 
+// ---- mean / scale of one column from its statistics (normalizercpu.cpp:31-66): mean s/n; CVN sqrt((n-1)/(s2 - s*(s/n)));
+// MINMAX 1/max(|mn-m|,|mx-m|); otherwise 1. The one copy of the rule: K1's cluster and ticket schemes, K2, the Normalizer
+// kernels and afe_cmvn_finalize_host all call it, so the device paths agree bit for bit.
+__host__ __device__ inline void finalize_column(int norm_type, double n, double s, double s2, float mn, float mx, float &mean,
+                                                float &scale)
+{
+    const float m = (float)(s / n);
+    float sc = 1.f;
+    if (norm_type == AFE_NORM_CVN) sc = (float)sqrt((n - 1.0) / (s2 - s * (s / n)));
+    else if (norm_type == AFE_NORM_MINMAX) sc = 1.f / fmaxf(fabsf(mn - m), fabsf(mx - m));
+    mean = m;
+    scale = sc;
+}
+
 // ---- host tables (afe_host.cpp)
 void build_filters(const Derived &d, float alpha, std::vector<int> &edges, std::vector<float> &filters);
 void build_dct(const Derived &d, std::vector<float> &dct);

@@ -227,23 +227,24 @@ void launch_delta(const float *d_in, float *d_out, int rows, int dim, int L, cud
 }
 
 // ------------------------------------------------------------------------------------------------ normalizer
-// One CTA per column; rows strided over threads, double accumulation, fixed-order tree: deterministic.
 // Replaces norm.cl kernelSum + kernelFinalizeSum with the CPU class' double statistics (normalizercpu.cpp:31-66).
-__global__ void k_colstats(const float *__restrict__ x, int rows, int dim, int norm_type, float *__restrict__ mean,
-                           float *__restrict__ scale)
+// Statistics of column c over the CTA (256 threads): rows strided over threads, double accumulation, fixed-order tree:
+// deterministic. Every thread gets the totals.
+__device__ __forceinline__ void block_column_stats(const float *__restrict__ x, int rows, int dim, int c, double &sum,
+                                                   double &sumsq, float &mn, float &mx)
 {
     __shared__ double s_sum[256], s_sq[256];
     __shared__ float s_mn[256], s_mx[256];
-    const int c = blockIdx.x, t = threadIdx.x;
+    const int t = threadIdx.x;
     double s = 0.0, s2 = 0.0;
-    float mn = FLT_MAX, mx = -FLT_MAX;
+    float lo = FLT_MAX, hi = -FLT_MAX;
     for (int r = t; r < rows; r += blockDim.x) {
         const float v = x[(long long)r * dim + c];
         s += (double)v;
         s2 += (double)__fmul_rn(v, v);
-        mn = fminf(mn, v); mx = fmaxf(mx, v);
+        lo = fminf(lo, v); hi = fmaxf(hi, v);
     }
-    s_sum[t] = s; s_sq[t] = s2; s_mn[t] = mn; s_mx[t] = mx;
+    s_sum[t] = s; s_sq[t] = s2; s_mn[t] = lo; s_mx[t] = hi;
     __syncthreads();
     for (int o = blockDim.x / 2; o > 0; o >>= 1) {
         if (t < o) {
@@ -252,14 +253,18 @@ __global__ void k_colstats(const float *__restrict__ x, int rows, int dim, int n
         }
         __syncthreads();
     }
-    if (t == 0) {
-        const double n = (double)rows, sum = s_sum[0];
-        const float m = (float)(sum / n);
-        mean[c] = m;
-        if (norm_type == AFE_NORM_CVN) scale[c] = (float)sqrt((n - 1.0) / (s_sq[0] - sum * (sum / n)));
-        else if (norm_type == AFE_NORM_MINMAX) scale[c] = 1.f / fmaxf(fabsf(s_mn[0] - m), fabsf(s_mx[0] - m));
-        else scale[c] = 1.f;
-    }
+    sum = s_sum[0]; sumsq = s_sq[0]; mn = s_mn[0]; mx = s_mx[0];
+}
+
+// one CTA per column -> the column's mean / scale
+__global__ void k_colstats(const float *__restrict__ x, int rows, int dim, int norm_type, float *__restrict__ mean,
+                           float *__restrict__ scale)
+{
+    const int c = blockIdx.x;
+    double s, s2;
+    float mn, mx;
+    block_column_stats(x, rows, dim, c, s, s2, mn, mx);
+    if (threadIdx.x == 0) finalize_column(norm_type, (double)rows, s, s2, mn, mx, mean[c], scale[c]);
 }
 void launch_colstats(const float *d_x, int rows, int dim, int norm_type, float *d_mean, float *d_scale, cudaStream_t st)
 {
@@ -276,33 +281,17 @@ __global__ void k_record_reset(double *rec, int dim)
     if (c < dim) { rec[c] = 0.0; rec[dim + c] = 0.0; rec[2 * dim + 1 + c] = (double)FLT_MAX; rec[3 * dim + 1 + c] = -(double)FLT_MAX; }
     if (c == 0) rec[2 * dim] = 0.0;
 }
-// one CTA per column, same fixed-order tree as k_colstats; the column's totals are ADDED to the record (calls are stream ordered)
+// one CTA per column, same reduction as k_colstats; the column's totals are ADDED to the record (calls are stream ordered)
 __global__ void k_record_accumulate(const float *__restrict__ x, int rows, int dim, double *__restrict__ rec)
 {
-    __shared__ double s_sum[256], s_sq[256];
-    __shared__ float s_mn[256], s_mx[256];
-    const int c = blockIdx.x, t = threadIdx.x;
-    double s = 0.0, s2 = 0.0;
-    float mn = FLT_MAX, mx = -FLT_MAX;
-    for (int r = t; r < rows; r += blockDim.x) {
-        const float v = x[(long long)r * dim + c];
-        s += (double)v;
-        s2 += (double)__fmul_rn(v, v);
-        mn = fminf(mn, v); mx = fmaxf(mx, v);
-    }
-    s_sum[t] = s; s_sq[t] = s2; s_mn[t] = mn; s_mx[t] = mx;
-    __syncthreads();
-    for (int o = blockDim.x / 2; o > 0; o >>= 1) {
-        if (t < o) {
-            s_sum[t] += s_sum[t + o]; s_sq[t] += s_sq[t + o];
-            s_mn[t] = fminf(s_mn[t], s_mn[t + o]); s_mx[t] = fmaxf(s_mx[t], s_mx[t + o]);
-        }
-        __syncthreads();
-    }
-    if (t == 0) {
-        rec[c] += s_sum[0]; rec[dim + c] += s_sq[0];
-        rec[2 * dim + 1 + c] = fmin(rec[2 * dim + 1 + c], (double)s_mn[0]);
-        rec[3 * dim + 1 + c] = fmax(rec[3 * dim + 1 + c], (double)s_mx[0]);
+    const int c = blockIdx.x;
+    double s, s2;
+    float mn, mx;
+    block_column_stats(x, rows, dim, c, s, s2, mn, mx);
+    if (threadIdx.x == 0) {
+        rec[c] += s; rec[dim + c] += s2;
+        rec[2 * dim + 1 + c] = fmin(rec[2 * dim + 1 + c], (double)mn);
+        rec[3 * dim + 1 + c] = fmax(rec[3 * dim + 1 + c], (double)mx);
         if (c == 0) rec[2 * dim] += (double)rows;
     }
 }
@@ -311,13 +300,8 @@ __global__ void k_record_finalize(const double *__restrict__ rec, int dim, int n
 {
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= dim) return;
-    const double n = rec[2 * dim], s = rec[c], s2 = rec[dim + c];
-    const float mn = (float)rec[2 * dim + 1 + c], mx = (float)rec[3 * dim + 1 + c];
-    const float m = (float)(s / n);
-    mean[c] = m;
-    if (norm_type == AFE_NORM_CVN) scale[c] = (float)sqrt((n - 1.0) / (s2 - s * (s / n)));
-    else if (norm_type == AFE_NORM_MINMAX) scale[c] = 1.f / fmaxf(fabsf(mn - m), fabsf(mx - m));
-    else scale[c] = 1.f;
+    finalize_column(norm_type, rec[2 * dim], rec[c], rec[dim + c], (float)rec[2 * dim + 1 + c], (float)rec[3 * dim + 1 + c],
+                    mean[c], scale[c]);
 }
 void launch_record_reset(double *d_rec, int dim, cudaStream_t st)
 {

@@ -23,7 +23,9 @@ extern "C" {
 /* 2: Normalizer-owned corpus verbs (afe_normalizer_accumulate / allreduce / finalize / apply; afe_normalizer_allreduce now takes
  *    the Normalizer, afe_batch_normalizer() hands out the batch's), pre-emphasis setters, afe_build_flags, the streaming
  *    object runs on the fused kernel, AFE_BATCH_WS_KERNEL / AFE_BATCH_FAST_MATH removed. */
-#define AFE_ABI_VERSION 2
+/* 3: the tensor-core phase-2 flag (64) removed; afe_batch_set_options refuses flag bits outside AFE_BATCH_Q1_EXACT |
+ *    AFE_BATCH_NO_TMA | AFE_BATCH_UNFUSED_NORM | AFE_BATCH_NO_CLUSTER. */
+#define AFE_ABI_VERSION 3
 
 /* normalizer.h:5 */
 enum afe_norm { AFE_NORM_NONE = 0, AFE_NORM_CMN = 1, AFE_NORM_CVN = 2, AFE_NORM_MINMAX = 3 };
@@ -181,10 +183,8 @@ enum afe_batch_flags {
     AFE_BATCH_Q1_EXACT = 1,        /* reproduce the single-block flush quirk Q1 (statics of the last D rows) */
     AFE_BATCH_NO_TMA = 2,          /* stage PCM with plain vector loads instead of cp.async.bulk (debug / A-B test) */
     AFE_BATCH_UNFUSED_NORM = 8,    /* normalise with the separate K2/K3 kernels instead of inside the fused kernel (A-B test) */
-    AFE_BATCH_NO_CLUSTER = 32,     /* fused normalisation through the ticket scheme (last tile of an utterance normalises it in
+    AFE_BATCH_NO_CLUSTER = 32      /* fused normalisation through the ticket scheme (last tile of an utterance normalises it in
                                       place via L2) instead of thread-block clusters + distributed shared memory (A-B test) */
-    AFE_BATCH_MMA_PHASE2 = 64      /* mel + log + DCT on the tensor cores (mma.sync m16n8k8, 3xTF32 split, FP32 accumulate) instead of
-                                      the CUDA-core FMA phase; same tolerance, not the same bits (A-B test, see DESIGN.md §4) */
 };
 
 int afe_batch_create(const afe_params *p, int cuda_device, afe_batch **out);
@@ -192,7 +192,7 @@ void afe_batch_destroy(afe_batch *b);
 int afe_batch_set_window(afe_batch *b, const float *window);
 int afe_batch_set_alpha(afe_batch *b, float alpha);
 int afe_batch_set_preemphasis(afe_batch *b, float coefficient);                   /* see afe_mfcc_set_preemphasis */
-int afe_batch_set_options(afe_batch *b, int stats_scope, int flags);
+int afe_batch_set_options(afe_batch *b, int stats_scope, int flags);              /* flags: afe_batch_flags; other bits fail */
 /* Use the caller's CUDA stream (cudaStream_t / CUstream as void*); NULL -> the handle's own stream. */
 int afe_batch_set_stream(afe_batch *b, void *cuda_stream);
 /* sample_offsets / sample_lengths: HOST int64[n_utts], start (in samples, even) and length of each utterance inside

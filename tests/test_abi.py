@@ -23,11 +23,17 @@ def test_header_and_binding_agree():
     assert header_symbols() == sorted(afe.SYMBOLS)
 
 
-def test_library_exports_every_declared_symbol():
+def header_abi_version():
+    return int(re.search(r"#define AFE_ABI_VERSION (\d+)", open(os.path.join(ROOT, "include", "afe_cuda.h")).read()).group(1))
+
+
+def test_library_abi_version_and_exported_symbols():
+    """The library, the header and the binding name the same ABI version (3: the tensor-core phase-2 flag removed, unknown
+    batch flags refused), and the library exports every symbol the header declares."""
     L = afe.lib()
     for name in header_symbols():
         assert hasattr(L, name), name
-    assert L.afe_abi_version() == afe.ABI_VERSION == 2
+    assert L.afe_abi_version() == afe.ABI_VERSION == header_abi_version() == 3
     assert L.afe_build_flags() == 0, "the product library must not be a -DAFE_DEVTOOLS build"
 
 

@@ -297,25 +297,32 @@ def test_batch_is_deterministic_and_order_independent():
 @pytest.mark.parametrize("cfg", [dict(num_banks=40), dict(num_banks=23), dict(num_banks=64),
                                  dict(num_banks=20, window_size=200, shift=80, sample_rate=8000.0, high_freq=4000.0),
                                  dict(num_banks=40, ceps_len=0, want_c0=0), dict(num_banks=26, ceps_len=15, want_c0=1)])
-def test_batch_tensor_core_phase2_matches_oracle(oracle, cfg):
-    """AFE_BATCH_MMA_PHASE2: mel sums and DCT as mma.sync m16n8k8 products with 3xTF32 operands (FP32 accumulate) instead of the
-    CUDA-core FMA phase. Not the same bits (different summation order, split operands) but the same stated tolerance against the
-    reference's CPU classes, and within 1e-4 of the default kernel; VTLN-warped banks and ragged lengths included."""
+def test_batch_filterbank_shapes_match_oracle(oracle, cfg):
+    """Phase 2 of the fused kernel (mel sums, logs, DCT) against the reference's CPU classes for all three filters-per-warp
+    instantiations (20 to 64 banks), 256- and 512-point FFTs, FBANK output and 16 DCT columns, VTLN-warped banks and ragged
+    lengths; the handle names the instantiation that runs."""
     p = ol.default_params(norm="cmn", dyn="acc", **cfg)
     utts = synth_utterances(10, 60000, seed=51, sr=p["sample_rate"], ragged=True)
     for alpha in (1.0, 0.9):
         q = dict(p, alpha=alpha)
-        a = run_batch(q, utts, flags=afe.BATCH_Q1_EXACT | afe.BATCH_MMA_PHASE2)
-        b = run_batch(q, utts, flags=afe.BATCH_Q1_EXACT)
+        got = run_batch(q, utts, flags=afe.BATCH_Q1_EXACT)
         want = oracle_extract(oracle, q, utts, BIG)
         for i in range(len(utts)):
-            assert_close(a[i], want[i], q, f"mma phase 2 utt {i} alpha {alpha}")
-            assert np.abs(a[i] - b[i]).max() < 1e-4
-    bm = afe.BatchMfcc(to_afe_params(p, BIG), 0, flags=afe.BATCH_MMA_PHASE2)
+            assert_close(got[i], want[i], q, f"utt {i} alpha {alpha}")
+    bm = afe.BatchMfcc(to_afe_params(p, BIG), 0)
     try:
-        assert bm.kernel_name.endswith("MMA>"), bm.kernel_name
+        kf = (p["num_banks"] + 7) // 8
+        n2 = 512 if p["window_size"] > 256 else 256
+        assert bm.kernel_name == f"k_fused_mfcc<{n2},13,8,{3 if kf <= 3 else 5 if kf <= 5 else 8},false>", bm.kernel_name
     finally:
         bm.close()
+
+
+def test_batch_refuses_unknown_flags():
+    """Flag bits outside AFE_BATCH_Q1_EXACT | NO_TMA | UNFUSED_NORM | NO_CLUSTER fail loudly instead of being ignored
+    (64 selected the tensor-core phase 2 before ABI 3)."""
+    with pytest.raises(afe.AfeError, match="unknown batch flag bits 64"):
+        afe.BatchMfcc(afe.make_params(), 0, flags=64)
 
 
 @pytest.mark.parametrize("norm", ["cmn", "cvn", "minmax"])

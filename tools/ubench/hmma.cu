@@ -1,5 +1,6 @@
 // Rate of the legacy warp-level tensor path on B200: mma.sync.m16n8k8 TF32 (SASS HMMA.1688.F32.TF32), the instruction of the
-// AFE_BATCH_MMA_PHASE2 variant of k_fused_mfcc. 8 independent accumulator chains per warp, 1 / 2 / 4 warps per scheduler.
+// AFE_BATCH_MMA_PHASE2 variant of k_fused_mfcc (removed; its code is in commit c5ab662). 8 independent accumulator chains per
+// warp, 1 / 2 / 4 warps per scheduler.
 // Build: nvcc -gencode arch=compute_100a,code=sm_100a -O3 -o hmma hmma.cu
 #include <cstdio>
 #include <cstdint>
