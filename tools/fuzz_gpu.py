@@ -14,7 +14,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 import oracle_lib as ol  # noqa: E402
-from common import afe, assert_close, run_batch, synth_utterances, to_afe_params  # noqa: E402
+from common import afe, compare, run_batch, synth_utterances, to_afe_params  # noqa: E402
 
 
 def random_params(rng):
@@ -39,17 +39,6 @@ def random_params(rng):
                              lift_coef=float(rng.choice([22.0, 1.0, 16.0])) if ceps > 0 else 22.0,  # 0 divides by zero in the reference (mfcccpu.cpp:127)
                              norm=int(rng.integers(0, 4)), dyn=dyn, delta_l1=int(rng.integers(1, 5)), delta_l2=int(rng.integers(1, 5)),
                              norm_after_dyn=int(rng.random() < 0.75), alpha=float(rng.choice([1.0, 1.0, 0.9, 1.08])))
-
-
-def compare(got, want, p, what):
-    """assert_close, except that where the REFERENCE is not finite (MINMAX / CVN over a constant column, e.g. an empty filter:
-    scale = 1/0) the result only has to be non-finite in the same places."""
-    bad = ~np.isfinite(want)
-    if bad.any():
-        assert got.shape == want.shape, (what, got.shape, want.shape)
-        assert np.array_equal(bad, ~np.isfinite(got)), f"{what}: non-finite entries differ from the reference's"
-        got, want = np.where(bad, 0.0, got).astype(np.float32), np.where(bad, 0.0, want).astype(np.float32)
-    return assert_close(got, want, p, what)
 
 
 def reference_blocking_is_memory_safe(p, n, limit):
