@@ -17,7 +17,6 @@ namespace afe {
 // ------------------------------------------------------------------------------------------------ FFT tables
 void FftTables::build(int n2)
 {
-    release();
     N2 = n2;
     const int M = n2 / 2, R = M / 16;
     std::vector<float2> a((size_t)R * 16), p((size_t)M / 2);
@@ -30,27 +29,8 @@ void FftTables::build(int n2)
         const double ang = -2.0 * M_PI * (double)k / (double)n2;
         p[k] = make_float2((float)cos(ang), (float)sin(ang));
     }
-    AFE_CUDA(cudaMalloc(&d_tw_a, a.size() * sizeof(float2)));
-    AFE_CUDA(cudaMalloc(&d_tw_p, p.size() * sizeof(float2)));
-    AFE_CUDA(cudaMemcpy(d_tw_a, a.data(), a.size() * sizeof(float2), cudaMemcpyHostToDevice));
-    AFE_CUDA(cudaMemcpy(d_tw_p, p.data(), p.size() * sizeof(float2), cudaMemcpyHostToDevice));
-}
-void FftTables::release()
-{
-    if (d_tw_a) cudaFree(d_tw_a);
-    if (d_tw_p) cudaFree(d_tw_p);
-    d_tw_a = d_tw_p = nullptr;
-}
-
-void MelTables::release()
-{
-    if (d_edges) cudaFree(d_edges);
-    if (d_pairs) cudaFree(d_pairs);
-    if (d_dct) cudaFree(d_dct);
-    if (d_window) cudaFree(d_window);
-    if (d_window2) cudaFree(d_window2);
-    d_edges = nullptr; d_pairs = nullptr; d_dct = nullptr; d_window = nullptr; d_window2 = nullptr;
-    alpha_built = -1.f;
+    d_tw_a.upload(a);
+    d_tw_p.upload(p);
 }
 
 void upload_mel_tables(const Derived &d, float alpha, MelTables &t, cudaStream_t st)
@@ -61,15 +41,15 @@ void upload_mel_tables(const Derived &d, float alpha, MelTables &t, cudaStream_t
         if (edges[i + 1] < edges[i]) throw Error("mel filter edges are not monotonic");
     if (edges.front() < 0 || edges.back() > d.M) throw Error("mel filterbank exceeds the Nyquist bin (check low_freq/high_freq)");
     build_mel_pairs(d, edges, filters, pairs);
-    if (!t.d_edges) AFE_CUDA(cudaMalloc(&t.d_edges, sizeof(int) * (d.nb + 2)));
-    if (!t.d_pairs) AFE_CUDA(cudaMalloc(&t.d_pairs, sizeof(float) * 2 * d.bins));
+    if (!t.d_edges.p) t.d_edges.alloc(d.nb + 2);
+    if (!t.d_pairs.p) t.d_pairs.alloc(2 * d.bins);
     // pageable source + stream-ordered copy: cudaMemcpyAsync from pageable memory stages synchronously, safe with locals
-    AFE_CUDA(cudaMemcpyAsync(t.d_edges, edges.data(), sizeof(int) * (d.nb + 2), cudaMemcpyHostToDevice, st));
-    AFE_CUDA(cudaMemcpyAsync(t.d_pairs, pairs.data(), sizeof(float) * 2 * d.bins, cudaMemcpyHostToDevice, st));
-    if (d.C > 0 && !t.d_dct) {
+    AFE_CUDA(cudaMemcpyAsync(t.d_edges.p, edges.data(), sizeof(int) * (d.nb + 2), cudaMemcpyHostToDevice, st));
+    AFE_CUDA(cudaMemcpyAsync(t.d_pairs.p, pairs.data(), sizeof(float) * 2 * d.bins, cudaMemcpyHostToDevice, st));
+    if (d.C > 0 && !t.d_dct.p) {
         build_dct(d, dct);
-        AFE_CUDA(cudaMalloc(&t.d_dct, sizeof(float) * dct.size()));
-        AFE_CUDA(cudaMemcpyAsync(t.d_dct, dct.data(), sizeof(float) * dct.size(), cudaMemcpyHostToDevice, st));
+        t.d_dct.alloc(dct.size());
+        AFE_CUDA(cudaMemcpyAsync(t.d_dct.p, dct.data(), sizeof(float) * dct.size(), cudaMemcpyHostToDevice, st));
     }
     AFE_CUDA(cudaStreamSynchronize(st));
     t.alpha_built = alpha;
@@ -77,12 +57,12 @@ void upload_mel_tables(const Derived &d, float alpha, MelTables &t, cudaStream_t
 
 void upload_window(const Derived &d, const float *window, MelTables &t, cudaStream_t st)
 {
-    if (!t.d_window) AFE_CUDA(cudaMalloc(&t.d_window, sizeof(float) * d.W));
-    if (!t.d_window2) AFE_CUDA(cudaMalloc(&t.d_window2, sizeof(float2) * d.M));
+    if (!t.d_window.p) t.d_window.alloc(d.W);
+    if (!t.d_window2.p) t.d_window2.alloc(d.M);
     std::vector<float> w2((size_t)d.N2, 0.f);
     memcpy(w2.data(), window, sizeof(float) * d.W);
-    AFE_CUDA(cudaMemcpyAsync(t.d_window, window, sizeof(float) * d.W, cudaMemcpyHostToDevice, st));
-    AFE_CUDA(cudaMemcpyAsync(t.d_window2, w2.data(), sizeof(float) * d.N2, cudaMemcpyHostToDevice, st));
+    AFE_CUDA(cudaMemcpyAsync(t.d_window.p, window, sizeof(float) * d.W, cudaMemcpyHostToDevice, st));
+    AFE_CUDA(cudaMemcpyAsync(t.d_window2.p, w2.data(), sizeof(float) * d.N2, cudaMemcpyHostToDevice, st));
     AFE_CUDA(cudaStreamSynchronize(st));
 }
 
@@ -234,7 +214,6 @@ FusedEngine::FusedEngine(const Derived &dd, int dev) : d(dd), device(dev)
     const int kf = (d.nb + 7) / 8;     // filters per warp (8 warps): instantiated for 3, 5 and 8
     key = (d.N2 == 512 ? 0 : 6) + (pruned ? 0 : 3) + (kf <= 3 ? 0 : kf <= 5 ? 1 : 2);
 }
-FusedEngine::~FusedEngine() { fft.release(); mel.release(); }
 
 void FusedEngine::set_window(const float *window, cudaStream_t st)
 {
@@ -301,7 +280,7 @@ int FusedEngine::plan_rows(std::vector<Tile> &tiles, long long pcm_off, long lon
 FusedArgs FusedEngine::base_args(int q1, bool use_tma) const
 {
     FusedArgs a{};
-    a.window2 = mel.d_window2; a.tw_a = fft.d_tw_a; a.tw_p = fft.d_tw_p;
+    a.window2 = mel.d_window2.p; a.tw_a = fft.d_tw_a.p; a.tw_p = fft.d_tw_p.p;
     a.norm_type = d.p.norm; a.norm_after_dyn = d.p.norm_after_dyn;
     a.W = d.W; a.S = d.S; a.nb = d.nb; a.dct_len = d.C > 0 ? d.dct_len : 0; a.cols = d.cols; a.width = d.width;
     a.l1 = d.l1; a.l2 = d.l2; a.nstreams = d.width / d.cols;
@@ -350,10 +329,16 @@ void FusedEngine::launch(const FusedArgs &a, int grid, int cluster, cudaStream_t
 using namespace afe;
 
 // ================================================================================================== afe_batch
+struct NormalizerDestroy {
+    void operator()(afe_normalizer *n) const { afe_normalizer_destroy(n); }
+};
+
 struct afe_batch {
     Derived d;
     int device;
-    cudaStream_t own_stream = nullptr, stream = nullptr;
+    Stream own_stream, s_in, s_out;         // s_in / s_out: the copy streams of run_host, created by its first call
+    std::vector<Event> ev_in, ev_k;
+    cudaStream_t stream = nullptr;          // the stream in use: own_stream or the caller's
     std::unique_ptr<FusedEngine> eng;
     float alpha = 1.f;
     int scope = AFE_STATS_REFERENCE_BLOCK, flags = 0;
@@ -362,47 +347,31 @@ struct afe_batch {
     bool aligned = false;
     std::vector<int64_t> sample_off, sample_len, frame_off;
     std::vector<int> h_tile_begin;          // [n_utts+1] first tile of every utterance
-    cudaStream_t s_in = nullptr, s_out = nullptr;
-    std::vector<cudaEvent_t> ev_in, ev_k;
     int64_t pcm_extent = 0;
-    Tile *d_tiles = nullptr;
-    int *d_tile_begin = nullptr;
-    double *d_counts = nullptr, *d_partials = nullptr, *d_stats = nullptr, *d_scratch = nullptr;
-    int *d_counters = nullptr;      // [n_groups] arrival tickets + [1] role tickets of the long-utterance scheme
-    unsigned *d_flags = nullptr;    // [n_groups]
+    struct Plan {                           // the device side of a plan, replaced as a whole by afe_batch_plan
+        DevBuf<Tile> tiles;
+        DevBuf<int> tile_begin, scratch_begin;
+        DevBuf<double> counts, partials, scratch;
+        DevBuf<double> group_stats;         // per-utterance scopes: the statistics records
+        DevBuf<int> counters;               // [n_groups] arrival tickets + [1] role tickets of the long-utterance scheme
+        DevBuf<unsigned> flags;             // [n_groups]
+        DevBuf<float> mean, scale;
+        std::unique_ptr<afe_normalizer, NormalizerDestroy> cnorm; // corpus scope: the Normalizer that owns the record
+        double *stats() const { return cnorm ? cnorm->ns.rec.p : group_stats.p; } // [n_groups][4 * width + 1]
+    } plan;
     unsigned epoch = 0;
-    int *d_scratch_begin = nullptr;
-    float *d_mean = nullptr, *d_scale = nullptr;
     int corpus_blocks = 0;          // level-1 blocks of the corpus reduction (2 per SM)
-    afe_normalizer *cnorm = nullptr; // corpus scope: the Normalizer that owns the record (d_stats aliases its buffer)
     int max_tiles_per_utt = 0;
     // One tile normalising its whole utterance is right for short utterances and a serial bottleneck for long ones:
     // up to 8 tiles -> clusters / ticket scheme; more -> the role scheme (normaliser CTAs, one per tile, same launch).
     bool fuse_norm() const { return !(flags & AFE_BATCH_UNFUSED_NORM); }
     bool long_scheme() const { return max_tiles_per_utt > 8; }
     int last_launches = 0;
-    // host staging for run_host
-    int16_t *d_pcm_stage = nullptr; float *d_out_stage = nullptr;
-    size_t pcm_stage_bytes = 0, out_stage_bytes = 0;
+    // device staging for run_host (grow-only)
+    DevBuf<int16_t> pcm_stage;
+    DevBuf<float> out_stage;
 
     explicit afe_batch(const afe_params &p, int dev) : d(p), device(dev) {}
-    void free_plan()
-    {
-        if (d_tiles) cudaFree(d_tiles);
-        if (d_tile_begin) cudaFree(d_tile_begin);
-        if (d_counts) cudaFree(d_counts);
-        if (d_partials) cudaFree(d_partials);
-        if (d_stats && !cnorm) cudaFree(d_stats);
-        if (d_scratch) cudaFree(d_scratch);
-        if (d_counters) cudaFree(d_counters);
-        if (d_flags) cudaFree(d_flags);
-        if (d_scratch_begin) cudaFree(d_scratch_begin);
-        if (d_mean) cudaFree(d_mean);
-        if (d_scale) cudaFree(d_scale);
-        if (cnorm) { cnorm->st = nullptr; afe_normalizer_destroy(cnorm); cnorm = nullptr; }
-        d_tiles = nullptr; d_tile_begin = nullptr; d_counts = d_partials = d_stats = d_scratch = nullptr;
-        d_counters = nullptr; d_flags = nullptr; d_scratch_begin = nullptr; d_mean = d_scale = nullptr;
-    }
 };
 
 static FusedArgs make_fused_args(afe_batch *b, const int16_t *d_pcm, float *d_out, bool want_stats, int t0)
@@ -410,8 +379,8 @@ static FusedArgs make_fused_args(afe_batch *b, const int16_t *d_pcm, float *d_ou
     const Derived &d = b->d;
     const bool tma = b->aligned && !(b->flags & AFE_BATCH_NO_TMA) && (reinterpret_cast<uintptr_t>(d_pcm) & 15) == 0;
     FusedArgs a = b->eng->base_args((b->flags & AFE_BATCH_Q1_EXACT) ? 1 : 0, tma);
-    a.pcm = d_pcm; a.out = d_out; a.tiles = b->d_tiles; a.tile_base = t0;
-    a.partials = want_stats ? b->d_partials : nullptr;
+    a.pcm = d_pcm; a.out = d_out; a.tiles = b->plan.tiles.p; a.tile_base = t0;
+    a.partials = want_stats ? b->plan.partials.p : nullptr;
     if (!want_stats) a.stats_rows_mode = 0;
     else if (!d.p.norm_after_dyn) a.stats_rows_mode = 2;
     else a.stats_rows_mode = b->scope == AFE_STATS_REFERENCE_BLOCK ? 1 : 2;
@@ -430,7 +399,7 @@ static void run_extract(afe_batch *b, const int16_t *d_pcm, float *d_out, int t0
 {
     if (t1 < 0) t1 = b->n_tiles;
     if (t1 <= t0) return;
-    if (!b->d_tiles) throw Error("afe_batch_plan must be called before running");
+    if (!b->plan.tiles.p) throw Error("afe_batch_plan must be called before running");
     FusedEngine &eng = *b->eng;
     eng.ensure_mel(b->alpha);
     const Derived &d = b->d;
@@ -439,9 +408,9 @@ static void run_extract(afe_batch *b, const int16_t *d_pcm, float *d_out, int t0
     auto launch = [&](const FusedArgs &args, int grid, int cluster) { eng.launch(args, grid, cluster, b->stream); b->last_launches++; };
     if (!(fuse_norm && want_stats)) { launch(a, t1 - t0, 0); return; }
     if (b->long_scheme()) {
-        a.counters = b->d_counters; a.work_counter = b->d_counters + b->n_groups;
-        a.flags = b->d_flags; a.epoch = ++b->epoch; a.ntiles_launch = t1 - t0;
-        a.g_mean = b->d_mean; a.g_scale = b->d_scale;
+        a.counters = b->plan.counters.p; a.work_counter = b->plan.counters.p + b->n_groups;
+        a.flags = b->plan.flags.p; a.epoch = ++b->epoch; a.ntiles_launch = t1 - t0;
+        a.g_mean = b->plan.mean.p; a.g_scale = b->plan.scale.p;
         launch(a, (t1 - t0) + std::min(t1 - t0, 2 * eng.sm_count), 0); // + one wave of normaliser roles
         return;
     }
@@ -462,21 +431,21 @@ static void run_extract(afe_batch *b, const int16_t *d_pcm, float *d_out, int t0
                 FusedArgs ar = a;
                 ar.tile_base = r.t0;
                 if (r.cluster > 0) { ar.cluster_norm = 1; ar.counters = nullptr; }
-                else ar.counters = b->d_counters;
+                else ar.counters = b->plan.counters.p;
                 try {
                     launch(ar, r.t1 - r.t0, r.cluster);
                 } catch (const Error &) {
                     if (r.cluster == 0) throw;
                     // the clustered launch was refused (nothing ran): this run takes the ticket scheme instead
                     eng.cluster_probe[r.cluster] = 0;
-                    ar.cluster_norm = 0; ar.counters = b->d_counters;
+                    ar.cluster_norm = 0; ar.counters = b->plan.counters.p;
                     launch(ar, r.t1 - r.t0, 0);
                 }
             }
             return;
         }
     }
-    a.counters = b->d_counters;
+    a.counters = b->plan.counters.p;
     launch(a, t1 - t0, 0);
 }
 
@@ -485,16 +454,17 @@ static void run_reduce(afe_batch *b, int g0 = 0, int g1 = -1)
     if (g1 < 0) g1 = b->n_groups;
     if (g1 <= g0) return;
     const int w = b->d.width;
+    const afe_batch::Plan &pl = b->plan;
     if (b->scope == AFE_STATS_CORPUS && b->n_tiles > 2 * b->corpus_blocks) {
-        k_reduce_partials_level1<<<b->corpus_blocks, 128, 0, b->stream>>>(b->d_partials, b->n_tiles, w, b->d_scratch);
+        k_reduce_partials_level1<<<b->corpus_blocks, 128, 0, b->stream>>>(pl.partials.p, b->n_tiles, w, pl.scratch.p);
         AFE_CUDA(cudaGetLastError());
-        k_reduce_partials<<<1, 256, dev::kSegs * w * 4 * sizeof(double), b->stream>>>(b->d_scratch, b->d_scratch_begin, b->d_counts, w, b->d_stats);
+        k_reduce_partials<<<1, 256, dev::kSegs * w * 4 * sizeof(double), b->stream>>>(pl.scratch.p, pl.scratch_begin.p, pl.counts.p, w, pl.stats());
         AFE_CUDA(cudaGetLastError());
         count_launch(2); b->last_launches += 2;
         return;
     }
-    k_reduce_partials<<<g1 - g0, 256, dev::kSegs * w * 4 * sizeof(double), b->stream>>>(b->d_partials, b->d_tile_begin + g0, b->d_counts + g0, w,
-                                                                                       b->d_stats + (size_t)g0 * (4 * w + 1));
+    k_reduce_partials<<<g1 - g0, 256, dev::kSegs * w * 4 * sizeof(double), b->stream>>>(pl.partials.p, pl.tile_begin.p + g0, pl.counts.p + g0, w,
+                                                                                       pl.stats() + (size_t)g0 * (4 * w + 1));
     AFE_CUDA(cudaGetLastError());
     count_launch(); b->last_launches++;
 }
@@ -506,12 +476,13 @@ static void run_normalize(afe_batch *b, float *d_out, int t0 = 0, int t1 = -1, i
     if (g1 < 0) g1 = b->n_groups;
     if (t1 <= t0 || g1 <= g0) return;
     const size_t w = d.width;
-    k_finalize_stats<<<g1 - g0, 128, 0, b->stream>>>(b->d_stats + (size_t)g0 * (4 * w + 1), d.width, d.cols, d.p.norm,
-                                                      d.p.norm_after_dyn, b->d_mean + g0 * w, b->d_scale + g0 * w);
+    const afe_batch::Plan &pl = b->plan;
+    k_finalize_stats<<<g1 - g0, 128, 0, b->stream>>>(pl.stats() + (size_t)g0 * (4 * w + 1), d.width, d.cols, d.p.norm,
+                                                      d.p.norm_after_dyn, pl.mean.p + g0 * w, pl.scale.p + g0 * w);
     AFE_CUDA(cudaGetLastError());
     // Tile::group is absolute, so mean / scale keep their base
-    k_normalize_tiles<<<t1 - t0, 256, 2 * d.width * sizeof(float), b->stream>>>(d_out, b->d_tiles + t0, d.width, d.p.norm,
-                                                                              b->d_mean, b->d_scale);
+    k_normalize_tiles<<<t1 - t0, 256, 2 * d.width * sizeof(float), b->stream>>>(d_out, pl.tiles.p + t0, d.width, d.p.norm,
+                                                                              pl.mean.p, pl.scale.p);
     AFE_CUDA(cudaGetLastError());
     count_launch(2); b->last_launches += 2;
 }
@@ -540,11 +511,11 @@ int afe_batch_create(const afe_params *p, int cuda_device, afe_batch **out)
     *out = nullptr;
     return guarded([&] {
         if (afe_device_count() <= cuda_device) throw Error("no usable CUDA device " + std::to_string(cuda_device) + " (the product has no CPU fallback)");
+        DeviceGuard g(cuda_device);
         std::unique_ptr<afe_batch> b(new afe_batch(*p, cuda_device));
         const std::string why = fused_unsupported_reason(b->d);
         if (!why.empty()) throw Error(why + "; use the streaming object");
-        DeviceGuard g(cuda_device);
-        AFE_CUDA(cudaStreamCreateWithFlags(&b->own_stream, cudaStreamNonBlocking));
+        b->own_stream.create();
         b->stream = b->own_stream;
         b->eng.reset(new FusedEngine(b->d, cuda_device));
         *out = b.release();
@@ -556,15 +527,6 @@ void afe_batch_destroy(afe_batch *b)
     if (!b) return;
     cudaSetDevice(b->device);
     cudaStreamSynchronize(b->stream);
-    b->free_plan();
-    b->eng.reset();
-    if (b->d_pcm_stage) cudaFree(b->d_pcm_stage);
-    if (b->d_out_stage) cudaFree(b->d_out_stage);
-    if (b->own_stream) cudaStreamDestroy(b->own_stream);
-    if (b->s_in) cudaStreamDestroy(b->s_in);
-    if (b->s_out) cudaStreamDestroy(b->s_out);
-    for (auto e : b->ev_in) cudaEventDestroy(e);
-    for (auto e : b->ev_k) cudaEventDestroy(e);
     delete b;
 }
 
@@ -588,7 +550,7 @@ int afe_batch_set_options(afe_batch *b, int stats_scope, int flags)
     return guarded([&] {
         if (stats_scope < AFE_STATS_REFERENCE_BLOCK || stats_scope > AFE_STATS_CORPUS) throw Error("invalid stats scope");
         // the per-group row counts, the group table and the corpus Normalizer are laid down by afe_batch_plan from the scope
-        if (b->d_tiles && stats_scope != b->scope) throw Error("set the statistics scope before afe_batch_plan");
+        if (b->plan.tiles.p && stats_scope != b->scope) throw Error("set the statistics scope before afe_batch_plan");
         const int known = AFE_BATCH_Q1_EXACT | AFE_BATCH_NO_TMA | AFE_BATCH_UNFUSED_NORM | AFE_BATCH_NO_CLUSTER;
         if (flags & ~known) throw Error("unknown batch flag bits " + std::to_string(flags & ~known));
         b->scope = stats_scope; b->flags = flags; // every flag is read at run time
@@ -598,7 +560,7 @@ int afe_batch_set_options(afe_batch *b, int stats_scope, int flags)
 int afe_batch_set_stream(afe_batch *b, void *cuda_stream)
 {
     b->stream = cuda_stream ? (cudaStream_t)cuda_stream : b->own_stream;
-    if (b->cnorm) b->cnorm->st = b->stream;
+    if (b->plan.cnorm) b->plan.cnorm->st = b->stream;
     return 0;
 }
 
@@ -627,7 +589,7 @@ static int plan_impl(afe_batch *b, const int64_t *off, const int64_t *len, const
         const Derived &d = b->d;
         if (n_utts < 1) throw Error("plan: no utterances");
         DeviceGuard g(b->device);
-        b->free_plan();
+        b->plan = {};
         const FusedEngine &eng = *b->eng;
         b->n_utts = n_utts;
         b->sample_off.assign(off, off + n_utts);
@@ -695,34 +657,33 @@ static int plan_impl(afe_batch *b, const int64_t *off, const int64_t *len, const
         b->n_tiles = (int)tiles.size();
         b->n_groups = corpus ? 1 : n_utts;
         b->corpus_blocks = 2 * eng.sm_count;
-        AFE_CUDA(cudaMalloc(&b->d_tiles, sizeof(Tile) * tiles.size()));
-        AFE_CUDA(cudaMemcpy(b->d_tiles, tiles.data(), sizeof(Tile) * tiles.size(), cudaMemcpyHostToDevice));
+        // built aside and installed whole, so that a plan that fails here leaves the batch unplanned
+        afe_batch::Plan pl;
+        pl.tiles.upload(tiles);
         if (d.p.norm != AFE_NORM_NONE) {
             const size_t w = d.width;
-            AFE_CUDA(cudaMalloc(&b->d_tile_begin, sizeof(int) * tile_begin.size()));
-            AFE_CUDA(cudaMemcpy(b->d_tile_begin, tile_begin.data(), sizeof(int) * tile_begin.size(), cudaMemcpyHostToDevice));
-            AFE_CUDA(cudaMalloc(&b->d_counts, sizeof(double) * counts.size()));
-            AFE_CUDA(cudaMemcpy(b->d_counts, counts.data(), sizeof(double) * counts.size(), cudaMemcpyHostToDevice));
-            AFE_CUDA(cudaMalloc(&b->d_partials, sizeof(double) * 4 * w * tiles.size()));
+            pl.tile_begin.upload(tile_begin);
+            pl.counts.upload(counts);
+            pl.partials.alloc(4 * w * tiles.size());
             if (corpus) {
                 // the corpus record lives in a Normalizer of dim = width (all three streams in one record)
-                if (afe_normalizer_create(d.p.norm, d.width, b->device, &b->cnorm) != 0) throw Error(afe_last_error());
-                b->cnorm->st = b->stream;
-                b->d_stats = b->cnorm->ns.rec.p;
-                const int sb[2] = {0, b->corpus_blocks};
-                AFE_CUDA(cudaMalloc(&b->d_scratch, sizeof(double) * 4 * w * b->corpus_blocks));
-                AFE_CUDA(cudaMalloc(&b->d_scratch_begin, sizeof(sb)));
-                AFE_CUDA(cudaMemcpy(b->d_scratch_begin, sb, sizeof(sb), cudaMemcpyHostToDevice));
+                afe_normalizer *n = nullptr;
+                if (afe_normalizer_create(d.p.norm, d.width, b->device, &n) != 0) throw Error(afe_last_error());
+                pl.cnorm.reset(n);
+                n->st = b->stream;
+                pl.scratch.alloc(4 * w * b->corpus_blocks);
+                pl.scratch_begin.upload({0, b->corpus_blocks});
             } else
-                AFE_CUDA(cudaMalloc(&b->d_stats, sizeof(double) * (4 * w + 1) * b->n_groups));
-            AFE_CUDA(cudaMalloc(&b->d_counters, sizeof(int) * (b->n_groups + 1)));
-            AFE_CUDA(cudaMemset(b->d_counters, 0, sizeof(int) * (b->n_groups + 1)));
-            AFE_CUDA(cudaMalloc(&b->d_flags, sizeof(unsigned) * b->n_groups));
-            AFE_CUDA(cudaMemset(b->d_flags, 0, sizeof(unsigned) * b->n_groups));
+                pl.group_stats.alloc((4 * w + 1) * b->n_groups);
+            pl.counters.alloc(b->n_groups + 1);
+            AFE_CUDA(cudaMemset(pl.counters.p, 0, sizeof(int) * (b->n_groups + 1)));
+            pl.flags.alloc(b->n_groups);
+            AFE_CUDA(cudaMemset(pl.flags.p, 0, sizeof(unsigned) * b->n_groups));
             b->epoch = 0;
-            AFE_CUDA(cudaMalloc(&b->d_mean, sizeof(float) * w * b->n_groups));
-            AFE_CUDA(cudaMalloc(&b->d_scale, sizeof(float) * w * b->n_groups));
+            pl.mean.alloc(w * b->n_groups);
+            pl.scale.alloc(w * b->n_groups);
         }
+        b->plan = std::move(pl);
         if (total_frames) *total_frames = b->frame_off[n_utts];
     });
 }
@@ -740,7 +701,7 @@ const char *afe_batch_kernel_name(const afe_batch *b)
     name = b->eng ? b->eng->kernel_label() : "k_fused_mfcc";
     return name.c_str();
 }
-afe_normalizer *afe_batch_normalizer(afe_batch *b) { return b->cnorm; }
+afe_normalizer *afe_batch_normalizer(afe_batch *b) { return b->plan.cnorm.get(); }
 
 int afe_batch_extract_device(afe_batch *b, const int16_t *d_pcm, float *d_out)
 {
@@ -766,7 +727,7 @@ int afe_batch_corpus_stats(afe_batch *b, double **d_stats, int *stats_len)
         DeviceGuard g(b->device);
         if (b->d.p.norm == AFE_NORM_NONE) throw Error("corpus_stats: norm is NONE");
         run_reduce(b);
-        if (d_stats) *d_stats = b->d_stats;
+        if (d_stats) *d_stats = b->plan.stats();
         if (stats_len) *stats_len = (4 * b->d.width + 1) * b->n_groups;
     });
 }
@@ -777,7 +738,7 @@ int afe_batch_set_corpus_stats(afe_batch *b, const double *h_stats, int stats_le
         DeviceGuard g(b->device);
         if (b->d.p.norm == AFE_NORM_NONE) throw Error("set_corpus_stats: norm is NONE");
         if (stats_len != (4 * b->d.width + 1) * b->n_groups) throw Error("set_corpus_stats: wrong length");
-        AFE_CUDA(cudaMemcpyAsync(b->d_stats, h_stats, sizeof(double) * stats_len, cudaMemcpyHostToDevice, b->stream));
+        AFE_CUDA(cudaMemcpyAsync(b->plan.stats(), h_stats, sizeof(double) * stats_len, cudaMemcpyHostToDevice, b->stream));
         AFE_CUDA(cudaStreamSynchronize(b->stream));
     });
 }
@@ -804,34 +765,22 @@ int afe_batch_run_host(afe_batch *b, const int16_t *h_pcm, float *h_out)
     return guarded([&] {
         DeviceGuard g(b->device);
         const Derived &d = b->d;
-        if (!b->d_tiles) throw Error("afe_batch_plan must be called before running");
+        if (!b->plan.tiles.p) throw Error("afe_batch_plan must be called before running");
         if (b->scope == AFE_STATS_CORPUS && d.p.norm != AFE_NORM_NONE)
             throw Error("run_host: corpus statistics need the two-pass device sequence");
         const size_t n_samples = (size_t)b->pcm_extent;
-        const size_t pcm_bytes = n_samples * 2 + 32, out_bytes = (size_t)b->frame_off.back() * d.width * 4;
-        if (pcm_bytes > b->pcm_stage_bytes) {
-            if (b->d_pcm_stage) cudaFree(b->d_pcm_stage);
-            AFE_CUDA(cudaMalloc(&b->d_pcm_stage, pcm_bytes));
-            b->pcm_stage_bytes = pcm_bytes;
-        }
-        if (out_bytes > b->out_stage_bytes) {
-            if (b->d_out_stage) cudaFree(b->d_out_stage);
-            AFE_CUDA(cudaMalloc(&b->d_out_stage, out_bytes));
-            b->out_stage_bytes = out_bytes;
-        }
-        if (!b->s_in) {
-            AFE_CUDA(cudaStreamCreateWithFlags(&b->s_in, cudaStreamNonBlocking));
-            AFE_CUDA(cudaStreamCreateWithFlags(&b->s_out, cudaStreamNonBlocking));
-        }
+        const size_t pcm_len = n_samples + 16, out_len = (size_t)b->frame_off.back() * d.width;
+        if (pcm_len > b->pcm_stage.n) b->pcm_stage.alloc(pcm_len);
+        if (out_len > b->out_stage.n) b->out_stage.alloc(out_len);
+        if (!b->s_in) { b->s_in.create(); b->s_out.create(); }
         // chunks are contiguous in samples only when the utterances are packed in increasing order
         bool ordered = true;
         for (int u = 0; u + 1 < b->n_utts; u++) ordered = ordered && b->sample_off[u] + b->sample_len[u] <= b->sample_off[u + 1];
         const int n_chunks = ordered ? std::max(1, std::min(32, b->n_utts / 8)) : 1;
         while ((int)b->ev_in.size() < n_chunks) {
-            cudaEvent_t e1, e2;
-            AFE_CUDA(cudaEventCreateWithFlags(&e1, cudaEventDisableTiming));
-            AFE_CUDA(cudaEventCreateWithFlags(&e2, cudaEventDisableTiming));
-            b->ev_in.push_back(e1); b->ev_k.push_back(e2);
+            Event e1, e2;
+            e1.create(); e2.create();
+            b->ev_in.push_back(std::move(e1)); b->ev_k.push_back(std::move(e2));
         }
         b->last_launches = 0;
         const bool norm = d.p.norm != AFE_NORM_NONE;
@@ -840,17 +789,17 @@ int afe_batch_run_host(afe_batch *b, const int16_t *h_pcm, float *h_out)
             if (u1 <= u0) continue;
             const int64_t s0 = n_chunks == 1 ? 0 : b->sample_off[u0];
             const int64_t s1 = n_chunks == 1 ? (int64_t)n_samples : b->sample_off[u1 - 1] + b->sample_len[u1 - 1];
-            AFE_CUDA(cudaMemcpyAsync(b->d_pcm_stage + s0, h_pcm + s0, (size_t)(s1 - s0) * 2, cudaMemcpyHostToDevice, b->s_in));
+            AFE_CUDA(cudaMemcpyAsync(b->pcm_stage.p + s0, h_pcm + s0, (size_t)(s1 - s0) * 2, cudaMemcpyHostToDevice, b->s_in));
             AFE_CUDA(cudaEventRecord(b->ev_in[c], b->s_in));
             AFE_CUDA(cudaStreamWaitEvent(b->stream, b->ev_in[c], 0));
             const int t0 = b->h_tile_begin[u0], t1 = b->h_tile_begin[u1];
             const bool fuse = b->fuse_norm();
-            run_extract(b, b->d_pcm_stage, b->d_out_stage, t0, t1, fuse);
-            if (norm && !fuse) { run_reduce(b, u0, u1); run_normalize(b, b->d_out_stage, t0, t1, u0, u1); }
+            run_extract(b, b->pcm_stage.p, b->out_stage.p, t0, t1, fuse);
+            if (norm && !fuse) { run_reduce(b, u0, u1); run_normalize(b, b->out_stage.p, t0, t1, u0, u1); }
             AFE_CUDA(cudaEventRecord(b->ev_k[c], b->stream));
             AFE_CUDA(cudaStreamWaitEvent(b->s_out, b->ev_k[c], 0));
             const size_t r0 = (size_t)b->frame_off[u0] * d.width, r1 = (size_t)b->frame_off[u1] * d.width;
-            AFE_CUDA(cudaMemcpyAsync(h_out + r0, b->d_out_stage + r0, (r1 - r0) * 4, cudaMemcpyDeviceToHost, b->s_out));
+            AFE_CUDA(cudaMemcpyAsync(h_out + r0, b->out_stage.p + r0, (r1 - r0) * 4, cudaMemcpyDeviceToHost, b->s_out));
         }
         AFE_CUDA(cudaStreamSynchronize(b->s_out));
         AFE_CUDA(cudaStreamSynchronize(b->stream));

@@ -26,9 +26,6 @@ struct FusedEngine {
     int cluster_probe[5] = {-1, -1, -1, -1, -1}; // max active clusters per cluster size (lazy; 0 = not schedulable)
 
     explicit FusedEngine(const Derived &dd, int dev);
-    ~FusedEngine();
-    FusedEngine(const FusedEngine &) = delete;
-    FusedEngine &operator=(const FusedEngine &) = delete;
 
     void set_window(const float *window, cudaStream_t st);
     void ensure_mel(float alpha);   // rebuilds the constant-bank tables when alpha changed (refresh_filters, mfcccpu.cpp:24-60)

@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <string>
+#include <utility>
 #include <vector>
 #include <stdexcept>
 
@@ -78,24 +79,71 @@ void build_dct(const Derived &d, std::vector<float> &dct);
 void build_mel_pairs(const Derived &d, const std::vector<int> &edges, const std::vector<float> &filters,
                      std::vector<float> &pairs /* [bins][2] */);
 
+// ---- owners of the library's CUDA resources. Each is move-only (declaring the move operations deletes the copies) and
+// releases its resource in its destructor, ignoring CUDA errors there like every release path of the library: a
+// destructor never throws.
+template <class T> struct DevBuf {
+    T *p = nullptr;
+    size_t n = 0;
+    DevBuf() = default;
+    DevBuf(DevBuf &&o) noexcept : p(std::exchange(o.p, nullptr)), n(std::exchange(o.n, 0)) {}
+    DevBuf &operator=(DevBuf &&o) noexcept { std::swap(p, o.p); std::swap(n, o.n); return *this; }
+    ~DevBuf() { release(); }
+    void alloc(size_t count) { release(); AFE_CUDA(cudaMalloc(&p, sizeof(T) * (count > 0 ? count : 1))); n = count; }
+    void upload(const std::vector<T> &h) // alloc + synchronous copy
+    {
+        alloc(h.size());
+        AFE_CUDA(cudaMemcpy(p, h.data(), sizeof(T) * h.size(), cudaMemcpyHostToDevice));
+    }
+    void release() { if (p) cudaFree(p); p = nullptr; n = 0; }
+};
+
+template <class T> struct PinnedBuf { // page-locked host memory
+    T *p = nullptr;
+    PinnedBuf() = default;
+    PinnedBuf(PinnedBuf &&o) noexcept : p(std::exchange(o.p, nullptr)) {}
+    PinnedBuf &operator=(PinnedBuf &&o) noexcept { std::swap(p, o.p); return *this; }
+    ~PinnedBuf() { release(); }
+    void alloc(size_t count) { release(); AFE_CUDA(cudaMallocHost(&p, sizeof(T) * (count > 0 ? count : 1))); }
+    void release() { if (p) cudaFreeHost(p); p = nullptr; }
+};
+
+struct Stream { // non-blocking stream; empty until create()
+    cudaStream_t h = nullptr;
+    Stream() = default;
+    Stream(Stream &&o) noexcept : h(std::exchange(o.h, nullptr)) {}
+    Stream &operator=(Stream &&o) noexcept { std::swap(h, o.h); return *this; }
+    ~Stream() { if (h) cudaStreamDestroy(h); }
+    void create() { AFE_CUDA(cudaStreamCreateWithFlags(&h, cudaStreamNonBlocking)); }
+    operator cudaStream_t() const { return h; }
+};
+
+struct Event { // event without timing; empty until create()
+    cudaEvent_t h = nullptr;
+    Event() = default;
+    Event(Event &&o) noexcept : h(std::exchange(o.h, nullptr)) {}
+    Event &operator=(Event &&o) noexcept { std::swap(h, o.h); return *this; }
+    ~Event() { if (h) cudaEventDestroy(h); }
+    void create() { AFE_CUDA(cudaEventCreateWithFlags(&h, cudaEventDisableTiming)); }
+    operator cudaEvent_t() const { return h; }
+};
+
 // ---- device-side constant tables for the in-register FFT (afe_fft.cuh)
 struct FftTables {
-    float2 *d_tw_a = nullptr;   // [R][16]   exp(-2 pi i n2 k1 / M)
-    float2 *d_tw_p = nullptr;   // [M/2]     exp(-2 pi i k / N2)
+    DevBuf<float2> d_tw_a;      // [R][16]   exp(-2 pi i n2 k1 / M)
+    DevBuf<float2> d_tw_p;      // [M/2]     exp(-2 pi i k / N2)
     int N2 = 0;
     void build(int N2);
-    void release();
 };
 
 // ---- kernels / launchers (afe_stages.cu)
 struct MelTables {              // device copies, rebuilt when alpha changes
-    int *d_edges = nullptr;     // [nb+2]
-    float *d_pairs = nullptr;   // [bins][2]
-    float *d_dct = nullptr;     // [nb][dct_len] (null when ceps_len == 0)
-    float *d_window = nullptr;  // [W]
-    float2 *d_window2 = nullptr; // [M] (w[2n], w[2n+1]) zero padded
+    DevBuf<int> d_edges;        // [nb+2]
+    DevBuf<float> d_pairs;      // [bins][2]
+    DevBuf<float> d_dct;        // [nb][dct_len] (null when ceps_len == 0)
+    DevBuf<float> d_window;     // [W]
+    DevBuf<float2> d_window2;   // [M] (w[2n], w[2n+1]) zero padded
     float alpha_built = -1.f;
-    void release();
 };
 void upload_mel_tables(const Derived &d, float alpha, MelTables &t, cudaStream_t st);
 void upload_window(const Derived &d, const float *window, MelTables &t, cudaStream_t st);
@@ -129,19 +177,6 @@ int kernel_launch_count();      // monotonically increasing count of kernel laun
 void count_launch(int n = 1);
 int sm_count_of(int device);    // cudaDevAttrMultiProcessorCount, cached per device
 
-template <class T> struct DevBuf {
-    T *p = nullptr;
-    size_t n = 0;
-    void alloc(size_t count)
-    {
-        release();
-        n = count;
-        AFE_CUDA(cudaMalloc(&p, sizeof(T) * (count > 0 ? count : 1)));
-    }
-    void release() { if (p) cudaFree(p); p = nullptr; n = 0; }
-    ~DevBuf() { release(); }
-};
-
 // ---- Normalizer state (NormalizerCPU / NormalizerOpenCL, normalizercpu.h:7-9): last statistics + a running record.
 // record layout (the one all-reduced across ranks): sum[dim] | sumsq[dim] | count | min[dim] | max[dim], doubles
 struct NormState {
@@ -163,6 +198,7 @@ struct NormState {
 // ---- the C-ABI Normalizer object (afe_stream.cu); afe_batch routes its corpus statistics through one of these
 struct afe_normalizer {
     int device = 0;
-    cudaStream_t own_st = nullptr, st = nullptr; // st: the stream in use (own, or the owning batch's)
+    afe::Stream own_st;
+    cudaStream_t st = nullptr; // the stream in use (own, or the owning batch's)
     afe::NormState ns;
 };

@@ -124,16 +124,16 @@ void launch_fft_mag(const Derived &d, const FftTables &ft, const MelTables &mt, 
         const int grid = std::min((frames + per_iter - 1) / per_iter, grid_cap(8));
         const bool pruned = d.W <= 26 * R;
         if (d.N2 == 512) {
-            if (pruned) k_fft_mag<512, 13><<<grid, 128, 0, st>>>(d_pcm, mt.d_window2, ft.d_tw_a, ft.d_tw_p, d_mag, frames, d.S, pre);
-            else k_fft_mag<512, 16><<<grid, 128, 0, st>>>(d_pcm, mt.d_window2, ft.d_tw_a, ft.d_tw_p, d_mag, frames, d.S, pre);
+            if (pruned) k_fft_mag<512, 13><<<grid, 128, 0, st>>>(d_pcm, mt.d_window2.p, ft.d_tw_a.p, ft.d_tw_p.p, d_mag, frames, d.S, pre);
+            else k_fft_mag<512, 16><<<grid, 128, 0, st>>>(d_pcm, mt.d_window2.p, ft.d_tw_a.p, ft.d_tw_p.p, d_mag, frames, d.S, pre);
         } else {
-            if (pruned) k_fft_mag<256, 13><<<grid, 128, 0, st>>>(d_pcm, mt.d_window2, ft.d_tw_a, ft.d_tw_p, d_mag, frames, d.S, pre);
-            else k_fft_mag<256, 16><<<grid, 128, 0, st>>>(d_pcm, mt.d_window2, ft.d_tw_a, ft.d_tw_p, d_mag, frames, d.S, pre);
+            if (pruned) k_fft_mag<256, 13><<<grid, 128, 0, st>>>(d_pcm, mt.d_window2.p, ft.d_tw_a.p, ft.d_tw_p.p, d_mag, frames, d.S, pre);
+            else k_fft_mag<256, 16><<<grid, 128, 0, st>>>(d_pcm, mt.d_window2.p, ft.d_tw_a.p, ft.d_tw_p.p, d_mag, frames, d.S, pre);
         }
     } else {
         if (d.N2 > 4096) throw Error("window_size above 4096 is not supported");
         const int threads = std::max(32, std::min(256, d.N2 / 2));
-        k_fft_mag_generic<<<std::min(frames, grid_cap(8)), threads, sizeof(float2) * 2 * d.N2, st>>>(d_pcm, mt.d_window, d_mag,
+        k_fft_mag_generic<<<std::min(frames, grid_cap(8)), threads, sizeof(float2) * 2 * d.N2, st>>>(d_pcm, mt.d_window.p, d_mag,
                                                                                                  frames, d.W, d.S, d.N2, pre);
     }
     AFE_CUDA(cudaGetLastError());
@@ -177,7 +177,7 @@ void launch_mel_dct(const Derived &d, const MelTables &mt, const float *d_mag, f
     const size_t sm = ((d.nb + 2) * 4 + 15) / 16 * 16 + (size_t)d.bins * 8 + (size_t)d.nb * dl * 4;
     if (sm > 200 * 1024) throw Error("mel/DCT tables do not fit in shared memory");
     AFE_CUDA(cudaFuncSetAttribute(k_mel_dct, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-    k_mel_dct<<<(frames + 63) / 64, 64, sm, st>>>(d_mag, mt.d_edges, reinterpret_cast<const float2 *>(mt.d_pairs), mt.d_dct,
+    k_mel_dct<<<(frames + 63) / 64, 64, sm, st>>>(d_mag, mt.d_edges.p, reinterpret_cast<const float2 *>(mt.d_pairs.p), mt.d_dct.p,
                                                   d_mel, d_cep, frames, d.bins, d.nb, dl);
     AFE_CUDA(cudaGetLastError());
     count_launch();

@@ -27,9 +27,8 @@ struct SegState {
     DevBuf<int16_t> buf[2];
     // pinned staging (two buffers, alternating) so that the H2D copy is asynchronous and the caller may reuse its buffer
     // at once; a buffer is reused only after the copy that read it has completed (event), which by then it normally has
-    int16_t *h_pin[2] = {nullptr, nullptr};
+    PinnedBuf<int16_t> h_pin[2];
     bool pin_busy[2] = {false, false}; // an H2D copy out of this staging buffer may still be running; cleared by synced()
-    size_t pin_cap = 0;
     int cur = 0, pin = 0;
     bool carry_pending = false; // the tail of buf[cur] still has to move to the front of buf[cur ^ 1] (done by the next set_input;
                                 // flush() reads the tail where it lies, so a single-block stream never copies it)
@@ -44,18 +43,7 @@ struct SegState {
             b.alloc(cap + N2 + 16);                          // + slack: the FFT kernel reads whole N2-sample words
             AFE_CUDA(cudaMemset(b.p, 0, sizeof(int16_t) * (cap + N2 + 16)));
         }
-        pin_cap = cap;
-        for (int i = 0; i < 2; i++) {
-            AFE_CUDA(cudaMallocHost(&h_pin[i], sizeof(int16_t) * std::max<size_t>(pin_cap, 1)));
-        }
-    }
-    void release()
-    {
-        buf[0].release(); buf[1].release();
-        for (int i = 0; i < 2; i++) {
-            if (h_pin[i]) cudaFreeHost(h_pin[i]);
-            h_pin[i] = nullptr;
-        }
+        for (auto &h : h_pin) h.alloc(cap);
     }
     void reset() { remaining = samples = 0; flushed = true; last_calc_flushed = false; carry_pending = false; }
     void synced() { pin_busy[0] = pin_busy[1] = false; } // the owner synchronised the stream: every staged copy has landed
@@ -86,15 +74,15 @@ struct SegState {
         last_calc_flushed = flushed;
         pin ^= 1;
         if (pin_busy[pin]) { AFE_CUDA(cudaStreamSynchronize(st)); synced(); } // rare: two blocks without a get_output between
-        memcpy(h_pin[pin], in, sizeof(int16_t) * n);
+        memcpy(h_pin[pin].p, in, sizeof(int16_t) * n);
         pin_busy[pin] = true;
         if (flushed) {
-            AFE_CUDA(cudaMemcpyAsync(dst, h_pin[pin], sizeof(int16_t) * n, cudaMemcpyHostToDevice, st));
+            AFE_CUDA(cudaMemcpyAsync(dst, h_pin[pin].p, sizeof(int16_t) * n, cudaMemcpyHostToDevice, st));
             const int used = (wc - D) * S + W - S;
             remaining = total - used + W - S;
             flushed = false;
         } else {                                             // append to the carry-over (segmentercpu.cpp:76-93)
-            AFE_CUDA(cudaMemcpyAsync(dst + remaining, h_pin[pin], sizeof(int16_t) * n, cudaMemcpyHostToDevice, st));
+            AFE_CUDA(cudaMemcpyAsync(dst + remaining, h_pin[pin].p, sizeof(int16_t) * n, cudaMemcpyHostToDevice, st));
             total = n + remaining;
             wc_nd = est(total);
             wc = wc_nd - 2 * D;
@@ -124,13 +112,13 @@ struct SegState {
 struct afe_mfcc {
     Derived d;
     int device;
-    cudaStream_t st = nullptr;
+    Stream st;
     SegState seg;
     float alpha = 1.f, pre = 0.f;
     bool window_set = false, last_block = false, fix_q1 = false;
     std::vector<float> window;
     DevBuf<float> outb;
-    float *h_out = nullptr; size_t h_out_cap = 0;
+    PinnedBuf<float> h_out;
     // ---- fused route: every block is ONE launch of K1
     std::unique_ptr<FusedEngine> eng;
     const int16_t *blk_pcm = nullptr;   // device PCM of the current block (carry-over + new samples)
@@ -186,11 +174,11 @@ int afe_mfcc_create(const afe_params *p, int cuda_device, afe_mfcc **out)
     *out = nullptr;
     return guarded([&] {
         if (afe_device_count() <= cuda_device) throw Error("no usable CUDA device " + std::to_string(cuda_device) + " (the product has no CPU fallback)");
+        DeviceGuard g(cuda_device);
         std::unique_ptr<afe_mfcc> h(new afe_mfcc(*p, cuda_device));
         const Derived &d = h->d;
         if (d.in_frames_cap < 1) throw Error("input_buffer_size is smaller than one window");
-        DeviceGuard g(cuda_device);
-        AFE_CUDA(cudaStreamCreateWithFlags(&h->st, cudaStreamNonBlocking));
+        h->st.create();
         h->seg.init(d.W, d.S, d.frame_cap, d.D);
         const size_t fc = d.frame_cap;
         // K1 covers the block when the parameter set fits it and normalisation (if any) comes after the deltas: normalising
@@ -209,8 +197,7 @@ int afe_mfcc_create(const afe_params *p, int cuda_device, afe_mfcc **out)
         } else
             alloc_staged(h.get());
         h->outb.alloc((fc + d.D) * d.width);
-        h->h_out_cap = (fc + d.D) * d.width;
-        AFE_CUDA(cudaMallocHost(&h->h_out, sizeof(float) * h->h_out_cap));
+        h->h_out.alloc((fc + d.D) * d.width);
         *out = h.release();
     });
 }
@@ -220,10 +207,6 @@ void afe_mfcc_destroy(afe_mfcc *h)
     if (!h) return;
     cudaSetDevice(h->device);
     cudaStreamSynchronize(h->st);
-    h->eng.reset();
-    h->fft.release(); h->mel.release(); h->seg.release();
-    if (h->h_out) cudaFreeHost(h->h_out);
-    cudaStreamDestroy(h->st);
     delete h;
 }
 
@@ -434,20 +417,20 @@ int afe_mfcc_get_output(afe_mfcc *h, float *out, int frames)
             if (frames > d.D) throw Error("Window count too high");
             const size_t off = (size_t)h->spec_row0 * d.width;
             if (!h->spec_on_host) {
-                AFE_CUDA(cudaMemcpyAsync(h->h_out + off, h->outb.p + off, sizeof(float) * d.D * d.width, cudaMemcpyDeviceToHost, h->st));
+                AFE_CUDA(cudaMemcpyAsync(h->h_out.p + off, h->outb.p + off, sizeof(float) * d.D * d.width, cudaMemcpyDeviceToHost, h->st));
                 AFE_CUDA(cudaStreamSynchronize(h->st));
                 h->pending = false; h->seg.synced(); h->spec_on_host = true;
             }
-            memcpy(out, h->h_out + off, sizeof(float) * n);
+            memcpy(out, h->h_out.p + off, sizeof(float) * n);
             return;
         }
         // the speculative flush rows sit right behind the block's rows: one copy fetches both
         const bool with_spec = h->spec_valid && frames == h->spec_row0;
         const size_t n_copy = n + (with_spec ? (size_t)d.D * d.width : 0);
-        AFE_CUDA(cudaMemcpyAsync(h->h_out, h->outb.p, sizeof(float) * n_copy, cudaMemcpyDeviceToHost, h->st));
+        AFE_CUDA(cudaMemcpyAsync(h->h_out.p, h->outb.p, sizeof(float) * n_copy, cudaMemcpyDeviceToHost, h->st));
         AFE_CUDA(cudaStreamSynchronize(h->st));
         h->pending = false; h->seg.synced(); h->spec_on_host = with_spec;
-        memcpy(out, h->h_out, sizeof(float) * n);
+        memcpy(out, h->h_out.p, sizeof(float) * n);
     });
 }
 
@@ -456,14 +439,14 @@ int afe_mfcc_get_output(afe_mfcc *h, float *out, int frames)
 // ================================================================================================== stage objects
 struct afe_segmenter {
     int device;
-    cudaStream_t st = nullptr;
+    Stream st;
     SegState seg;
     DevBuf<float> window;
     bool window_set = false;
 };
 struct afe_delta {
     int device, dim, window_limit, L;
-    cudaStream_t st = nullptr;
+    Stream st;
     DevBuf<float> out;
 };
 
@@ -474,10 +457,10 @@ int afe_segmenter_create(int W, int S, int window_limit, int deltasize, int cuda
     *out = nullptr;
     return guarded([&] {
         if (afe_device_count() <= cuda_device) throw Error("no usable CUDA device (the product has no CPU fallback)");
+        DeviceGuard g(cuda_device);
         std::unique_ptr<afe_segmenter> s(new afe_segmenter());
         s->device = cuda_device;
-        DeviceGuard g(cuda_device);
-        AFE_CUDA(cudaStreamCreateWithFlags(&s->st, cudaStreamNonBlocking));
+        s->st.create();
         s->seg.init(W, S, window_limit, deltasize);
         s->window.alloc(W);
         *out = s.release();
@@ -488,8 +471,6 @@ void afe_segmenter_destroy(afe_segmenter *s)
     if (!s) return;
     cudaSetDevice(s->device);
     cudaStreamSynchronize(s->st);
-    s->seg.release();
-    cudaStreamDestroy(s->st);
     delete s;
 }
 int afe_segmenter_set_window(afe_segmenter *s, const float *w)
@@ -538,10 +519,10 @@ int afe_delta_create(int dim, int window_limit, int delta_size, int cuda_device,
     *out = nullptr;
     return guarded([&] {
         if (afe_device_count() <= cuda_device) throw Error("no usable CUDA device (the product has no CPU fallback)");
+        DeviceGuard g(cuda_device);
         std::unique_ptr<afe_delta> d(new afe_delta());
         d->device = cuda_device; d->dim = dim; d->window_limit = window_limit; d->L = delta_size;
-        DeviceGuard g(cuda_device);
-        AFE_CUDA(cudaStreamCreateWithFlags(&d->st, cudaStreamNonBlocking));
+        d->st.create();
         d->out.alloc((size_t)dim * window_limit);
         *out = d.release();
     });
@@ -551,7 +532,6 @@ void afe_delta_destroy(afe_delta *d)
     if (!d) return;
     cudaSetDevice(d->device);
     cudaStreamSynchronize(d->st);
-    cudaStreamDestroy(d->st);
     delete d;
 }
 int afe_delta_apply(afe_delta *d, const float *d_data, int window_count)
@@ -571,10 +551,10 @@ int afe_normalizer_create(int norm_type, int dim, int cuda_device, afe_normalize
     return guarded([&] {
         if (afe_device_count() <= cuda_device) throw Error("no usable CUDA device (the product has no CPU fallback)");
         if (norm_type < AFE_NORM_NONE || norm_type > AFE_NORM_MINMAX || dim < 1) throw Error("invalid normalizer arguments");
+        DeviceGuard g(cuda_device);
         std::unique_ptr<afe_normalizer> n(new afe_normalizer());
         n->device = cuda_device;
-        DeviceGuard g(cuda_device);
-        AFE_CUDA(cudaStreamCreateWithFlags(&n->own_st, cudaStreamNonBlocking));
+        n->own_st.create();
         n->st = n->own_st;
         n->ns.init(norm_type, dim);
         n->ns.reset_record(n->st);
@@ -586,7 +566,6 @@ void afe_normalizer_destroy(afe_normalizer *n)
     if (!n) return;
     cudaSetDevice(n->device);
     cudaStreamSynchronize(n->own_st);
-    cudaStreamDestroy(n->own_st);
     delete n;
 }
 static cudaStream_t norm_stream(afe_normalizer *n) { return n->st ? n->st : n->own_st; }
