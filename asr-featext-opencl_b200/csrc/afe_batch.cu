@@ -226,10 +226,10 @@ void FusedEngine::ensure_mel(float alpha)
 }
 std::string FusedEngine::kernel_label() const
 {
-    const int kf = (d.nb + 7) / 8;
+    const int k = launch_key();
     char buf[96];
-    snprintf(buf, sizeof buf, "k_fused_mfcc<%d,%d,8,%d,%s>", d.N2, pruned ? 13 : 16, kf <= 3 ? 3 : kf <= 5 ? 5 : 8,
-             pre != 0.f ? "true" : "false");
+    snprintf(buf, sizeof buf, "k_fused_mfcc<%d,%d,8,%d,%s>", k % 12 < 6 ? 512 : 256, k % 6 < 3 ? 13 : 16,
+             k % 3 == 0 ? 3 : k % 3 == 1 ? 5 : 8, k >= 12 ? "true" : "false");
     return buf;
 }
 
@@ -277,15 +277,16 @@ int FusedEngine::plan_rows(std::vector<Tile> &tiles, long long pcm_off, long lon
     return count;
 }
 
-FusedArgs FusedEngine::base_args(int q1, bool use_tma) const
+FusedArgs FusedEngine::base_args(int q1, const int16_t *pcm, bool tma_ok) const
 {
     FusedArgs a{};
+    a.pcm = pcm;
+    a.use_tma = tma_ok && d.S % 8 == 0 && (reinterpret_cast<uintptr_t>(pcm) & 15) == 0 ? 1 : 0;
     a.window2 = mel.d_window2.p; a.tw_a = fft.d_tw_a.p; a.tw_p = fft.d_tw_p.p;
     a.norm_type = d.p.norm; a.norm_after_dyn = d.p.norm_after_dyn;
     a.W = d.W; a.S = d.S; a.nb = d.nb; a.dct_len = d.C > 0 ? d.dct_len : 0; a.cols = d.cols; a.width = d.width;
     a.l1 = d.l1; a.l2 = d.l2; a.nstreams = d.width / d.cols;
     a.q1 = d.D > 0 ? q1 : 0;
-    a.use_tma = use_tma ? 1 : 0;
     a.tc_max = tc_max;
     a.pre = pre;
     float den1 = 0, den2 = 0;
@@ -316,12 +317,42 @@ void FusedEngine::launch(const FusedArgs &a, int grid, int cluster, cudaStream_t
 {
     if (!window_set) throw Error("set_window must be called before running");
     FusedLaunch fl{a, L, &mc, grid, cluster, st};
-    const cudaError_t e = launch_fused_variant(key + (a.pre != 0.f ? 12 : 0), fl);
+    const cudaError_t e = launch_fused_variant(launch_key(), fl);
     if (e != cudaSuccess) {
         cudaGetLastError();
         throw Error(std::string("CUDA error: ") + cudaGetErrorString(e) + " at k_fused_mfcc launch" + (cluster > 0 ? " (clustered)" : ""));
     }
     count_launch();
+}
+
+void FusedNormState::alloc(int n_groups, size_t n_tiles, int width)
+{
+    partials.alloc(4 * (size_t)width * n_tiles);
+    counters.alloc(n_groups + 1); flags.alloc(n_groups);
+    AFE_CUDA(cudaMemset(counters.p, 0, sizeof(int) * (n_groups + 1)));
+    AFE_CUDA(cudaMemset(flags.p, 0, sizeof(unsigned) * n_groups));
+    epoch = 0;
+    mean.alloc((size_t)width * n_groups); scale.alloc((size_t)width * n_groups);
+}
+
+void FusedEngine::launch_roles(FusedArgs a, int ntiles, FusedNormState &ns, cudaStream_t st)
+{
+    a.counters = ns.counters.p; a.work_counter = ns.counters.p + ns.counters.n - 1;
+    a.flags = ns.flags.p; a.epoch = ++ns.epoch; a.ntiles_launch = ntiles;
+    a.g_mean = ns.mean.p; a.g_scale = ns.scale.p;
+    launch(a, ntiles + std::min(ntiles, 2 * sm_count), 0, st);
+}
+
+void FusedEngine::launch_clustered(FusedArgs a, int grid, int cluster, FusedNormState &ns, cudaStream_t st)
+{
+    a.cluster_norm = 1;
+    try {
+        launch(a, grid, cluster, st);
+    } catch (const Error &) {
+        cluster_probe[cluster] = 0; // the clustered launch was refused (nothing ran): no more tries at this size
+        a.cluster_norm = 0;
+        launch_ticket(a, grid, ns, st);
+    }
 }
 
 } // namespace afe
@@ -342,30 +373,26 @@ struct afe_batch {
     std::unique_ptr<FusedEngine> eng;
     float alpha = 1.f;
     int scope = AFE_STATS_REFERENCE_BLOCK, flags = 0;
-    // plan
-    int n_utts = 0, n_tiles = 0, n_groups = 0;
-    bool aligned = false;
-    std::vector<int64_t> sample_off, sample_len, frame_off;
-    std::vector<int> h_tile_begin;          // [n_utts+1] first tile of every utterance
-    int64_t pcm_extent = 0;
-    struct Plan {                           // the device side of a plan, replaced as a whole by afe_batch_plan
+    struct Plan {                           // everything afe_batch_plan derives, replaced as a whole by it
+        int n_utts = 0, n_tiles = 0, n_groups = 0;
+        bool aligned = false;               // every utterance starts on a 16-byte boundary
+        std::vector<int64_t> sample_off, sample_len, frame_off;
+        std::vector<int> h_tile_begin;      // [n_utts+1] first tile of every utterance
+        int64_t pcm_extent = 0;
+        int corpus_blocks = 0;              // level-1 blocks of the corpus reduction (2 per SM)
+        int max_tiles_per_utt = 0;
         DevBuf<Tile> tiles;
         DevBuf<int> tile_begin, scratch_begin;
-        DevBuf<double> counts, partials, scratch;
+        DevBuf<double> counts, scratch;
         DevBuf<double> group_stats;         // per-utterance scopes: the statistics records
-        DevBuf<int> counters;               // [n_groups] arrival tickets + [1] role tickets of the long-utterance scheme
-        DevBuf<unsigned> flags;             // [n_groups]
-        DevBuf<float> mean, scale;
+        FusedNormState norm;                // also K2's partials and K3's mean / scale
         std::unique_ptr<afe_normalizer, NormalizerDestroy> cnorm; // corpus scope: the Normalizer that owns the record
         double *stats() const { return cnorm ? cnorm->ns.rec.p : group_stats.p; } // [n_groups][4 * width + 1]
     } plan;
-    unsigned epoch = 0;
-    int corpus_blocks = 0;          // level-1 blocks of the corpus reduction (2 per SM)
-    int max_tiles_per_utt = 0;
     // One tile normalising its whole utterance is right for short utterances and a serial bottleneck for long ones:
     // up to 8 tiles -> clusters / ticket scheme; more -> the role scheme (normaliser CTAs, one per tile, same launch).
     bool fuse_norm() const { return !(flags & AFE_BATCH_UNFUSED_NORM); }
-    bool long_scheme() const { return max_tiles_per_utt > 8; }
+    bool long_scheme() const { return plan.max_tiles_per_utt > 8; }
     int last_launches = 0;
     // device staging for run_host (grow-only)
     DevBuf<int16_t> pcm_stage;
@@ -373,20 +400,6 @@ struct afe_batch {
 
     explicit afe_batch(const afe_params &p, int dev) : d(p), device(dev) {}
 };
-
-static FusedArgs make_fused_args(afe_batch *b, const int16_t *d_pcm, float *d_out, bool want_stats, int t0)
-{
-    const Derived &d = b->d;
-    const bool tma = b->aligned && !(b->flags & AFE_BATCH_NO_TMA) && (reinterpret_cast<uintptr_t>(d_pcm) & 15) == 0;
-    FusedArgs a = b->eng->base_args((b->flags & AFE_BATCH_Q1_EXACT) ? 1 : 0, tma);
-    a.pcm = d_pcm; a.out = d_out; a.tiles = b->plan.tiles.p; a.tile_base = t0;
-    a.partials = want_stats ? b->plan.partials.p : nullptr;
-    if (!want_stats) a.stats_rows_mode = 0;
-    else if (!d.p.norm_after_dyn) a.stats_rows_mode = 2;
-    else a.stats_rows_mode = b->scope == AFE_STATS_REFERENCE_BLOCK ? 1 : 2;
-    a.stats_kind = !want_stats ? 0 : (d.p.norm == AFE_NORM_CMN ? 1 : d.p.norm == AFE_NORM_CVN ? 2 : 3);
-    return a;
-}
 
 // Tiles [t0, t1) (whole utterances) through K1. With fused normalisation:
 //  * the default regression and utterances of 1..4 tiles: runs of equal tile count become ONE clustered launch each
@@ -397,73 +410,60 @@ constexpr int kMaxClusterRuns = 8;
 constexpr int kMaxClusterTiles = 4; // utterances of up to 4 tiles (~20 s) form a cluster; longer ones keep the ticket scheme
 static void run_extract(afe_batch *b, const int16_t *d_pcm, float *d_out, int t0 = 0, int t1 = -1, bool fuse_norm = false)
 {
-    if (t1 < 0) t1 = b->n_tiles;
+    afe_batch::Plan &pl = b->plan;
+    if (!pl.tiles.p) throw Error("afe_batch_plan must be called before running");
+    if (t1 < 0) t1 = pl.n_tiles;
     if (t1 <= t0) return;
-    if (!b->plan.tiles.p) throw Error("afe_batch_plan must be called before running");
     FusedEngine &eng = *b->eng;
     eng.ensure_mel(b->alpha);
     const Derived &d = b->d;
     const bool want_stats = d.p.norm != AFE_NORM_NONE;
-    FusedArgs a = make_fused_args(b, d_pcm, d_out, want_stats, t0);
-    auto launch = [&](const FusedArgs &args, int grid, int cluster) { eng.launch(args, grid, cluster, b->stream); b->last_launches++; };
-    if (!(fuse_norm && want_stats)) { launch(a, t1 - t0, 0); return; }
-    if (b->long_scheme()) {
-        a.counters = b->plan.counters.p; a.work_counter = b->plan.counters.p + b->n_groups;
-        a.flags = b->plan.flags.p; a.epoch = ++b->epoch; a.ntiles_launch = t1 - t0;
-        a.g_mean = b->plan.mean.p; a.g_scale = b->plan.scale.p;
-        launch(a, (t1 - t0) + std::min(t1 - t0, 2 * eng.sm_count), 0); // + one wave of normaliser roles
-        return;
-    }
-    const bool cluster_ok = !(b->flags & AFE_BATCH_NO_CLUSTER) && d.width == 3 * d.cols && d.l1 == 3 && d.l2 == 3;
-    if (cluster_ok) {
+    FusedArgs a = eng.base_args((b->flags & AFE_BATCH_Q1_EXACT) ? 1 : 0, d_pcm, pl.aligned && !(b->flags & AFE_BATCH_NO_TMA));
+    a.out = d_out; a.tiles = pl.tiles.p; a.tile_base = t0;
+    if (want_stats) eng.set_stats(a, pl.norm, d.p.norm_after_dyn && b->scope == AFE_STATS_REFERENCE_BLOCK ? 1 : 2);
+    if (!(fuse_norm && want_stats)) { eng.launch_plain(a, t1 - t0, b->stream); b->last_launches++; return; }
+    if (b->long_scheme()) { eng.launch_roles(a, t1 - t0, pl.norm, b->stream); b->last_launches++; return; }
+    if (!(b->flags & AFE_BATCH_NO_CLUSTER) && eng.default_regression()) {
         struct Run { int t0, t1, cluster; };
         std::vector<Run> runs;
-        const int u0 = (int)(std::lower_bound(b->h_tile_begin.begin(), b->h_tile_begin.end(), t0) - b->h_tile_begin.begin());
+        const std::vector<int> &tb = pl.h_tile_begin;
+        const int u0 = (int)(std::lower_bound(tb.begin(), tb.end(), t0) - tb.begin());
         bool schedulable = true;
-        for (int u = u0; u < b->n_utts && b->h_tile_begin[u] < t1 && (int)runs.size() <= kMaxClusterRuns; u++) {
-            const int nt = b->h_tile_begin[u + 1] - b->h_tile_begin[u], cl = nt <= kMaxClusterTiles ? nt : 0;
+        for (int u = u0; u < pl.n_utts && tb[u] < t1 && (int)runs.size() <= kMaxClusterRuns; u++) {
+            const int nt = tb[u + 1] - tb[u], cl = nt <= kMaxClusterTiles ? nt : 0;
             if (cl > 0 && !eng.cluster_schedulable(cl, a, b->stream)) { schedulable = false; break; }
-            if (!runs.empty() && runs.back().cluster == cl) runs.back().t1 = b->h_tile_begin[u + 1];
-            else runs.push_back({b->h_tile_begin[u], b->h_tile_begin[u + 1], cl});
+            if (!runs.empty() && runs.back().cluster == cl) runs.back().t1 = tb[u + 1];
+            else runs.push_back({tb[u], tb[u + 1], cl});
         }
         if (schedulable && (int)runs.size() <= kMaxClusterRuns && !runs.empty() && runs.front().t0 == t0 && runs.back().t1 == t1) {
             for (const Run &r : runs) {
-                FusedArgs ar = a;
-                ar.tile_base = r.t0;
-                if (r.cluster > 0) { ar.cluster_norm = 1; ar.counters = nullptr; }
-                else ar.counters = b->plan.counters.p;
-                try {
-                    launch(ar, r.t1 - r.t0, r.cluster);
-                } catch (const Error &) {
-                    if (r.cluster == 0) throw;
-                    // the clustered launch was refused (nothing ran): this run takes the ticket scheme instead
-                    eng.cluster_probe[r.cluster] = 0;
-                    ar.cluster_norm = 0; ar.counters = b->plan.counters.p;
-                    launch(ar, r.t1 - r.t0, 0);
-                }
+                a.tile_base = r.t0;
+                if (r.cluster > 0) eng.launch_clustered(a, r.t1 - r.t0, r.cluster, pl.norm, b->stream);
+                else eng.launch_ticket(a, r.t1 - r.t0, pl.norm, b->stream);
+                b->last_launches++;
             }
             return;
         }
     }
-    a.counters = b->plan.counters.p;
-    launch(a, t1 - t0, 0);
+    eng.launch_ticket(a, t1 - t0, pl.norm, b->stream);
+    b->last_launches++;
 }
 
 static void run_reduce(afe_batch *b, int g0 = 0, int g1 = -1)
 {
-    if (g1 < 0) g1 = b->n_groups;
+    const afe_batch::Plan &pl = b->plan;
+    if (g1 < 0) g1 = pl.n_groups;
     if (g1 <= g0) return;
     const int w = b->d.width;
-    const afe_batch::Plan &pl = b->plan;
-    if (b->scope == AFE_STATS_CORPUS && b->n_tiles > 2 * b->corpus_blocks) {
-        k_reduce_partials_level1<<<b->corpus_blocks, 128, 0, b->stream>>>(pl.partials.p, b->n_tiles, w, pl.scratch.p);
+    if (b->scope == AFE_STATS_CORPUS && pl.n_tiles > 2 * pl.corpus_blocks) {
+        k_reduce_partials_level1<<<pl.corpus_blocks, 128, 0, b->stream>>>(pl.norm.partials.p, pl.n_tiles, w, pl.scratch.p);
         AFE_CUDA(cudaGetLastError());
         k_reduce_partials<<<1, 256, dev::kSegs * w * 4 * sizeof(double), b->stream>>>(pl.scratch.p, pl.scratch_begin.p, pl.counts.p, w, pl.stats());
         AFE_CUDA(cudaGetLastError());
         count_launch(2); b->last_launches += 2;
         return;
     }
-    k_reduce_partials<<<g1 - g0, 256, dev::kSegs * w * 4 * sizeof(double), b->stream>>>(pl.partials.p, pl.tile_begin.p + g0, pl.counts.p + g0, w,
+    k_reduce_partials<<<g1 - g0, 256, dev::kSegs * w * 4 * sizeof(double), b->stream>>>(pl.norm.partials.p, pl.tile_begin.p + g0, pl.counts.p + g0, w,
                                                                                        pl.stats() + (size_t)g0 * (4 * w + 1));
     AFE_CUDA(cudaGetLastError());
     count_launch(); b->last_launches++;
@@ -472,17 +472,17 @@ static void run_reduce(afe_batch *b, int g0 = 0, int g1 = -1)
 static void run_normalize(afe_batch *b, float *d_out, int t0 = 0, int t1 = -1, int g0 = 0, int g1 = -1)
 {
     const Derived &d = b->d;
-    if (t1 < 0) t1 = b->n_tiles;
-    if (g1 < 0) g1 = b->n_groups;
+    const afe_batch::Plan &pl = b->plan;
+    if (t1 < 0) t1 = pl.n_tiles;
+    if (g1 < 0) g1 = pl.n_groups;
     if (t1 <= t0 || g1 <= g0) return;
     const size_t w = d.width;
-    const afe_batch::Plan &pl = b->plan;
     k_finalize_stats<<<g1 - g0, 128, 0, b->stream>>>(pl.stats() + (size_t)g0 * (4 * w + 1), d.width, d.cols, d.p.norm,
-                                                      d.p.norm_after_dyn, pl.mean.p + g0 * w, pl.scale.p + g0 * w);
+                                                      d.p.norm_after_dyn, pl.norm.mean.p + g0 * w, pl.norm.scale.p + g0 * w);
     AFE_CUDA(cudaGetLastError());
     // Tile::group is absolute, so mean / scale keep their base
     k_normalize_tiles<<<t1 - t0, 256, 2 * d.width * sizeof(float), b->stream>>>(d_out, pl.tiles.p + t0, d.width, d.p.norm,
-                                                                              pl.mean.p, pl.scale.p);
+                                                                              pl.norm.mean.p, pl.norm.scale.p);
     AFE_CUDA(cudaGetLastError());
     count_launch(2); b->last_launches += 2;
 }
@@ -591,20 +591,19 @@ static int plan_impl(afe_batch *b, const int64_t *off, const int64_t *len, const
         DeviceGuard g(b->device);
         b->plan = {};
         const FusedEngine &eng = *b->eng;
-        b->n_utts = n_utts;
-        b->sample_off.assign(off, off + n_utts);
-        b->sample_len.assign(len, len + n_utts);
-        b->h_tile_begin.assign(n_utts + 1, 0);
-        b->max_tiles_per_utt = 0;
-        b->pcm_extent = 0;
-        b->frame_off.assign(n_utts + 1, 0);
+        // built aside and installed whole, so that a plan that fails here leaves the batch unplanned
+        afe_batch::Plan pl;
+        pl.n_utts = n_utts;
+        pl.sample_off.assign(off, off + n_utts);
+        pl.sample_len.assign(len, len + n_utts);
+        pl.h_tile_begin.assign(n_utts + 1, 0);
+        pl.frame_off.assign(n_utts + 1, 0);
         std::vector<Tile> tiles;
-        std::vector<int> tile_begin;
         std::vector<double> counts;
         const bool corpus = b->scope == AFE_STATS_CORPUS;
         if (seg_first && d.p.norm != AFE_NORM_NONE && !corpus)
             throw Error("plan_segments: normalisation over segments needs the CORPUS statistics scope");
-        bool aligned = d.S % 8 == 0;
+        pl.aligned = true;
         double corpus_count = 0;
         // Wave balancing for small batches (a single long stream, a handful of files): with fewer than ~8 waves of CTAs the
         // tail of a partly filled last wave costs a whole tile time, so pick the tile size for which
@@ -633,67 +632,55 @@ static int plan_impl(afe_batch *b, const int64_t *off, const int64_t *len, const
         for (int u = 0; u < n_utts; u++) {
             const int64_t n = len[u];
             if (n < 0 || n > 0x7fffffff || off[u] < 0) throw Error("plan: invalid utterance offset/length");
-            b->pcm_extent = std::max<int64_t>(b->pcm_extent, off[u] + n);
+            pl.pcm_extent = std::max<int64_t>(pl.pcm_extent, off[u] + n);
             if (off[u] % 2) throw Error("plan: utterance offsets must be even (32-bit PCM word loads)");
-            if (off[u] % 8) aligned = false;
+            if (off[u] % 8) pl.aligned = false;
             // parambase.cpp:16-19 evaluates in float32, which is inexact above 2^24 samples: never let it exceed the
             // exact count (the extra frame would lie outside the utterance)
             const int T = std::min(afe_estimated_window_count((int)n, d.W, d.S), (int)std::max<int64_t>(0, (n - (d.W - d.S)) / d.S));
             if (T <= 2 * d.D || T < 1) throw Error("Can't process data, window count is too small"); // segmentercpu.cpp:65-66
             const int t_first = seg_first ? seg_first[u] : 0, rows = seg_rows ? seg_rows[u] : T;
             if (t_first < 0 || rows < 1 || t_first + rows > T) throw Error("plan_segments: segment outside its frames");
-            b->frame_off[u + 1] = b->frame_off[u] + rows;
-            b->h_tile_begin[u] = (int)tiles.size();
-            if (!corpus) tile_begin.push_back((int)tiles.size());
-            const int ntile = eng.plan_rows(tiles, off[u], b->frame_off[u] - t_first, T, t_first, rows, corpus ? 0 : u, nout_cap);
-            b->max_tiles_per_utt = std::max(b->max_tiles_per_utt, ntile);
+            pl.frame_off[u + 1] = pl.frame_off[u] + rows;
+            pl.h_tile_begin[u] = (int)tiles.size();
+            const int ntile = eng.plan_rows(tiles, off[u], pl.frame_off[u] - t_first, T, t_first, rows, corpus ? 0 : u, nout_cap);
+            pl.max_tiles_per_utt = std::max(pl.max_tiles_per_utt, ntile);
             const double cnt = seg_first ? rows : !d.p.norm_after_dyn ? T : (b->scope == AFE_STATS_REFERENCE_BLOCK ? T - d.D : T);
             if (corpus) corpus_count += cnt; else counts.push_back(cnt);
         }
-        if (corpus) { tile_begin.push_back(0); counts.push_back(corpus_count); }
-        tile_begin.push_back((int)tiles.size());
-        b->h_tile_begin[n_utts] = (int)tiles.size();
-        b->aligned = aligned;
-        b->n_tiles = (int)tiles.size();
-        b->n_groups = corpus ? 1 : n_utts;
-        b->corpus_blocks = 2 * eng.sm_count;
-        // built aside and installed whole, so that a plan that fails here leaves the batch unplanned
-        afe_batch::Plan pl;
+        if (corpus) counts.push_back(corpus_count);
+        pl.h_tile_begin[n_utts] = (int)tiles.size();
+        pl.n_tiles = (int)tiles.size();
+        pl.n_groups = corpus ? 1 : n_utts;
+        pl.corpus_blocks = 2 * eng.sm_count;
         pl.tiles.upload(tiles);
         if (d.p.norm != AFE_NORM_NONE) {
             const size_t w = d.width;
-            pl.tile_begin.upload(tile_begin);
+            pl.tile_begin.upload(corpus ? std::vector<int>{0, pl.n_tiles} : pl.h_tile_begin); // first tile of every group
             pl.counts.upload(counts);
-            pl.partials.alloc(4 * w * tiles.size());
+            pl.norm.alloc(pl.n_groups, tiles.size(), d.width);
             if (corpus) {
                 // the corpus record lives in a Normalizer of dim = width (all three streams in one record)
                 afe_normalizer *n = nullptr;
                 if (afe_normalizer_create(d.p.norm, d.width, b->device, &n) != 0) throw Error(afe_last_error());
                 pl.cnorm.reset(n);
                 n->st = b->stream;
-                pl.scratch.alloc(4 * w * b->corpus_blocks);
-                pl.scratch_begin.upload({0, b->corpus_blocks});
+                pl.scratch.alloc(4 * w * pl.corpus_blocks);
+                pl.scratch_begin.upload({0, pl.corpus_blocks});
             } else
-                pl.group_stats.alloc((4 * w + 1) * b->n_groups);
-            pl.counters.alloc(b->n_groups + 1);
-            AFE_CUDA(cudaMemset(pl.counters.p, 0, sizeof(int) * (b->n_groups + 1)));
-            pl.flags.alloc(b->n_groups);
-            AFE_CUDA(cudaMemset(pl.flags.p, 0, sizeof(unsigned) * b->n_groups));
-            b->epoch = 0;
-            pl.mean.alloc(w * b->n_groups);
-            pl.scale.alloc(w * b->n_groups);
+                pl.group_stats.alloc((4 * w + 1) * pl.n_groups);
         }
+        if (total_frames) *total_frames = pl.frame_off[n_utts];
         b->plan = std::move(pl);
-        if (total_frames) *total_frames = b->frame_off[n_utts];
     });
 }
 
 int afe_batch_frame_offsets(const afe_batch *b, int64_t *fo)
 {
-    memcpy(fo, b->frame_off.data(), sizeof(int64_t) * b->frame_off.size());
+    memcpy(fo, b->plan.frame_off.data(), sizeof(int64_t) * b->plan.frame_off.size());
     return 0;
 }
-int afe_batch_num_tiles(const afe_batch *b) { return b->n_tiles; }
+int afe_batch_num_tiles(const afe_batch *b) { return b->plan.n_tiles; }
 int afe_batch_kernel_launches(const afe_batch *b) { return b->last_launches; }
 const char *afe_batch_kernel_name(const afe_batch *b)
 {
@@ -728,7 +715,7 @@ int afe_batch_corpus_stats(afe_batch *b, double **d_stats, int *stats_len)
         if (b->d.p.norm == AFE_NORM_NONE) throw Error("corpus_stats: norm is NONE");
         run_reduce(b);
         if (d_stats) *d_stats = b->plan.stats();
-        if (stats_len) *stats_len = (4 * b->d.width + 1) * b->n_groups;
+        if (stats_len) *stats_len = (4 * b->d.width + 1) * b->plan.n_groups;
     });
 }
 
@@ -737,7 +724,7 @@ int afe_batch_set_corpus_stats(afe_batch *b, const double *h_stats, int stats_le
     return guarded([&] {
         DeviceGuard g(b->device);
         if (b->d.p.norm == AFE_NORM_NONE) throw Error("set_corpus_stats: norm is NONE");
-        if (stats_len != (4 * b->d.width + 1) * b->n_groups) throw Error("set_corpus_stats: wrong length");
+        if (stats_len != (4 * b->d.width + 1) * b->plan.n_groups) throw Error("set_corpus_stats: wrong length");
         AFE_CUDA(cudaMemcpyAsync(b->plan.stats(), h_stats, sizeof(double) * stats_len, cudaMemcpyHostToDevice, b->stream));
         AFE_CUDA(cudaStreamSynchronize(b->stream));
     });
@@ -765,18 +752,19 @@ int afe_batch_run_host(afe_batch *b, const int16_t *h_pcm, float *h_out)
     return guarded([&] {
         DeviceGuard g(b->device);
         const Derived &d = b->d;
-        if (!b->plan.tiles.p) throw Error("afe_batch_plan must be called before running");
+        const afe_batch::Plan &pl = b->plan;
+        if (!pl.tiles.p) throw Error("afe_batch_plan must be called before running");
         if (b->scope == AFE_STATS_CORPUS && d.p.norm != AFE_NORM_NONE)
             throw Error("run_host: corpus statistics need the two-pass device sequence");
-        const size_t n_samples = (size_t)b->pcm_extent;
-        const size_t pcm_len = n_samples + 16, out_len = (size_t)b->frame_off.back() * d.width;
+        const size_t n_samples = (size_t)pl.pcm_extent;
+        const size_t pcm_len = n_samples + 16, out_len = (size_t)pl.frame_off.back() * d.width;
         if (pcm_len > b->pcm_stage.n) b->pcm_stage.alloc(pcm_len);
         if (out_len > b->out_stage.n) b->out_stage.alloc(out_len);
         if (!b->s_in) { b->s_in.create(); b->s_out.create(); }
         // chunks are contiguous in samples only when the utterances are packed in increasing order
         bool ordered = true;
-        for (int u = 0; u + 1 < b->n_utts; u++) ordered = ordered && b->sample_off[u] + b->sample_len[u] <= b->sample_off[u + 1];
-        const int n_chunks = ordered ? std::max(1, std::min(32, b->n_utts / 8)) : 1;
+        for (int u = 0; u + 1 < pl.n_utts; u++) ordered = ordered && pl.sample_off[u] + pl.sample_len[u] <= pl.sample_off[u + 1];
+        const int n_chunks = ordered ? std::max(1, std::min(32, pl.n_utts / 8)) : 1;
         while ((int)b->ev_in.size() < n_chunks) {
             Event e1, e2;
             e1.create(); e2.create();
@@ -785,20 +773,20 @@ int afe_batch_run_host(afe_batch *b, const int16_t *h_pcm, float *h_out)
         b->last_launches = 0;
         const bool norm = d.p.norm != AFE_NORM_NONE;
         for (int c = 0; c < n_chunks; c++) {
-            const int u0 = (int)((int64_t)b->n_utts * c / n_chunks), u1 = (int)((int64_t)b->n_utts * (c + 1) / n_chunks);
+            const int u0 = (int)((int64_t)pl.n_utts * c / n_chunks), u1 = (int)((int64_t)pl.n_utts * (c + 1) / n_chunks);
             if (u1 <= u0) continue;
-            const int64_t s0 = n_chunks == 1 ? 0 : b->sample_off[u0];
-            const int64_t s1 = n_chunks == 1 ? (int64_t)n_samples : b->sample_off[u1 - 1] + b->sample_len[u1 - 1];
+            const int64_t s0 = n_chunks == 1 ? 0 : pl.sample_off[u0];
+            const int64_t s1 = n_chunks == 1 ? (int64_t)n_samples : pl.sample_off[u1 - 1] + pl.sample_len[u1 - 1];
             AFE_CUDA(cudaMemcpyAsync(b->pcm_stage.p + s0, h_pcm + s0, (size_t)(s1 - s0) * 2, cudaMemcpyHostToDevice, b->s_in));
             AFE_CUDA(cudaEventRecord(b->ev_in[c], b->s_in));
             AFE_CUDA(cudaStreamWaitEvent(b->stream, b->ev_in[c], 0));
-            const int t0 = b->h_tile_begin[u0], t1 = b->h_tile_begin[u1];
+            const int t0 = pl.h_tile_begin[u0], t1 = pl.h_tile_begin[u1];
             const bool fuse = b->fuse_norm();
             run_extract(b, b->pcm_stage.p, b->out_stage.p, t0, t1, fuse);
             if (norm && !fuse) { run_reduce(b, u0, u1); run_normalize(b, b->out_stage.p, t0, t1, u0, u1); }
             AFE_CUDA(cudaEventRecord(b->ev_k[c], b->stream));
             AFE_CUDA(cudaStreamWaitEvent(b->s_out, b->ev_k[c], 0));
-            const size_t r0 = (size_t)b->frame_off[u0] * d.width, r1 = (size_t)b->frame_off[u1] * d.width;
+            const size_t r0 = (size_t)pl.frame_off[u0] * d.width, r1 = (size_t)pl.frame_off[u1] * d.width;
             AFE_CUDA(cudaMemcpyAsync(h_out + r0, b->out_stage.p + r0, (r1 - r0) * 4, cudaMemcpyDeviceToHost, b->s_out));
         }
         AFE_CUDA(cudaStreamSynchronize(b->s_out));

@@ -131,11 +131,7 @@ struct afe_mfcc {
     int spec_row0 = 0;
     bool spec_on_host = false;          // the speculative rows already travelled to h_out with the block's rows
     bool pending = false;               // work enqueued on the stream since the last synchronisation
-    DevBuf<double> partials;
-    DevBuf<int> counters;               // [1] arrival tickets + [1] role tickets
-    DevBuf<unsigned> flags;
-    unsigned epoch = 0;
-    DevBuf<float> g_mean, g_scale;      // statistics of the last normalised block (use_last_stats for the flush block)
+    FusedNormState norm;                // one group: the block; mean / scale also serve the flush block (use_last_stats)
     int launches = 0;
     // ---- staged route (parameter sets K1 does not cover): one kernel per reference stage, spectrum persisted
     FftTables fft;
@@ -187,13 +183,7 @@ int afe_mfcc_create(const afe_params *p, int cuda_device, afe_mfcc **out)
         if (fused) {
             h->eng.reset(new FusedEngine(d, cuda_device));
             h->tiles_cap = fc / 32 + 2 * (size_t)h->eng->sm_count + 8;
-            if (d.p.norm != AFE_NORM_NONE) {
-                h->partials.alloc((h->tiles_cap + 1) * 4 * d.width);
-                h->counters.alloc(2); h->flags.alloc(1);
-                AFE_CUDA(cudaMemset(h->counters.p, 0, sizeof(int) * 2));
-                AFE_CUDA(cudaMemset(h->flags.p, 0, sizeof(unsigned)));
-                h->g_mean.alloc(d.width); h->g_scale.alloc(d.width);
-            }
+            if (d.p.norm != AFE_NORM_NONE) h->norm.alloc(1, h->tiles_cap + 1, d.width);
         } else
             alloc_staged(h.get());
         h->outb.alloc((fc + d.D) * d.width);
@@ -333,35 +323,25 @@ static void apply_fused(afe_mfcc *h, int wc, int wc_nd, bool first, bool last)
     int ntiles, nout;
     eng.plan_uniform(wc_nd, t_first, wc, eng.latency_tile(wc), ntiles, nout);
     if ((size_t)ntiles + 1 > h->tiles_cap) throw Error("block needs more tiles than the object was sized for");
-    const bool tma = d.S % 8 == 0 && (reinterpret_cast<uintptr_t>(h->blk_pcm) & 15) == 0;
     // quirk Q1: flushing after a single set_input reads every static D rows early (static_row_offset() == 0 there)
     const bool q1_flush = h->seg.last_calc_flushed && !h->fix_q1;
-    FusedArgs a = eng.base_args((last && q1_flush) ? 2 : 0, tma);
-    a.pcm = h->blk_pcm; a.out = h->outb.p; a.tiles = nullptr; a.tile_base = 0;
+    FusedArgs a = eng.base_args((last && q1_flush) ? 2 : 0, h->blk_pcm, true);
+    a.out = h->outb.p;
     a.blk_ntiles = ntiles; a.blk_T = wc_nd; a.blk_t_first = t_first; a.blk_n_out = wc; a.blk_nout = nout;
     // the rows a flush() right after this block would return ride along as one more tile (rows [wc, wc + D) of outb)
     const bool spec = !last && d.D > 0 && wc_nd >= 2 * d.D;
     a.blk_spec = spec ? 1 : 0; a.blk_spec_q1 = q1_flush ? 1 : 0;
     const int total = ntiles + (spec ? 1 : 0);
-    int grid = total, cluster = 0;
-    if (d.p.norm != AFE_NORM_NONE) {
-        a.g_mean = h->g_mean.p; a.g_scale = h->g_scale.p;
-        if (last) a.use_last = 1;                             // mfcccpu.cpp:389: use_last_stats
-        else {
-            a.stats_rows_mode = 3; a.stats_count = wc;        // this block's output rows (normalizercpu.cpp:22-30)
-            a.stats_kind = d.p.norm == AFE_NORM_CMN ? 1 : d.p.norm == AFE_NORM_CVN ? 2 : 3;
-            a.partials = h->partials.p;
-            const bool fast3 = d.width == 3 * d.cols && d.l1 == 3 && d.l2 == 3;
-            if (!spec && fast3 && total <= 4 && eng.cluster_schedulable(total, a, h->st)) { a.cluster_norm = 1; cluster = total; }
-            else if (!spec && total <= 8) a.counters = h->counters.p;
-            else { // role scheme: one launch, the statistics of the block are final before any row is normalised
-                a.counters = h->counters.p; a.work_counter = h->counters.p + 1;
-                a.flags = h->flags.p; a.epoch = ++h->epoch; a.ntiles_launch = total;
-                grid = total + std::min(total, 2 * eng.sm_count);
-            }
-        }
+    const bool norm = d.p.norm != AFE_NORM_NONE;
+    if (norm) { a.g_mean = h->norm.mean.p; a.g_scale = h->norm.scale.p; a.use_last = last ? 1 : 0; } // mfcccpu.cpp:389
+    if (!norm || last) eng.launch_plain(a, total, h->st);
+    else {
+        eng.set_stats(a, h->norm, 3, wc);                     // this block's output rows (normalizercpu.cpp:22-30)
+        if (!spec && eng.default_regression() && total <= 4 && eng.cluster_schedulable(total, a, h->st))
+            eng.launch_clustered(a, total, total, h->norm, h->st);
+        else if (!spec && total <= 8) eng.launch_ticket(a, total, h->norm, h->st);
+        else eng.launch_roles(a, total, h->norm, h->st);
     }
-    eng.launch(a, grid, cluster, h->st);
     h->launches++;
     h->pending = true;
     h->out_is_spec = false; h->spec_on_host = false;
