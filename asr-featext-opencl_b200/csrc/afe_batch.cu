@@ -128,7 +128,7 @@ void count_launch(int n) { g_launches.fetch_add(n); }
 // ------------------------------------------------------------------------------------------------ K1 launch table
 #define AFE_DECL_INST(k) cudaError_t fused_launch_##k(const FusedLaunch &); int fused_max_clusters_##k(const FusedLaunch &);
 #define AFE_FOR_EACH_INST(X) X(0) X(1) X(2) X(3) X(4) X(5) X(6) X(7) X(8) X(9) X(10) X(11) X(12) X(13) X(14) X(15) X(16) X(17) \
-    X(18) X(19) X(20) X(21) X(22) X(23)
+    X(18) X(19) X(20) X(21) X(22) X(23) X(24) X(25) X(26) X(27) X(28) X(29) X(30) X(31)
 AFE_FOR_EACH_INST(AFE_DECL_INST)
 #undef AFE_DECL_INST
 
@@ -158,14 +158,15 @@ std::string fused_unsupported_reason(const Derived &d)
     if (d.S % 2) return "fused path needs an even shift";
     if (d.dct_len > 16) return "fused path supports ceps_len + c0 <= 16";
     if (d.width > 128) return "fused path supports output width <= 128";
-    if (d.nb > kMaxBanks) return "fused path supports num_banks <= 64";
+    if (d.nb > kMaxBanksWide) return "fused path supports num_banks <= 128";
     if (d.W > 26 * (d.M / 16) && d.W > d.N2) return "window longer than the FFT";
     return "";
 }
 
 // Mel weights + DCT matrix as a by-value kernel parameter (constant bank). Per filter b: bins [edges[b], edges[b+2]) with
 // weights filters[b%2][bin] — the per-filter form of the reference's two-running-sums sweep (mfcccpu.cpp:192-220).
-static void build_mel_const(const Derived &d, float alpha, MelConst &mc)
+template <int NB>
+static void build_mel_const(const Derived &d, float alpha, MelConstT<NB> &mc)
 {
     std::vector<int> edges; std::vector<float> filters, dct;
     build_filters(d, alpha, edges, filters);
@@ -179,7 +180,7 @@ static void build_mel_const(const Derived &d, float alpha, MelConst &mc)
         mc.wstart[w] = (short)off4;
         for (int b = w; b < d.nb; b += 8) {
             const int j0 = edges[b], j1 = edges[b + 2], s4 = j0 & ~3, n8 = std::max(1, (j1 - s4 + 7) / 8);
-            if (off4 + 2 * n8 > kMaxWl4) throw Error("mel weight list exceeds the kernel-parameter budget");
+            if (off4 + 2 * n8 > MelConstT<NB>::kWl4) throw Error("mel weight list exceeds the kernel-parameter budget");
             if (s4 + 8 * n8 > kMagStride + 16) throw Error("mel filter too wide for the fused kernel");
             mc.desc[b] = (s4 / 4) | (n8 << 16);
             float *wt = reinterpret_cast<float *>(mc.wl4 + off4);
@@ -200,19 +201,25 @@ FusedEngine::FusedEngine(const Derived &dd, int dev) : d(dd), device(dev)
     if (!why.empty()) throw Error(why);
     sm_count = sm_count_of(dev);
     fft.build(d.N2);
-    // tile geometry (2 CTAs per SM): the cepstra tile holds up to 512 frames (<= 27 KB of shared memory)
-    int tc = 512;
-    tc = std::min(tc, (6912 / d.cols) / kRoundFrames * kRoundFrames);
-    tc = std::max(tc, kRoundFrames * ((2 * d.D + 1 + kRoundFrames - 1) / kRoundFrames + 1));
-    tc_max = tc; nout_max = tc - 2 * d.D;
+    const int nfw = (d.nb + 7) / 8;  // filters per warp (8 warps): instantiated for 3, 5, 8 and 16
+    kf = nfw <= 3 ? 3 : nfw <= 5 ? 5 : nfw <= 8 ? 8 : 16;
+    if (kf == 16 && d.C == 0) {
+        // 65..128-column log-mel (D = 0, see k_fused_mfcc): the kernel writes each 32-frame round's rows as soon as they are
+        // computed, so the cepstra buffer holds one round and the tile size is not bound by shared memory
+        tc_max = kRoundFrames; nout_max = 512;
+    } else {
+        // tile geometry (2 CTAs per SM): the cepstra tile holds up to 512 frames (<= 27 KB of shared memory)
+        int tc = 512;
+        tc = std::min(tc, (6912 / d.cols) / kRoundFrames * kRoundFrames);
+        tc = std::max(tc, kRoundFrames * ((2 * d.D + 1 + kRoundFrames - 1) / kRoundFrames + 1));
+        tc_max = tc; nout_max = tc - 2 * d.D;
+    }
     const int ns = d.width / d.cols;
     L = d.N2 == 512 ? fused_smem_layout<512>(8, d.S, d.cols, tc_max, nout_max, d.l2, ns)
                     : fused_smem_layout<256>(8, d.S, d.cols, tc_max, nout_max, d.l2, ns);
     if (L.total > 227 * 1024) throw Error("fused kernel shared-memory budget exceeded");
     const int R = d.M / 16;
     pruned = d.W <= 26 * R;            // window tail is zero from n1 = 13 on (400/512 and 200/256 both qualify)
-    const int kf = (d.nb + 7) / 8;     // filters per warp (8 warps): instantiated for 3, 5 and 8
-    key = (d.N2 == 512 ? 0 : 6) + (pruned ? 0 : 3) + (kf <= 3 ? 0 : kf <= 5 ? 1 : 2);
 }
 
 void FusedEngine::set_window(const float *window, cudaStream_t st)
@@ -222,14 +229,17 @@ void FusedEngine::set_window(const float *window, cudaStream_t st)
 }
 void FusedEngine::ensure_mel(float alpha)
 {
-    if (mc_alpha != alpha) { build_mel_const(d, alpha, mc); mc_alpha = alpha; }
+    if (mc_alpha == alpha) return;
+    if (kf == 16) build_mel_const(d, alpha, mc_wide);
+    else build_mel_const(d, alpha, mc);
+    mc_alpha = alpha;
 }
 std::string FusedEngine::kernel_label() const
 {
     const int k = launch_key();
     char buf[96];
-    snprintf(buf, sizeof buf, "k_fused_mfcc<%d,%d,8,%d,%s>", k % 12 < 6 ? 512 : 256, k % 6 < 3 ? 13 : 16,
-             k % 3 == 0 ? 3 : k % 3 == 1 ? 5 : 8, k >= 12 ? "true" : "false");
+    snprintf(buf, sizeof buf, "k_fused_mfcc<%d,%d,8,%d,%s>", fused_key_n2(k), fused_key_nz(k), fused_key_kf(k),
+             fused_key_pre(k) ? "true" : "false");
     return buf;
 }
 
@@ -306,8 +316,8 @@ bool FusedEngine::cluster_schedulable(int cluster, const FusedArgs &a, cudaStrea
 {
     if (cluster < 1 || cluster > 4) return false;
     if (cluster_probe[cluster] < 0) {
-        FusedLaunch fl{a, L, &mc, cluster, cluster, st};
-        const int n = fused_variant_max_clusters(key, fl); // same footprint with and without pre-emphasis
+        FusedLaunch fl{a, L, mel_const(), cluster, cluster, st};
+        const int n = fused_variant_max_clusters(fused_key(d.N2, pruned ? 13 : 16, kf, false), fl); // same footprint with and without pre-emphasis
         cluster_probe[cluster] = n > 0 ? n : 0;
     }
     return cluster_probe[cluster] > 0;
@@ -316,7 +326,7 @@ bool FusedEngine::cluster_schedulable(int cluster, const FusedArgs &a, cudaStrea
 void FusedEngine::launch(const FusedArgs &a, int grid, int cluster, cudaStream_t st)
 {
     if (!window_set) throw Error("set_window must be called before running");
-    FusedLaunch fl{a, L, &mc, grid, cluster, st};
+    FusedLaunch fl{a, L, mel_const(), grid, cluster, st};
     const cudaError_t e = launch_fused_variant(launch_key(), fl);
     if (e != cudaSuccess) {
         cudaGetLastError();

@@ -49,24 +49,30 @@ struct Tile {
 constexpr int kTileNoStats = 1; // the tile's rows do not enter the group's statistics (speculative flush rows of a stream block)
 constexpr int kTileQ1All = 2;   // every row of the tile takes its static D rows early (FusedArgs::q1 == 2 for this tile only)
 
-constexpr int kMaxBanks = 64;
-constexpr int kMaxWl4 = (2 * 257 + 10 * kMaxBanks + 3) / 4; // every bin feeds a rising and a falling side; lists start on a
-                                                            // multiple of 4 bins and are padded to whole 8-bin chunks
+constexpr int kMaxBanks = 64;      // bank capacity of the instantiations with KF <= 8 (up to 64 banks)
+constexpr int kMaxBanksWide = 128; // bank capacity of the KF = 16 instantiations (65..128 banks)
 constexpr int kMagStride = 260; // floats per magnitude row (16-byte aligned rows)
 // row of frame f (0..31) of a round: pair k = f>>1 -> rows 8*(k>>2) + (k&3) and +4
 __host__ __device__ constexpr int mag_row(int f) { return 8 * (f >> 3) + ((f >> 1) & 3) + 4 * (f & 1); }
 
-// Mel / DCT tables passed BY VALUE as a kernel parameter (constant bank): indexed with warp-uniform indices only,
-// read with 128-bit constant loads. Weight lists are zero padded to a multiple of 4 bins; DCT rows to 16 columns.
-struct MelConst {
-    float4 wl4[kMaxWl4];         // weights of filter b: 2*n8[b] float4 = bins 4*fchunk[b] + 8*i + {0..7}, i < n8[b]. The lists
+// Mel / DCT tables for up to NB banks, passed BY VALUE as a kernel parameter (constant bank): indexed with warp-uniform
+// indices only, read with 128-bit constant loads. Weight lists are zero padded to a multiple of 4 bins; DCT rows to 16
+// columns. NB = 64: 7 KB; NB = 128: 16 KB (the parameter list must stay under 32 764 bytes, see below).
+template <int NB>
+struct MelConstT {
+    static constexpr int kBanks = NB;
+    static constexpr int kWl4 = (2 * 257 + 10 * NB + 3) / 4; // every bin feeds a rising and a falling side; lists start on
+                                                              // a multiple of 4 bins and are padded to whole 8-bin chunks
+    float4 wl4[kWl4];            // weights of filter b: 2*n8[b] float4 = bins 4*fchunk[b] + 8*i + {0..7}, i < n8[b]. The lists
                                  // of the filters of one warp class (b = w, w + 8, w + 16, ...) are CONTIGUOUS from
                                  // wstart[w], in that order, so phase 2 walks them with one running offset. The weights
                                  // carry the 0.5/N2 magnitude scale (an exact power of two), see fft_frame_mag
-    float4 dct4[kMaxBanks][4];   // [nb][16]
-    int desc[kMaxBanks];         // fchunk[b] (first 4-bin chunk = edges[b] / 4; leading weights are zero) | n8[b] << 16
+    float4 dct4[NB][4];          // [nb][16]
+    int desc[NB];                // fchunk[b] (first 4-bin chunk = edges[b] / 4; leading weights are zero) | n8[b] << 16
     short wstart[8];             // first float4 of warp class w (8 warps per CTA)
 };
+using MelConst = MelConstT<kMaxBanks>;
+using MelConstWide = MelConstT<kMaxBanksWide>;
 
 struct FusedArgs {
     const int16_t *pcm;
@@ -116,6 +122,9 @@ struct FusedSmem {
     int off_mbar, off_mags, off_part, off_warp, warp_bytes, w_pcm, w_scratch, pcm_bytes, off_dhat, off_dd, off_red,
         off_cep, total;
 };
+
+// CUDA 12.1+ accepts kernel parameter lists of up to 32 764 bytes; the widest one is (FusedArgs, FusedSmem, MelConstWide)
+static_assert(sizeof(FusedArgs) + sizeof(FusedSmem) + sizeof(MelConstWide) + 16 <= 32764, "K1 kernel parameters too large");
 
 inline int align_up(int v, int a) { return (v + a - 1) / a * a; }
 
@@ -540,11 +549,12 @@ __device__ __forceinline__ void normalise_role(const FusedArgs &a, const Tile tl
 }
 } // namespace dev
 
-// KF = filters per warp in phase 2 (ceil(num_banks / WARPS), rounded up to 3, 5 or 8): the phase is unrolled KF times,
-// so a tight bound keeps the round loop inside the instruction cache.
+// KF = filters per warp in phase 2 (ceil(num_banks / WARPS), rounded up to 3, 5, 8 or 16): up to 8 the phase is unrolled
+// KF times, so a tight bound keeps the round loop inside the instruction cache. KF = 16 (65..128 banks) runs the warp's
+// filters in passes of 4: 16 unrolled filters do not fit the register budget of 2 CTAs per SM.
 template <int N2, int NZ, int kFusedWarps, int KF, bool PRE>
 __global__ void __launch_bounds__(32 * kFusedWarps, 2)
-k_fused_mfcc(const FusedArgs a, const FusedSmem L, const __grid_constant__ MelConst mc)
+k_fused_mfcc(const FusedArgs a, const FusedSmem L, const __grid_constant__ MelConstT<(KF <= 8 ? kMaxBanks : kMaxBanksWide)> mc)
 {
     constexpr bool FAST = false; // MUFU log approximation: measured in round 1, not shipped
     using C = dev::FftCfg<N2>;
@@ -617,6 +627,13 @@ k_fused_mfcc(const FusedArgs a, const FusedSmem L, const __grid_constant__ MelCo
     // shared-memory address of this lane's magnitude row in phase 2 (lane = frame of the round), pinned in a register
     const uint32_t mrow_s = dev::opaque(dev::smem_u32(s_mags) + mag_row(lane) * kMagStride * 4);
     uint32_t parity = 0;
+    // Log-mel rows of 65..128 columns (KF = 16 and no DCT; their width <= 128 leaves no room for deltas, so D = 0): the
+    // cepstra buffer holds ONE round and each round's rows are written, and their statistics kept, right after phase 2.
+    // A whole-tile buffer would allow 64-frame tiles only (2 CTAs per SM); this keeps tiles of up to 512 frames.
+    const bool round_rows = KF > 8 && a.dct_len == 0;
+    int wr_next = tid / a.width; // next row of this thread: rows tid / width + k * (256 / width), ascending (write_rows)
+    double wr_sum = 0.0, wr_sumsq = 0.0;
+    float wr_mn = FLT_MAX, wr_mx = -FLT_MAX;
     for (int r = 0; r < nrounds; r++) {
         const int f0 = r * kRoundFrames;            // first frame of the round (tile-local)
         const int nfr = min(kRoundFrames, ncomp - f0); // live frames of the round
@@ -664,81 +681,107 @@ k_fused_mfcc(const FusedArgs a, const FusedSmem L, const __grid_constant__ MelCo
 #else
         if (lane < nfr) {
 #endif
-            float es[KF];
+            constexpr int KP = KF <= 8 ? KF : 4; // filters per pass
             int woff = mc.wstart[warp]; // running float4 offset into this warp class's weight lists (uniform)
-            // the first 8-bin chunk of every filter of this warp is loaded up front (2*KF independent 128-bit loads in
-            // flight): 40 of the 89 chunks of the 40-filter bank, so most filters never wait for shared memory
-            int dsc[KF];
-            float4 mf0[KF], mf1[KF];
+            float2 cep[8];              // DCT accumulators, carried across passes
 #pragma unroll
-            for (int k = 0; k < KF; k++) {
-                const int b = warp + k * kFusedWarps;
-                dsc[k] = b < a.nb ? mc.desc[b] : 0;
-                const uint32_t maddr = mrow_s + ((dsc[k] & 0xffff) << 4);
-                mf0[k] = dev::lds128(maddr);
-                mf1[k] = dev::lds128(maddr + 16);
-            }
+            for (int c = 0; c < 8; c++) cep[c] = make_float2(0.f, 0.f);
+            const int npass = KF <= 8 ? 1 : ((a.nb - warp + kFusedWarps - 1) / kFusedWarps + KP - 1) / KP;
+#pragma unroll 1
+            for (int kb = 0; kb < npass * KP; kb += KP) { // filter slots kb .. kb + KP - 1 (b < 8 * KF always)
+                float es[KP];
+                // the first 8-bin chunk of every filter of this pass is loaded up front (2*KP independent 128-bit loads in
+                // flight): 40 of the 89 chunks of the 40-filter bank, so most filters never wait for shared memory
+                int dsc[KP];
+                float4 mf0[KP], mf1[KP];
 #pragma unroll
-            for (int k = 0; k < KF; k++) {
-                // four chains (bins 0,1 | 2,3 of every 4-bin group) in two register pairs: FFMA2, ascending bins in each
-                float2 acc0 = make_float2(0.f, 0.f), acc1 = acc0;
-                int n8 = dsc[k] >> 16;       // 0 for a slot past num_banks (warp uniform), else >= 1
-                if (n8 > 0) {
-                    uint32_t maddr = mrow_s + ((dsc[k] & 0xffff) << 4);
-                    float4 m0 = mf0[k], m1 = mf1[k];
-                    for (;;) {
-                        const float4 w0 = mc.wl4[woff], w1 = mc.wl4[woff + 1];
-                        acc0 = __ffma2_rn(make_float2(m0.x, m0.y), make_float2(w0.x, w0.y), acc0);
-                        acc1 = __ffma2_rn(make_float2(m0.z, m0.w), make_float2(w0.z, w0.w), acc1);
-                        acc0 = __ffma2_rn(make_float2(m1.x, m1.y), make_float2(w1.x, w1.y), acc0);
-                        acc1 = __ffma2_rn(make_float2(m1.z, m1.w), make_float2(w1.z, w1.w), acc1);
-                        woff += 2;
-                        if (--n8 == 0) break;
-                        maddr += 32;
-                        m0 = dev::lds128(maddr);
-                        m1 = dev::lds128(maddr + 16);
-                    }
+                for (int k = 0; k < KP; k++) {
+                    const int b = warp + (kb + k) * kFusedWarps;
+                    dsc[k] = b < a.nb ? mc.desc[b] : 0;
+                    const uint32_t maddr = mrow_s + ((dsc[k] & 0xffff) << 4);
+                    mf0[k] = dev::lds128(maddr);
+                    mf1[k] = dev::lds128(maddr + 16);
                 }
-                const float2 t = __fadd2_rn(acc0, acc1);
-                es[k] = t.x + t.y;
-            }
-            // logs two at a time (packed); a filter slot past num_banks holds 0 -> log(1e-30), never used
 #pragma unroll
-            for (int k = 0; k + 1 < KF; k += 2) {
-                const float2 e2 = dev::mel_log2<FAST>(make_float2(es[k], es[k + 1]));
-                es[k] = e2.x; es[k + 1] = e2.y;
-            }
-            if (KF & 1) es[KF - 1] = dev::mel_log<FAST>(es[KF - 1]);
-            if (a.dct_len > 0) {
-                float2 cep[8];
-#pragma unroll
-                for (int c = 0; c < 8; c++) cep[c] = make_float2(0.f, 0.f);
-                // no branch on b < num_banks: the DCT rows of the slots past it are zero (MelConst is zero filled) and their
-                // es is the finite log(1e-30), so the straight-line code lets the constant loads run ahead of the FMAs
-                // (6.23 -> 6.15 ms)
-#pragma unroll
-                for (int k = 0; k < KF; k++) {
-                    const int b = warp + k * kFusedWarps;
-                    const float2 e2 = make_float2(es[k], es[k]);
-#pragma unroll
-                    for (int c4 = 0; c4 < 4; c4++) {
-                        const float4 d4 = mc.dct4[b][c4];
-                        cep[2 * c4 + 0] = __ffma2_rn(e2, make_float2(d4.x, d4.y), cep[2 * c4 + 0]);
-                        cep[2 * c4 + 1] = __ffma2_rn(e2, make_float2(d4.z, d4.w), cep[2 * c4 + 1]);
+                for (int k = 0; k < KP; k++) {
+                    // four chains (bins 0,1 | 2,3 of every 4-bin group) in two register pairs: FFMA2, ascending bins in each
+                    float2 acc0 = make_float2(0.f, 0.f), acc1 = acc0;
+                    int n8 = dsc[k] >> 16;       // 0 for a slot past num_banks (warp uniform), else >= 1
+                    if (n8 > 0) {
+                        uint32_t maddr = mrow_s + ((dsc[k] & 0xffff) << 4);
+                        float4 m0 = mf0[k], m1 = mf1[k];
+                        for (;;) {
+                            const float4 w0 = mc.wl4[woff], w1 = mc.wl4[woff + 1];
+                            acc0 = __ffma2_rn(make_float2(m0.x, m0.y), make_float2(w0.x, w0.y), acc0);
+                            acc1 = __ffma2_rn(make_float2(m0.z, m0.w), make_float2(w0.z, w0.w), acc1);
+                            acc0 = __ffma2_rn(make_float2(m1.x, m1.y), make_float2(w1.x, w1.y), acc0);
+                            acc1 = __ffma2_rn(make_float2(m1.z, m1.w), make_float2(w1.z, w1.w), acc1);
+                            woff += 2;
+                            if (--n8 == 0) break;
+                            maddr += 32;
+                            m0 = dev::lds128(maddr);
+                            m1 = dev::lds128(maddr + 16);
+                        }
                     }
+                    const float2 t = __fadd2_rn(acc0, acc1);
+                    es[k] = t.x + t.y;
                 }
-                // partial cepstra of this filter class -> the exchange tile of the warp that will sum column group c4
+                // logs two at a time (packed); a filter slot past num_banks holds 0 -> log(1e-30), never used
 #pragma unroll
-                for (int c4 = 0; c4 < 4; c4++)
-                    reinterpret_cast<float4 *>(smem + L.off_part + c4 * L.w_scratch)[warp * kRoundFrames + lane] =
-                        make_float4(cep[2 * c4].x, cep[2 * c4].y, cep[2 * c4 + 1].x, cep[2 * c4 + 1].y);
-            } else {
+                for (int k = 0; k + 1 < KP; k += 2) {
+                    const float2 e2 = dev::mel_log2<FAST>(make_float2(es[k], es[k + 1]));
+                    es[k] = e2.x; es[k + 1] = e2.y;
+                }
+                if (KP & 1) es[KP - 1] = dev::mel_log<FAST>(es[KP - 1]);
+                if (a.dct_len > 0) {
+                    // no branch on b < num_banks: the DCT rows of the slots past it are zero (MelConst is zero filled) and their
+                    // es is the finite log(1e-30), so the straight-line code lets the constant loads run ahead of the FMAs
+                    // (6.23 -> 6.15 ms)
 #pragma unroll
-                for (int k = 0; k < KF; k++)
-                    if (warp + k * kFusedWarps < a.nb) s_cep[(f0 + lane) * cols + warp + k * kFusedWarps] = es[k];
+                    for (int k = 0; k < KP; k++) {
+                        const int b = warp + (kb + k) * kFusedWarps;
+                        const float2 e2 = make_float2(es[k], es[k]);
+#pragma unroll
+                        for (int c4 = 0; c4 < 4; c4++) {
+                            const float4 d4 = mc.dct4[b][c4];
+                            cep[2 * c4 + 0] = __ffma2_rn(e2, make_float2(d4.x, d4.y), cep[2 * c4 + 0]);
+                            cep[2 * c4 + 1] = __ffma2_rn(e2, make_float2(d4.z, d4.w), cep[2 * c4 + 1]);
+                        }
+                    }
+                    // partial cepstra of this filter class -> the exchange tile of the warp that will sum column group c4
+                    if (kb + KP == npass * KP) {
+#pragma unroll
+                        for (int c4 = 0; c4 < 4; c4++)
+                            reinterpret_cast<float4 *>(smem + L.off_part + c4 * L.w_scratch)[warp * kRoundFrames + lane] =
+                                make_float4(cep[2 * c4].x, cep[2 * c4].y, cep[2 * c4 + 1].x, cep[2 * c4 + 1].y);
+                    }
+                } else {
+#pragma unroll
+                    for (int k = 0; k < KP; k++)
+                        if (warp + (kb + k) * kFusedWarps < a.nb) s_cep[((round_rows ? 0 : f0) + lane) * cols + warp + (kb + k) * kFusedWarps] = es[k];
+                }
             }
         }
         __syncthreads(); // B: partial cepstra are complete; the magnitudes may be overwritten
+        if (round_rows && tid < kFusedThreads / a.width * a.width) {
+            // this round's rows [f0, f0 + nfr) (c0f = t0: no halo); the next round's phase 2 overwrites s_cep only after
+            // barrier A, which every thread reaches after its writes. Values recomputed per round: fewer live registers.
+            const int wr_rpp = kFusedThreads / a.width, wr_col = tid - tid / a.width * a.width;
+            const int wr_rs = (tl.flags & kTileNoStats) ? 0
+                              : a.stats_rows_mode == 3 ? tl.nout
+                              : a.stats_rows_mode == 0 ? 0
+                                                        : min(tl.nout, max(0, (a.stats_rows_mode == 1 ? tl.T - D : tl.T) - tl.t0));
+            float *orow = a.out + (tl.out_row0 + tl.t0 + f0) * (long long)a.width + wr_col;
+            const float *src = s_cep + wr_col;
+            const int r0 = wr_next - f0, rs = wr_rs - f0;
+            switch (a.stats_kind) {
+            case 0: dev::write_rows<0>(orow, src, r0, wr_rpp, nfr, nfr, rs, cols, a.width, 0, wr_sum, wr_sumsq, wr_mn, wr_mx); break;
+            case 1: dev::write_rows<1>(orow, src, r0, wr_rpp, nfr, nfr, rs, cols, a.width, 0, wr_sum, wr_sumsq, wr_mn, wr_mx); break;
+            case 2: dev::write_rows<2>(orow, src, r0, wr_rpp, nfr, nfr, rs, cols, a.width, 0, wr_sum, wr_sumsq, wr_mn, wr_mx); break;
+            default: dev::write_rows<3>(orow, src, r0, wr_rpp, nfr, nfr, rs, cols, a.width, 0, wr_sum, wr_sumsq, wr_mn, wr_mx); break;
+            }
+            while (wr_next < f0 + nfr) wr_next += wr_rpp;
+        }
         if (a.dct_len > 0 && warp < 4) {
             // warp w (< 4) sums columns 4w..4w+3 of every frame over the filter classes, in a fixed order. The partials
             // sit in ITS OWN exchange tile, so no CTA barrier is needed before the next round's FFTs reuse that memory.
@@ -870,7 +913,9 @@ k_fused_mfcc(const FusedArgs a, const FusedSmem L, const __grid_constant__ MelCo
         // 3c: rows out (coalesced: consecutive threads write consecutive floats), column statistics
         double sum = 0.0, sumsq = 0.0;
         float mn = FLT_MAX, mx = -FLT_MAX;
-        if (active) {
+        if (round_rows) { // rows already written round by round
+            sum = wr_sum; sumsq = wr_sumsq; mn = wr_mn; mx = wr_mx;
+        } else if (active) {
             float *orow = a.out + (tl.out_row0 + t0) * (long long)width + col;
             switch (a.stats_kind) {
             case 0: dev::write_rows<0>(orow, src, r_off, rpp, nout, rq, rs, cols, width, D, sum, sumsq, mn, mx); break;

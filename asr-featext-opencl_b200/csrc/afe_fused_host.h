@@ -26,20 +26,23 @@ struct FusedEngine {
     Derived d;
     int device = 0, sm_count = 0;
     FftTables fft;
-    MelTables mel;               // window tables only (the mel weights travel in `mc`)
-    MelConst mc;
+    MelTables mel;               // window tables only (the mel weights travel in `mc` / `mc_wide`)
+    MelConst mc;                 // up to 64 banks
+    MelConstWide mc_wide;        // 65..128 banks (KF = 16)
     float mc_alpha = -1.f;
     bool pruned = false;         // zero-padded window tail: the first FFT layer is pruned (NZ = 13)
     bool window_set = false;
     float pre = 0.f;             // pre-emphasis coefficient
     FusedSmem L{};
-    int tc_max = 0, nout_max = 0, key = 0;
+    int tc_max = 0, nout_max = 0;
+    int kf = 0;                  // filters per warp of the instantiation: 3, 5, 8 or 16
 
     explicit FusedEngine(const Derived &dd, int dev);
 
     void set_window(const float *window, cudaStream_t st);
     void ensure_mel(float alpha);   // rebuilds the constant-bank tables when alpha changed (refresh_filters, mfcccpu.cpp:24-60)
-    int launch_key() const { return key + (pre != 0.f ? 12 : 0); }
+    int launch_key() const { return fused_key(d.N2, pruned ? 13 : 16, kf, pre != 0.f); }
+    const void *mel_const() const { return kf == 16 ? (const void *)&mc_wide : (const void *)&mc; }
     std::string kernel_label() const; // the instantiation that runs, e.g. "k_fused_mfcc<512,13,8,5,false>"
     // Tiles for the output rows [t_first, t_first + n_out) of a sequence of T frames whose PCM starts at sample pcm_off;
     // output row of frame t = out_row0 + t. Appends to `tiles`; returns the number of tiles added.

@@ -1,21 +1,22 @@
-// One instantiation of the fused kernel per translation unit: nvcc -DAFE_INST_KEY=<0..23> (see the Makefile).
+// One instantiation of the fused kernel per translation unit: nvcc -DAFE_INST_KEY=<0..31> (see the Makefile).
 #include <atomic>
 
 #include "afe_internal.h"
 #include "afe_fused_launch.h"
 
 #ifndef AFE_INST_KEY
-#error "compile with -DAFE_INST_KEY=0..23"
+#error "compile with -DAFE_INST_KEY=0..31"
 #endif
 
 namespace afe {
 
 namespace {
-constexpr int kKey = AFE_INST_KEY % 12;
-constexpr bool kPre = AFE_INST_KEY >= 12;   // keys 12..23: the same shapes with per-frame pre-emphasis in the load
-constexpr int kN2 = kKey < 6 ? 512 : 256;
-constexpr int kNZ = (kKey % 6) < 3 ? 13 : 16;
-constexpr int kKF = (kKey % 3) == 0 ? 3 : (kKey % 3) == 1 ? 5 : 8;
+constexpr bool kPre = fused_key_pre(AFE_INST_KEY); // per-frame pre-emphasis in the load
+constexpr int kN2 = fused_key_n2(AFE_INST_KEY);
+constexpr int kNZ = fused_key_nz(AFE_INST_KEY);
+constexpr int kKF = fused_key_kf(AFE_INST_KEY);
+static_assert(fused_key(kN2, kNZ, kKF, kPre) == AFE_INST_KEY, "key encoding and decoding disagree");
+using Mel = MelConstT<(kKF <= 8 ? kMaxBanks : kMaxBanksWide)>;
 
 void fill(cudaLaunchConfig_t &cfg, cudaLaunchAttribute &attr, const FusedLaunch &fl)
 {
@@ -51,7 +52,7 @@ cudaError_t AFE_CAT(fused_launch_, AFE_INST_KEY)(const FusedLaunch &fl)
     if (e != cudaSuccess) return e;
     cudaLaunchConfig_t cfg; cudaLaunchAttribute attr;
     fill(cfg, attr, fl);
-    return cudaLaunchKernelEx(&cfg, kern, fl.a, fl.L, *fl.mc);
+    return cudaLaunchKernelEx(&cfg, kern, fl.a, fl.L, *static_cast<const Mel *>(fl.mc));
 }
 
 int AFE_CAT(fused_max_clusters_, AFE_INST_KEY)(const FusedLaunch &fl)

@@ -25,7 +25,7 @@ def random_params(rng):
     S = int(rng.integers(max(2, W // 5), W // 2 + 1))
     if rng.random() < 0.85:
         S -= S % 2
-    nb = int(rng.choice([8, 12, 20, 23, 24, 26, 32, 40, 41, 48, 64]))
+    nb = int(rng.choice([8, 12, 20, 23, 24, 26, 32, 40, 41, 48, 64, 72, 80, 96, 128]))
     ceps = int(rng.choice([0, 8, 12, 12, 12, 13, 15]))
     c0 = int(rng.integers(0, 2))
     if ceps + c0 > 16:
