@@ -128,7 +128,8 @@ void count_launch(int n) { g_launches.fetch_add(n); }
 // ------------------------------------------------------------------------------------------------ K1 launch table
 #define AFE_DECL_INST(k) cudaError_t fused_launch_##k(const FusedLaunch &); int fused_max_clusters_##k(const FusedLaunch &);
 #define AFE_FOR_EACH_INST(X) X(0) X(1) X(2) X(3) X(4) X(5) X(6) X(7) X(8) X(9) X(10) X(11) X(12) X(13) X(14) X(15) X(16) X(17) \
-    X(18) X(19) X(20) X(21) X(22) X(23) X(24) X(25) X(26) X(27) X(28) X(29) X(30) X(31)
+    X(18) X(19) X(20) X(21) X(22) X(23) X(24) X(25) X(26) X(27) X(28) X(29) X(30) X(31) X(32) X(33) X(34) X(35) X(36) X(37) \
+    X(38) X(39) X(40) X(41) X(42) X(43) X(44) X(45) X(46) X(47)
 AFE_FOR_EACH_INST(AFE_DECL_INST)
 #undef AFE_DECL_INST
 
@@ -156,17 +157,19 @@ std::string fused_unsupported_reason(const Derived &d)
 {
     if (d.N2 != 512 && d.N2 != 256) return "fused path supports 256/512-point FFTs (window_size 129..512)";
     if (d.S % 2) return "fused path needs an even shift";
-    if (d.dct_len > 16) return "fused path supports ceps_len + c0 <= 16";
+    if (d.C > 0 && d.dct_len > kMaxCepsWide) return "fused path supports ceps_len + c0 <= 48";
     if (d.width > 128) return "fused path supports output width <= 128";
     if (d.nb > kMaxBanksWide) return "fused path supports num_banks <= 128";
+    // 128 banks x 48 DCT columns of constant-bank tables would not fit the kernel parameter list
+    if (d.C > 0 && d.dct_len > 16 && d.nb > kMaxBanks) return "fused path supports ceps_len + c0 <= 16 with more than 64 banks";
     if (d.W > 26 * (d.M / 16) && d.W > d.N2) return "window longer than the FFT";
     return "";
 }
 
 // Mel weights + DCT matrix as a by-value kernel parameter (constant bank). Per filter b: bins [edges[b], edges[b+2]) with
 // weights filters[b%2][bin] — the per-filter form of the reference's two-running-sums sweep (mfcccpu.cpp:192-220).
-template <int NB>
-static void build_mel_const(const Derived &d, float alpha, MelConstT<NB> &mc)
+template <int NB, int NC>
+static void build_mel_const(const Derived &d, float alpha, MelConstT<NB, NC> &mc)
 {
     std::vector<int> edges; std::vector<float> filters, dct;
     build_filters(d, alpha, edges, filters);
@@ -180,7 +183,7 @@ static void build_mel_const(const Derived &d, float alpha, MelConstT<NB> &mc)
         mc.wstart[w] = (short)off4;
         for (int b = w; b < d.nb; b += 8) {
             const int j0 = edges[b], j1 = edges[b + 2], s4 = j0 & ~3, n8 = std::max(1, (j1 - s4 + 7) / 8);
-            if (off4 + 2 * n8 > MelConstT<NB>::kWl4) throw Error("mel weight list exceeds the kernel-parameter budget");
+            if (off4 + 2 * n8 > MelConstT<NB, NC>::kWl4) throw Error("mel weight list exceeds the kernel-parameter budget");
             if (s4 + 8 * n8 > kMagStride + 16) throw Error("mel filter too wide for the fused kernel");
             mc.desc[b] = (s4 / 4) | (n8 << 16);
             float *wt = reinterpret_cast<float *>(mc.wl4 + off4);
@@ -189,6 +192,7 @@ static void build_mel_const(const Derived &d, float alpha, MelConstT<NB> &mc)
         }
     }
     if (d.C > 0) {
+        if (d.dct_len > NC) throw Error("DCT exceeds the kernel-parameter budget");
         build_dct(d, dct);
         for (int k = 0; k < d.nb; k++)
             for (int j = 0; j < d.dct_len; j++) reinterpret_cast<float *>(mc.dct4[k])[j] = dct[(size_t)k * d.dct_len + j];
@@ -203,10 +207,26 @@ FusedEngine::FusedEngine(const Derived &dd, int dev) : d(dd), device(dev)
     fft.build(d.N2);
     const int nfw = (d.nb + 7) / 8;  // filters per warp (8 warps): instantiated for 3, 5, 8 and 16
     kf = nfw <= 3 ? 3 : nfw <= 5 ? 5 : nfw <= 8 ? 8 : 16;
-    if (kf == 16 && d.C == 0) {
-        // 65..128-column log-mel (D = 0, see k_fused_mfcc): the kernel writes each 32-frame round's rows as soon as they are
-        // computed, so the cepstra buffer holds one round and the tile size is not bound by shared memory
+    if (d.C > 0 && d.dct_len > 16) { nc = kMaxCepsWide; kf = nfw <= 5 ? 5 : 8; } // wide DCT: KF = 5 (<= 40 banks) or 8
+    const int ns = d.width / d.cols;
+    auto layout = [&](int tc, int nout) {
+        FusedSmem l = d.N2 == 512 ? fused_smem_layout<512>(8, d.S, d.cols, tc, nout, d.l2, ns)
+                                  : fused_smem_layout<256>(8, d.S, d.cols, tc, nout, d.l2, ns);
+        if (nc > 16) l.total += lm_tile_bytes(kf); // the wide DCT's log-mel tile follows everything else
+        return l;
+    };
+    if ((kf == 16 && d.C == 0) || (nc > 16 && d.D == 0)) {
+        // 65..128-column log-mel, and the wide DCT without deltas (D = 0, see k_fused_mfcc): the kernel writes each
+        // 32-frame round's rows as soon as they are computed, so the cepstra buffer holds one round and the tile size is
+        // not bound by shared memory
         tc_max = kRoundFrames; nout_max = 512;
+    } else if (nc > 16) {
+        // wide DCT with deltas: the largest whole-round cepstra tile that keeps 2 CTAs per SM (41 + c0 with deltas and
+        // delta-deltas: 128 frames)
+        const int tc_min = kRoundFrames * ((2 * d.D + 1 + kRoundFrames - 1) / kRoundFrames + 1);
+        int tc = 512;
+        while (tc > tc_min && layout(tc, tc - 2 * d.D).total > kSmemTwoCtas) tc -= kRoundFrames;
+        tc_max = tc; nout_max = tc - 2 * d.D;
     } else {
         // tile geometry (2 CTAs per SM): the cepstra tile holds up to 512 frames (<= 27 KB of shared memory)
         int tc = 512;
@@ -214,10 +234,13 @@ FusedEngine::FusedEngine(const Derived &dd, int dev) : d(dd), device(dev)
         tc = std::max(tc, kRoundFrames * ((2 * d.D + 1 + kRoundFrames - 1) / kRoundFrames + 1));
         tc_max = tc; nout_max = tc - 2 * d.D;
     }
-    const int ns = d.width / d.cols;
-    L = d.N2 == 512 ? fused_smem_layout<512>(8, d.S, d.cols, tc_max, nout_max, d.l2, ns)
-                    : fused_smem_layout<256>(8, d.S, d.cols, tc_max, nout_max, d.l2, ns);
+    L = layout(tc_max, nout_max);
     if (L.total > 227 * 1024) throw Error("fused kernel shared-memory budget exceeded");
+    // phase-3 scratch of the default regression and the clustered scheme (k_fused_mfcc): row-group records at off_mags,
+    // the tile's record at +25 KB, mean / scale at +30 KB, all below the cepstra
+    const int rp = kMaxFusedThreads / d.cols;
+    if (rp * d.width * 32 > 25 * 1024 || d.width * 32 > 5 * 1024 || L.off_mags + 30 * 1024 + 2 * d.width * 4 > L.off_cep)
+        throw Error("fused kernel phase-3 scratch does not fit its shared-memory slots");
     const int R = d.M / 16;
     pruned = d.W <= 26 * R;            // window tail is zero from n1 = 13 on (400/512 and 200/256 both qualify)
 }
@@ -230,7 +253,8 @@ void FusedEngine::set_window(const float *window, cudaStream_t st)
 void FusedEngine::ensure_mel(float alpha)
 {
     if (mc_alpha == alpha) return;
-    if (kf == 16) build_mel_const(d, alpha, mc_wide);
+    if (nc > 16) build_mel_const(d, alpha, mc_ceps);
+    else if (kf == 16) build_mel_const(d, alpha, mc_wide);
     else build_mel_const(d, alpha, mc);
     mc_alpha = alpha;
 }
@@ -238,8 +262,8 @@ std::string FusedEngine::kernel_label() const
 {
     const int k = launch_key();
     char buf[96];
-    snprintf(buf, sizeof buf, "k_fused_mfcc<%d,%d,8,%d,%s>", fused_key_n2(k), fused_key_nz(k), fused_key_kf(k),
-             fused_key_pre(k) ? "true" : "false");
+    snprintf(buf, sizeof buf, "k_fused_mfcc<%d,%d,8,%d,%s%s>", fused_key_n2(k), fused_key_nz(k), fused_key_kf(k),
+             fused_key_pre(k) ? "true" : "false", fused_key_nc(k) > 16 ? ",48" : "");
     return buf;
 }
 
@@ -317,7 +341,7 @@ bool FusedEngine::cluster_schedulable(int cluster, const FusedArgs &a, cudaStrea
     if (cluster < 1 || cluster > 4) return false;
     if (cluster_probe[cluster] < 0) {
         FusedLaunch fl{a, L, mel_const(), cluster, cluster, st};
-        const int n = fused_variant_max_clusters(fused_key(d.N2, pruned ? 13 : 16, kf, false), fl); // same footprint with and without pre-emphasis
+        const int n = fused_variant_max_clusters(fused_key(d.N2, pruned ? 13 : 16, kf, false, nc), fl); // same footprint with and without pre-emphasis
         cluster_probe[cluster] = n > 0 ? n : 0;
     }
     return cluster_probe[cluster] > 0;

@@ -55,24 +55,28 @@ constexpr int kMagStride = 260; // floats per magnitude row (16-byte aligned row
 // row of frame f (0..31) of a round: pair k = f>>1 -> rows 8*(k>>2) + (k&3) and +4
 __host__ __device__ constexpr int mag_row(int f) { return 8 * (f >> 3) + ((f >> 1) & 3) + 4 * (f & 1); }
 
-// Mel / DCT tables for up to NB banks, passed BY VALUE as a kernel parameter (constant bank): indexed with warp-uniform
-// indices only, read with 128-bit constant loads. Weight lists are zero padded to a multiple of 4 bins; DCT rows to 16
-// columns. NB = 64: 7 KB; NB = 128: 16 KB (the parameter list must stay under 32 764 bytes, see below).
-template <int NB>
+// Mel / DCT tables for up to NB banks and NC DCT columns, passed BY VALUE as a kernel parameter (constant bank): indexed
+// with warp-uniform indices only, read with 128-bit constant loads. Weight lists are zero padded to a multiple of 4 bins;
+// DCT rows to NC columns. NB = 64: 7 KB; NB = 128: 16 KB; NB = 64 with NC = 48: 17 KB (the parameter list must stay
+// under 32 764 bytes, see below).
+template <int NB, int NC = 16>
 struct MelConstT {
     static constexpr int kBanks = NB;
+    static constexpr int kCols = NC;
     static constexpr int kWl4 = (2 * 257 + 10 * NB + 3) / 4; // every bin feeds a rising and a falling side; lists start on
                                                               // a multiple of 4 bins and are padded to whole 8-bin chunks
     float4 wl4[kWl4];            // weights of filter b: 2*n8[b] float4 = bins 4*fchunk[b] + 8*i + {0..7}, i < n8[b]. The lists
                                  // of the filters of one warp class (b = w, w + 8, w + 16, ...) are CONTIGUOUS from
                                  // wstart[w], in that order, so phase 2 walks them with one running offset. The weights
                                  // carry the 0.5/N2 magnitude scale (an exact power of two), see fft_frame_mag
-    float4 dct4[NB][4];          // [nb][16]
+    float4 dct4[NB][NC / 4];     // [nb][NC]
     int desc[NB];                // fchunk[b] (first 4-bin chunk = edges[b] / 4; leading weights are zero) | n8[b] << 16
     short wstart[8];             // first float4 of warp class w (8 warps per CTA)
 };
+constexpr int kMaxCepsWide = 48; // DCT column capacity of the wide-DCT instantiations (ceps_len + c0 = 17..48, <= 64 banks)
 using MelConst = MelConstT<kMaxBanks>;
 using MelConstWide = MelConstT<kMaxBanksWide>;
+using MelConstCeps = MelConstT<kMaxBanks, kMaxCepsWide>;
 
 struct FusedArgs {
     const int16_t *pcm;
@@ -117,16 +121,27 @@ struct FusedArgs {
 
 constexpr int kRoundFrames = 32; // frames per CTA round; WARPS (4 or 8) warps share them, 32/WARPS frames each
 constexpr int kMaxFusedThreads = 256;
+// Wide-DCT instantiations: phase 2 leaves the round's log-mel values in a tile [32 frames][8 KF + 4 floats] that follows the
+// rest of the dynamic shared memory (FusedSmem::total includes it). A row is an odd number of 16-byte chunks, so the DCT's
+// "lane = frame" 128-bit reads are conflict free.
+__host__ __device__ constexpr int lm_stride(int kf) { return 8 * kf + 4; }
+__host__ __device__ constexpr int lm_tile_bytes(int kf) { return kRoundFrames * lm_stride(kf) * 4; }
 
 struct FusedSmem {
     int off_mbar, off_mags, off_part, off_warp, warp_bytes, w_pcm, w_scratch, pcm_bytes, off_dhat, off_dd, off_red,
         off_cep, total;
 };
 
-// CUDA 12.1+ accepts kernel parameter lists of up to 32 764 bytes; the widest one is (FusedArgs, FusedSmem, MelConstWide)
+// CUDA 12.1+ accepts kernel parameter lists of up to 32 764 bytes; the widest ones are (FusedArgs, FusedSmem, MelConstWide)
+// and (FusedArgs, FusedSmem, MelConstCeps)
 static_assert(sizeof(FusedArgs) + sizeof(FusedSmem) + sizeof(MelConstWide) + 16 <= 32764, "K1 kernel parameters too large");
+static_assert(sizeof(FusedArgs) + sizeof(FusedSmem) + sizeof(MelConstCeps) + 16 <= 32764, "K1 kernel parameters too large");
 
 inline int align_up(int v, int a) { return (v + a - 1) / a * a; }
+
+// dynamic shared memory of one CTA when 2 CTAs share an SM (sm_100: 228 KB per SM, 1 KB reserved per CTA, and the few
+// bytes of k_fused_mfcc's static shared variables)
+constexpr int kSmemTwoCtas = 113 * 1024 - 64;
 
 template <int N2>
 FusedSmem fused_smem_layout(int kFusedWarps, int S, int cols, int tc_max, int nout_max, int l2, int nstreams)
@@ -552,11 +567,18 @@ __device__ __forceinline__ void normalise_role(const FusedArgs &a, const Tile tl
 // KF = filters per warp in phase 2 (ceil(num_banks / WARPS), rounded up to 3, 5, 8 or 16): up to 8 the phase is unrolled
 // KF times, so a tight bound keeps the round loop inside the instruction cache. KF = 16 (65..128 banks) runs the warp's
 // filters in passes of 4: 16 unrolled filters do not fit the register budget of 2 CTAs per SM.
-template <int N2, int NZ, int kFusedWarps, int KF, bool PRE>
+// NC = DCT column capacity. NC = 16: every warp keeps the partial cepstra of its filter class, warps 0-3 sum them.
+// NC = 48 (ceps_len + c0 = 17..48, KF = 5 or 8): phase 2 writes log-mel values to a tile and, after barrier B, warps 0-3
+// compute the DCT split by column (12 each, lane = frame), in ascending bank order, straight into s_cep.
+template <int N2, int NZ, int kFusedWarps, int KF, bool PRE, int NC = 16>
 __global__ void __launch_bounds__(32 * kFusedWarps, 2)
-k_fused_mfcc(const FusedArgs a, const FusedSmem L, const __grid_constant__ MelConstT<(KF <= 8 ? kMaxBanks : kMaxBanksWide)> mc)
+k_fused_mfcc(const FusedArgs a, const FusedSmem L, const __grid_constant__ MelConstT<(KF <= 8 ? kMaxBanks : kMaxBanksWide), NC> mc)
 {
     constexpr bool FAST = false; // MUFU log approximation: measured in round 1, not shipped
+    constexpr bool kWideDct = NC > 16;
+    static_assert(!kWideDct || KF <= 8, "the wide DCT serves up to 64 banks");
+    // warps of the wide DCT and columns per warp: with 4, warps 4-7 run ahead into the next round's FFTs (DESIGN §4)
+    constexpr int kDctWarps = 4, kDctCols = NC / kDctWarps;
     using C = dev::FftCfg<N2>;
     constexpr int kFusedThreads = 32 * kFusedWarps, kWarpFrames = kRoundFrames / kFusedWarps;
     constexpr int R = C::R, FPW = C::FPW, SCR = C::SCR;
@@ -630,10 +652,31 @@ k_fused_mfcc(const FusedArgs a, const FusedSmem L, const __grid_constant__ MelCo
     // Log-mel rows of 65..128 columns (KF = 16 and no DCT; their width <= 128 leaves no room for deltas, so D = 0): the
     // cepstra buffer holds ONE round and each round's rows are written, and their statistics kept, right after phase 2.
     // A whole-tile buffer would allow 64-frame tiles only (2 CTAs per SM); this keeps tiles of up to 512 frames.
-    const bool round_rows = KF > 8 && a.dct_len == 0;
+    // The wide DCT without deltas (D = 0) does the same; its cepstra are complete only after the DCT that follows barrier B,
+    // so a round's rows leave after the next round's barrier A (the last round's after the loop).
+    const bool round_rows = (KF > 8 && a.dct_len == 0) || (kWideDct && D == 0);
     int wr_next = tid / a.width; // next row of this thread: rows tid / width + k * (256 / width), ascending (write_rows)
     double wr_sum = 0.0, wr_sumsq = 0.0;
     float wr_mn = FLT_MAX, wr_mx = -FLT_MAX;
+    // wide DCT: rows [f0, f0 + nfr) of the tile, held in s_cep[0 .. nfr) (c0f = t0: no halo)
+    auto write_round_rows = [&](int f0, int nfr) {
+        if (tid >= kFusedThreads / a.width * a.width) return;
+        const int wr_rpp = kFusedThreads / a.width, wr_col = tid - tid / a.width * a.width;
+        const int wr_rs = (tl.flags & kTileNoStats) ? 0
+                          : a.stats_rows_mode == 3 ? tl.nout
+                          : a.stats_rows_mode == 0 ? 0
+                                                    : min(tl.nout, max(0, (a.stats_rows_mode == 1 ? tl.T - D : tl.T) - tl.t0));
+        float *orow = a.out + (tl.out_row0 + tl.t0 + f0) * (long long)a.width + wr_col;
+        const float *src = s_cep + wr_col;
+        const int r0 = wr_next - f0, rs = wr_rs - f0;
+        switch (a.stats_kind) {
+        case 0: dev::write_rows<0>(orow, src, r0, wr_rpp, nfr, nfr, rs, cols, a.width, 0, wr_sum, wr_sumsq, wr_mn, wr_mx); break;
+        case 1: dev::write_rows<1>(orow, src, r0, wr_rpp, nfr, nfr, rs, cols, a.width, 0, wr_sum, wr_sumsq, wr_mn, wr_mx); break;
+        case 2: dev::write_rows<2>(orow, src, r0, wr_rpp, nfr, nfr, rs, cols, a.width, 0, wr_sum, wr_sumsq, wr_mn, wr_mx); break;
+        default: dev::write_rows<3>(orow, src, r0, wr_rpp, nfr, nfr, rs, cols, a.width, 0, wr_sum, wr_sumsq, wr_mn, wr_mx); break;
+        }
+        while (wr_next < f0 + nfr) wr_next += wr_rpp;
+    };
     for (int r = 0; r < nrounds; r++) {
         const int f0 = r * kRoundFrames;            // first frame of the round (tile-local)
         const int nfr = min(kRoundFrames, ncomp - f0); // live frames of the round
@@ -672,6 +715,7 @@ k_fused_mfcc(const FusedArgs a, const FusedSmem L, const __grid_constant__ MelCo
             if (a.use_tma && lane == 0 && r + 1 < nrounds) issue_tma(r + 1);
         }
         __syncthreads(); // A: all magnitudes of the round are in shared memory
+        if (kWideDct && round_rows && r > 0) write_round_rows(f0 - kRoundFrames, kRoundFrames);
 
         // ---- phase 2: lane = frame of the round, warp = filter class (filters warp, warp + WARPS, ...).
         //      Three unrolled passes over the warp's <= KF filters - sums, logs, DCT - so that the independent filters'
@@ -681,12 +725,12 @@ k_fused_mfcc(const FusedArgs a, const FusedSmem L, const __grid_constant__ MelCo
 #else
         if (lane < nfr) {
 #endif
-            constexpr int KP = KF <= 8 ? KF : 4; // filters per pass
+            constexpr int KP = KF <= 8 && !(kWideDct && KF == 8) ? KF : 4; // filters per pass
             int woff = mc.wstart[warp]; // running float4 offset into this warp class's weight lists (uniform)
             float2 cep[8];              // DCT accumulators, carried across passes
 #pragma unroll
             for (int c = 0; c < 8; c++) cep[c] = make_float2(0.f, 0.f);
-            const int npass = KF <= 8 ? 1 : ((a.nb - warp + kFusedWarps - 1) / kFusedWarps + KP - 1) / KP;
+            const int npass = KP == KF ? 1 : ((a.nb - warp + kFusedWarps - 1) / kFusedWarps + KP - 1) / KP;
 #pragma unroll 1
             for (int kb = 0; kb < npass * KP; kb += KP) { // filter slots kb .. kb + KP - 1 (b < 8 * KF always)
                 float es[KP];
@@ -733,7 +777,13 @@ k_fused_mfcc(const FusedArgs a, const FusedSmem L, const __grid_constant__ MelCo
                     es[k] = e2.x; es[k + 1] = e2.y;
                 }
                 if (KP & 1) es[KP - 1] = dev::mel_log<FAST>(es[KP - 1]);
-                if (a.dct_len > 0) {
+                if (kWideDct) {
+                    // every slot, also those past num_banks (the finite log(1e-30), against zero DCT rows): the DCT reads
+                    // whole 4-bank chunks
+                    float *lrow = reinterpret_cast<float *>(smem + L.total - lm_tile_bytes(KF)) + lane * lm_stride(KF) + warp;
+#pragma unroll
+                    for (int k = 0; k < KP; k++) lrow[(kb + k) * kFusedWarps] = es[k];
+                } else if (a.dct_len > 0) {
                     // no branch on b < num_banks: the DCT rows of the slots past it are zero (MelConst is zero filled) and their
                     // es is the finite log(1e-30), so the straight-line code lets the constant loads run ahead of the FMAs
                     // (6.23 -> 6.15 ms)
@@ -763,7 +813,9 @@ k_fused_mfcc(const FusedArgs a, const FusedSmem L, const __grid_constant__ MelCo
             }
         }
         __syncthreads(); // B: partial cepstra are complete; the magnitudes may be overwritten
-        if (round_rows && tid < kFusedThreads / a.width * a.width) {
+        // (the same code as write_round_rows, written out: called through the lambda, it compiled to a different schedule
+        // for the KF = 16 instantiations)
+        if (!kWideDct && round_rows && tid < kFusedThreads / a.width * a.width) {
             // this round's rows [f0, f0 + nfr) (c0f = t0: no halo); the next round's phase 2 overwrites s_cep only after
             // barrier A, which every thread reaches after its writes. Values recomputed per round: fewer live registers.
             const int wr_rpp = kFusedThreads / a.width, wr_col = tid - tid / a.width * a.width;
@@ -782,7 +834,36 @@ k_fused_mfcc(const FusedArgs a, const FusedSmem L, const __grid_constant__ MelCo
             }
             while (wr_next < f0 + nfr) wr_next += wr_rpp;
         }
-        if (a.dct_len > 0 && warp < 4) {
+        if (kWideDct) {
+            // warp w (< kDctWarps) computes columns kDctCols*w .. +kDctCols of every frame from the log-mel tile, one FFMA2
+            // chain per column pair in ascending bank order. The log-mel tile is rewritten only after the next barrier A,
+            // and s_cep is read (next round's rows, phase 3) only after a barrier: none is needed here.
+            if (warp < kDctWarps && kDctCols * warp < a.dct_len && lane < nfr) {
+                const float4 *lrow = reinterpret_cast<const float4 *>(smem + L.total - lm_tile_bytes(KF)) + lane * (lm_stride(KF) / 4);
+                float2 acc[kDctCols / 2];
+#pragma unroll
+                for (int j = 0; j < kDctCols / 2; j++) acc[j] = make_float2(0.f, 0.f);
+                const int nb4 = (a.nb + 3) >> 2;
+#pragma unroll 2
+                for (int b4 = 0; b4 < nb4; b4++) {
+                    const float4 e = lrow[b4];
+                    const float ev[4] = {e.x, e.y, e.z, e.w};
+#pragma unroll
+                    for (int i = 0; i < 4; i++) {
+                        const float2 e2 = make_float2(ev[i], ev[i]);
+                        const float2 *drow = reinterpret_cast<const float2 *>(mc.dct4[4 * b4 + i]) + warp * (kDctCols / 2);
+#pragma unroll
+                        for (int j = 0; j < kDctCols / 2; j++) acc[j] = __ffma2_rn(e2, drow[j], acc[j]);
+                    }
+                }
+                float *crow = s_cep + ((round_rows ? 0 : f0) + lane) * cols + kDctCols * warp;
+#pragma unroll
+                for (int j = 0; j < kDctCols / 2; j++) {
+                    if (kDctCols * warp + 2 * j < a.dct_len) crow[2 * j] = acc[j].x;
+                    if (kDctCols * warp + 2 * j + 1 < a.dct_len) crow[2 * j + 1] = acc[j].y;
+                }
+            }
+        } else if (a.dct_len > 0 && warp < 4) {
             // warp w (< 4) sums columns 4w..4w+3 of every frame over the filter classes, in a fixed order. The partials
             // sit in ITS OWN exchange tile, so no CTA barrier is needed before the next round's FFTs reuse that memory.
             // (Spreading this sum over all 8 warps was measured 6 % SLOWER, tools/gpu_ab.sh: warps 4-7 running ahead
@@ -805,6 +886,7 @@ k_fused_mfcc(const FusedArgs a, const FusedSmem L, const __grid_constant__ MelCo
         }
     }
     __syncthreads(); // all cepstra of the tile are in shared memory
+    if (kWideDct && round_rows) write_round_rows((nrounds - 1) * kRoundFrames, ncomp - (nrounds - 1) * kRoundFrames);
 
     // ---- phase 3: every thread owns ONE column (c = tid % cols / col = tid % width) and strides over rows, so the loops
     //      are uniform (no integer division, no stream-dependent branch inside them).

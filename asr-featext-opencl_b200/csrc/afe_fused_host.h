@@ -29,6 +29,7 @@ struct FusedEngine {
     MelTables mel;               // window tables only (the mel weights travel in `mc` / `mc_wide`)
     MelConst mc;                 // up to 64 banks
     MelConstWide mc_wide;        // 65..128 banks (KF = 16)
+    MelConstCeps mc_ceps;        // ceps_len + c0 = 17..48 (NC = 48, up to 64 banks)
     float mc_alpha = -1.f;
     bool pruned = false;         // zero-padded window tail: the first FFT layer is pruned (NZ = 13)
     bool window_set = false;
@@ -36,14 +37,19 @@ struct FusedEngine {
     FusedSmem L{};
     int tc_max = 0, nout_max = 0;
     int kf = 0;                  // filters per warp of the instantiation: 3, 5, 8 or 16
+    int nc = 16;                 // DCT column capacity of the instantiation: 16 or 48
 
     explicit FusedEngine(const Derived &dd, int dev);
 
     void set_window(const float *window, cudaStream_t st);
     void ensure_mel(float alpha);   // rebuilds the constant-bank tables when alpha changed (refresh_filters, mfcccpu.cpp:24-60)
-    int launch_key() const { return fused_key(d.N2, pruned ? 13 : 16, kf, pre != 0.f); }
-    const void *mel_const() const { return kf == 16 ? (const void *)&mc_wide : (const void *)&mc; }
-    std::string kernel_label() const; // the instantiation that runs, e.g. "k_fused_mfcc<512,13,8,5,false>"
+    int launch_key() const { return fused_key(d.N2, pruned ? 13 : 16, kf, pre != 0.f, nc); }
+    const void *mel_const() const
+    {
+        return nc > 16 ? (const void *)&mc_ceps : kf == 16 ? (const void *)&mc_wide : (const void *)&mc;
+    }
+    // the instantiation that runs, e.g. "k_fused_mfcc<512,13,8,5,false>" or, with NC = 48, "k_fused_mfcc<512,13,8,5,false,48>"
+    std::string kernel_label() const;
     // Tiles for the output rows [t_first, t_first + n_out) of a sequence of T frames whose PCM starts at sample pcm_off;
     // output row of frame t = out_row0 + t. Appends to `tiles`; returns the number of tiles added.
     // nout_cap: largest tile (output frames), 0 = as large as the kernel's cepstra buffer allows (best throughput for big

@@ -1,11 +1,11 @@
-// One instantiation of the fused kernel per translation unit: nvcc -DAFE_INST_KEY=<0..31> (see the Makefile).
+// One instantiation of the fused kernel per translation unit: nvcc -DAFE_INST_KEY=<0..47> (see the Makefile).
 #include <atomic>
 
 #include "afe_internal.h"
 #include "afe_fused_launch.h"
 
 #ifndef AFE_INST_KEY
-#error "compile with -DAFE_INST_KEY=0..31"
+#error "compile with -DAFE_INST_KEY=0..47"
 #endif
 
 namespace afe {
@@ -15,8 +15,9 @@ constexpr bool kPre = fused_key_pre(AFE_INST_KEY); // per-frame pre-emphasis in 
 constexpr int kN2 = fused_key_n2(AFE_INST_KEY);
 constexpr int kNZ = fused_key_nz(AFE_INST_KEY);
 constexpr int kKF = fused_key_kf(AFE_INST_KEY);
-static_assert(fused_key(kN2, kNZ, kKF, kPre) == AFE_INST_KEY, "key encoding and decoding disagree");
-using Mel = MelConstT<(kKF <= 8 ? kMaxBanks : kMaxBanksWide)>;
+constexpr int kNC = fused_key_nc(AFE_INST_KEY);
+static_assert(fused_key(kN2, kNZ, kKF, kPre, kNC) == AFE_INST_KEY, "key encoding and decoding disagree");
+using Mel = MelConstT<(kKF <= 8 ? kMaxBanks : kMaxBanksWide), kNC>;
 
 void fill(cudaLaunchConfig_t &cfg, cudaLaunchAttribute &attr, const FusedLaunch &fl)
 {
@@ -40,14 +41,14 @@ static cudaError_t ensure_smem_attr(int bytes)
     if (e != cudaSuccess) return e;
     if (dev < 0 || dev >= 64) dev = 63;
     if (done[dev].load(std::memory_order_acquire) >= bytes) return cudaSuccess;
-    e = cudaFuncSetAttribute(k_fused_mfcc<kN2, kNZ, 8, kKF, kPre>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+    e = cudaFuncSetAttribute(k_fused_mfcc<kN2, kNZ, 8, kKF, kPre, kNC>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
     if (e == cudaSuccess) done[dev].store(bytes, std::memory_order_release);
     return e;
 }
 
 cudaError_t AFE_CAT(fused_launch_, AFE_INST_KEY)(const FusedLaunch &fl)
 {
-    auto kern = k_fused_mfcc<kN2, kNZ, 8, kKF, kPre>;
+    auto kern = k_fused_mfcc<kN2, kNZ, 8, kKF, kPre, kNC>;
     cudaError_t e = ensure_smem_attr(fl.L.total);
     if (e != cudaSuccess) return e;
     cudaLaunchConfig_t cfg; cudaLaunchAttribute attr;
@@ -57,7 +58,7 @@ cudaError_t AFE_CAT(fused_launch_, AFE_INST_KEY)(const FusedLaunch &fl)
 
 int AFE_CAT(fused_max_clusters_, AFE_INST_KEY)(const FusedLaunch &fl)
 {
-    auto kern = k_fused_mfcc<kN2, kNZ, 8, kKF, kPre>;
+    auto kern = k_fused_mfcc<kN2, kNZ, 8, kKF, kPre, kNC>;
     if (ensure_smem_attr(fl.L.total) != cudaSuccess) return -1;
     cudaLaunchConfig_t cfg; cudaLaunchAttribute attr;
     fill(cfg, attr, fl);

@@ -26,10 +26,8 @@ def random_params(rng):
     if rng.random() < 0.85:
         S -= S % 2
     nb = int(rng.choice([8, 12, 20, 23, 24, 26, 32, 40, 41, 48, 64, 72, 80, 96, 128]))
-    ceps = int(rng.choice([0, 8, 12, 12, 12, 13, 15]))
+    ceps = int(rng.choice([0, 8, 12, 12, 12, 13, 15, 16, 19, 23, 29, 39, 40, 47]))
     c0 = int(rng.integers(0, 2))
-    if ceps + c0 > 16:
-        c0 = 0
     dyn = int(rng.integers(0, 3))
     cols = ceps + c0 if ceps > 0 else nb
     if cols * (dyn + 1) > 128:
