@@ -129,7 +129,8 @@ void count_launch(int n) { g_launches.fetch_add(n); }
 #define AFE_DECL_INST(k) cudaError_t fused_launch_##k(const FusedLaunch &); int fused_max_clusters_##k(const FusedLaunch &);
 #define AFE_FOR_EACH_INST(X) X(0) X(1) X(2) X(3) X(4) X(5) X(6) X(7) X(8) X(9) X(10) X(11) X(12) X(13) X(14) X(15) X(16) X(17) \
     X(18) X(19) X(20) X(21) X(22) X(23) X(24) X(25) X(26) X(27) X(28) X(29) X(30) X(31) X(32) X(33) X(34) X(35) X(36) X(37) \
-    X(38) X(39) X(40) X(41) X(42) X(43) X(44) X(45) X(46) X(47)
+    X(38) X(39) X(40) X(41) X(42) X(43) X(44) X(45) X(46) X(47) X(48) X(49) X(50) X(51) X(52) X(53) X(54) X(55) X(56) X(57) \
+    X(58) X(59) X(60) X(61) X(62) X(63)
 AFE_FOR_EACH_INST(AFE_DECL_INST)
 #undef AFE_DECL_INST
 
@@ -155,27 +156,29 @@ int fused_variant_max_clusters(int key, const FusedLaunch &fl)
 // ------------------------------------------------------------------------------------------------ FusedEngine
 std::string fused_unsupported_reason(const Derived &d)
 {
-    if (d.N2 != 512 && d.N2 != 256) return "fused path supports 256/512-point FFTs (window_size 129..512)";
+    if (d.N2 != 1024 && d.N2 != 512 && d.N2 != 256) return "fused path supports 256/512/1024-point FFTs (window_size 129..1024)";
     if (d.S % 2) return "fused path needs an even shift";
     if (d.C > 0 && d.dct_len > kMaxCepsWide) return "fused path supports ceps_len + c0 <= 48";
     if (d.width > 128) return "fused path supports output width <= 128";
     if (d.nb > kMaxBanksWide) return "fused path supports num_banks <= 128";
     // 128 banks x 48 DCT columns of constant-bank tables would not fit the kernel parameter list
     if (d.C > 0 && d.dct_len > 16 && d.nb > kMaxBanks) return "fused path supports ceps_len + c0 <= 16 with more than 64 banks";
+    if (d.C > 0 && d.dct_len > 16 && d.N2 == 1024) return "fused path supports ceps_len + c0 <= 16 with 1024-point FFTs";
     if (d.W > 26 * (d.M / 16) && d.W > d.N2) return "window longer than the FFT";
     return "";
 }
 
 // Mel weights + DCT matrix as a by-value kernel parameter (constant bank). Per filter b: bins [edges[b], edges[b+2]) with
 // weights filters[b%2][bin] — the per-filter form of the reference's two-running-sums sweep (mfcccpu.cpp:192-220).
-template <int NB, int NC>
-static void build_mel_const(const Derived &d, float alpha, MelConstT<NB, NC> &mc)
+template <int NB, int NC, int NBINS>
+static void build_mel_const(const Derived &d, float alpha, MelConstT<NB, NC, NBINS> &mc)
 {
     std::vector<int> edges; std::vector<float> filters, dct;
     build_filters(d, alpha, edges, filters);
     for (int i = 0; i + 1 < (int)edges.size(); i++)
         if (edges[i + 1] < edges[i]) throw Error("mel filter edges are not monotonic");
     if (edges.front() < 0 || edges.back() > d.M) throw Error("mel filterbank exceeds the Nyquist bin (check low_freq/high_freq)");
+    if (d.bins > NBINS) throw Error("FFT bins exceed the mel table capacity");
     memset(&mc, 0, sizeof mc);
     int off4 = 0;
     const float scale = 0.5f / (float)d.N2; // the kernel stores |2X|; scaling by a power of two commutes with rounding
@@ -183,8 +186,8 @@ static void build_mel_const(const Derived &d, float alpha, MelConstT<NB, NC> &mc
         mc.wstart[w] = (short)off4;
         for (int b = w; b < d.nb; b += 8) {
             const int j0 = edges[b], j1 = edges[b + 2], s4 = j0 & ~3, n8 = std::max(1, (j1 - s4 + 7) / 8);
-            if (off4 + 2 * n8 > MelConstT<NB, NC>::kWl4) throw Error("mel weight list exceeds the kernel-parameter budget");
-            if (s4 + 8 * n8 > kMagStride + 16) throw Error("mel filter too wide for the fused kernel");
+            if (off4 + 2 * n8 > MelConstT<NB, NC, NBINS>::kWl4) throw Error("mel weight list exceeds the kernel-parameter budget");
+            if (s4 + 8 * n8 > mag_stride(d.N2) + 16) throw Error("mel filter too wide for the fused kernel");
             mc.desc[b] = (s4 / 4) | (n8 << 16);
             float *wt = reinterpret_cast<float *>(mc.wl4 + off4);
             for (int j = j0; j < j1; j++) wt[j - s4] = filters[(size_t)(b % 2) * d.N2 + j] * scale;
@@ -208,10 +211,12 @@ FusedEngine::FusedEngine(const Derived &dd, int dev) : d(dd), device(dev)
     const int nfw = (d.nb + 7) / 8;  // filters per warp (8 warps): instantiated for 3, 5, 8 and 16
     kf = nfw <= 3 ? 3 : nfw <= 5 ? 5 : nfw <= 8 ? 8 : 16;
     if (d.C > 0 && d.dct_len > 16) { nc = kMaxCepsWide; kf = nfw <= 5 ? 5 : 8; } // wide DCT: KF = 5 (<= 40 banks) or 8
+    if (d.N2 == 1024) ctas_per_sm = 1; // the 66 KB magnitude tile (__launch_bounds__(256, 1) in k_fused_mfcc)
     const int ns = d.width / d.cols;
     auto layout = [&](int tc, int nout) {
-        FusedSmem l = d.N2 == 512 ? fused_smem_layout<512>(8, d.S, d.cols, tc, nout, d.l2, ns)
-                                  : fused_smem_layout<256>(8, d.S, d.cols, tc, nout, d.l2, ns);
+        FusedSmem l = d.N2 == 1024 ? fused_smem_layout<1024>(8, d.S, d.cols, tc, nout, d.l2, ns)
+                      : d.N2 == 512 ? fused_smem_layout<512>(8, d.S, d.cols, tc, nout, d.l2, ns)
+                                    : fused_smem_layout<256>(8, d.S, d.cols, tc, nout, d.l2, ns);
         if (nc > 16) l.total += lm_tile_bytes(kf); // the wide DCT's log-mel tile follows everything else
         return l;
     };
@@ -227,6 +232,13 @@ FusedEngine::FusedEngine(const Derived &dd, int dev) : d(dd), device(dev)
         int tc = 512;
         while (tc > tc_min && layout(tc, tc - 2 * d.D).total > kSmemTwoCtas) tc -= kRoundFrames;
         tc_max = tc; nout_max = tc - 2 * d.D;
+    } else if (d.N2 == 1024) {
+        // 1024 points: the 66 KB magnitude tile already limits K1 to one CTA per SM, so the cepstra tile is the largest
+        // whole-round tile, up to 512 frames, that fits one CTA's shared memory
+        const int tc_min = kRoundFrames * ((2 * d.D + 1 + kRoundFrames - 1) / kRoundFrames + 1);
+        int tc = 512;
+        while (tc > tc_min && layout(tc, tc - 2 * d.D).total > kSmemOneCta) tc -= kRoundFrames;
+        tc_max = tc; nout_max = tc - 2 * d.D;
     } else {
         // tile geometry (2 CTAs per SM): the cepstra tile holds up to 512 frames (<= 27 KB of shared memory)
         int tc = 512;
@@ -235,7 +247,7 @@ FusedEngine::FusedEngine(const Derived &dd, int dev) : d(dd), device(dev)
         tc_max = tc; nout_max = tc - 2 * d.D;
     }
     L = layout(tc_max, nout_max);
-    if (L.total > 227 * 1024) throw Error("fused kernel shared-memory budget exceeded");
+    if (L.total > kSmemOneCta) throw Error("fused kernel shared-memory budget exceeded");
     // phase-3 scratch of the default regression and the clustered scheme (k_fused_mfcc): row-group records at off_mags,
     // the tile's record at +25 KB, mean / scale at +30 KB, all below the cepstra
     const int rp = kMaxFusedThreads / d.cols;
@@ -253,7 +265,9 @@ void FusedEngine::set_window(const float *window, cudaStream_t st)
 void FusedEngine::ensure_mel(float alpha)
 {
     if (mc_alpha == alpha) return;
-    if (nc > 16) build_mel_const(d, alpha, mc_ceps);
+    if (d.N2 == 1024 && kf == 16) build_mel_const(d, alpha, mc_wide1024);
+    else if (d.N2 == 1024) build_mel_const(d, alpha, mc1024);
+    else if (nc > 16) build_mel_const(d, alpha, mc_ceps);
     else if (kf == 16) build_mel_const(d, alpha, mc_wide);
     else build_mel_const(d, alpha, mc);
     mc_alpha = alpha;
@@ -269,7 +283,7 @@ std::string FusedEngine::kernel_label() const
 
 int FusedEngine::latency_tile(int n_out) const
 {
-    const int target = std::max(1, 2 * sm_count);
+    const int target = std::max(1, ctas_per_sm * sm_count);
     const int want = (n_out + target - 1) / target;                          // rows per tile for ~2 tiles per SM
     const int rounds = std::max(2, (want + 2 * d.D + kRoundFrames - 1) / kRoundFrames);
     return std::max(1, std::min(nout_max, rounds * kRoundFrames - 2 * d.D));
@@ -374,7 +388,7 @@ void FusedEngine::launch_roles(FusedArgs a, int ntiles, FusedNormState &ns, cuda
     a.counters = ns.counters.p; a.work_counter = ns.counters.p + ns.counters.n - 1;
     a.flags = ns.flags.p; a.epoch = ++ns.epoch; a.ntiles_launch = ntiles;
     a.g_mean = ns.mean.p; a.g_scale = ns.scale.p;
-    launch(a, ntiles + std::min(ntiles, 2 * sm_count), 0, st);
+    launch(a, ntiles + std::min(ntiles, ctas_per_sm * sm_count), 0, st);
 }
 
 void FusedEngine::launch_clustered(FusedArgs a, int grid, int cluster, FusedNormState &ns, cudaStream_t st)
@@ -649,7 +663,7 @@ static int plan_impl(afe_batch *b, const int64_t *off, const int64_t *len, const
                 const int64_t T = std::max<int64_t>(0, (len[u] - (d.W - d.S)) / d.S);
                 total += T; longest = std::max(longest, T);
             }
-            const int slots = 2 * eng.sm_count;
+            const int slots = eng.ctas_per_sm * eng.sm_count;
             const int64_t tiles_default = (total + eng.nout_max - 1) / eng.nout_max;
             // only batches that hold a long utterance (more than 8 tiles: the role scheme anyway); batches of short
             // utterances keep the large tiles, whose 1..4-tile utterances normalise inside a thread-block cluster

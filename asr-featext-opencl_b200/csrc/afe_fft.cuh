@@ -1,13 +1,18 @@
-// In-register batched real FFT (256/512 point) + magnitude, replacing clfft.cpp / AppleFFT and mfcc.cl:kernelTranspose.
+// In-register batched real FFT (256/512/1024 point) + magnitude, replacing clfft.cpp / AppleFFT and mfcc.cl:kernelTranspose.
 //
 // An N2-point real frame is transformed as an M = N2/2 point complex FFT of z[n] = x[2n] + i*x[2n+1] (one 32-bit
 // shared-memory word holds both int16 samples), M = 16*R:
-//   R lanes cooperate on one frame (R = 16 for N2 = 512, R = 8 for N2 = 256), so a warp transforms 32/R frames at once.
+//   R lanes cooperate on one frame (R = 32 for N2 = 1024, 16 for 512, 8 for 256), so a warp transforms 32/R frames at once.
 //   stage A   lane n2 holds z[R*n1 + n2], n1 = 0..15, and runs a radix-16 butterfly (4x4) entirely in registers
 //   twiddle   * exp(-2 pi i n2 k1 / M) from per-lane registers
 //   exchange  one trip through a padded shared-memory tile S[k1][n2] (the only data exchange of the transform)
 //   stage B   R-point FFT over n2 (radix-16, or two radix-8) in registers -> Z[k1 + 16 k2]
 //   split     X[k], X[M-k] from Z[k] (own registers) and Z[M-k] (one warp shuffle from the mirror lane) -> |X| row
+// R = 32 (1024 points): the 32-point FFT over n2 = a + 16 b is split by decimation in frequency. Lane pairs (a, a + 16)
+// run the radix-2 butterfly over b BEFORE the exchange, after one swap of 8 values through __shfl_xor_sync(.., 16):
+// lanes with b = 1 load their odd-n1 window pairs negated, which rotates their stage-A outputs by 8 slots, so every lane
+// keeps the same slots (its own half of k1) and sends the same slots (the other half). The exchange tile then holds row
+// k1 + 16 d = 16 values over a, and stage B is one radix-16 per lane -> Z[lane + 32 c]: the split is the R = 16 one.
 // The index maps are modelled and checked against numpy.fft.rfft in tools/fft_model.py / tests/test_host_logic.py.
 // Reference semantics: fftwf r2c unnormalised (mfcccpu.cpp:114,189), v = sqrt(re^2+im^2)/N2 (mfcccpu.cpp:203).
 #pragma once
@@ -88,12 +93,13 @@ template <int O> __device__ __forceinline__ void fft8(float2 (&x)[16])
 __host__ __device__ constexpr int pos8(int k) { return 2 * (k % 4) + k / 4; }
 
 template <int N2> struct FftCfg {
-    static_assert(N2 == 512 || N2 == 256, "in-register FFT supports 256 and 512 points");
+    static_assert(N2 == 1024 || N2 == 512 || N2 == 256, "in-register FFT supports 256, 512 and 1024 points");
     static constexpr int M = N2 / 2;         // complex length
     static constexpr int R = M / 16;         // lanes per frame
     static constexpr int FPW = 32 / R;       // frames per warp
-    static constexpr int RS = R + 1;         // padded row stride of the exchange tile (float2 units)
-    static constexpr int SCR = 16 * RS + (R == 8 ? 1 : 0); // per-frame scratch (float2 units), >= M
+    // padded row stride of the exchange tile (float2 units): 16 rows of R values, or at 1024 points 32 rows of 16 values
+    static constexpr int RS = R == 32 ? 17 : R + 1;
+    static constexpr int SCR = R == 32 ? 32 * RS : 16 * RS + (R == 8 ? 1 : 0); // per-frame scratch (float2 units), >= M
     static constexpr int BINS = M + 1;
 };
 
@@ -129,10 +135,12 @@ template <int NZ> __device__ __forceinline__ void fft16_in(float2 (&x)[16])
 
 // Per-lane constants kept in registers for the whole kernel (shared memory bandwidth is the scarce resource here,
 // profiles/r01_v4b_8x4_k_fused_summary.txt): window pairs, exchange twiddles, split twiddles.
+// R = 32, lane = a + 16 b: b = 1 negates win[n1] for odd n1 and takes twa[j] for k1 = (j + 8) % 16; twb = (-1)^b W32^a.
 template <int N2, int NZ> struct LaneConsts {
     float2 win[NZ]; // (w[2n], w[2n+1]) for n = R*n1 + lane, n1 < NZ (zero beyond)
     float2 twa[16]; // exp(-2 pi i lane*k1 / M)
     float2 twp[8];  // exp(-2 pi i (lane + R*m) / N2)
+    float2 twb;     // R = 32 only: twiddle of the radix-2 difference
 };
 
 template <int N2, int NZ>
@@ -140,10 +148,23 @@ __device__ __forceinline__ void load_lane_consts(LaneConsts<N2, NZ> &lc, const f
                                                  const float2 *__restrict__ tw_a, const float2 *__restrict__ tw_p, int lf)
 {
     using C = FftCfg<N2>;
+    if (C::R == 32) {
+        const int b = lf >> 4;
 #pragma unroll
-    for (int n1 = 0; n1 < NZ; n1++) lc.win[n1] = window2[C::R * n1 + lf];
+        for (int n1 = 0; n1 < NZ; n1++) {
+            const float2 w = window2[C::R * n1 + lf];
+            lc.win[n1] = b && (n1 & 1) ? make_float2(-w.x, -w.y) : w;
+        }
 #pragma unroll
-    for (int k1 = 0; k1 < 16; k1++) lc.twa[k1] = tw_a[lf * 16 + k1];
+        for (int j = 0; j < 16; j++) lc.twa[j] = tw_a[lf * 16 + ((j + 8 * b) & 15)];
+        const float2 t = tw_a[(lf & 15) * 32 + 8]; // exp(-2 pi i 16 a / M) = W32^a
+        lc.twb = b ? make_float2(-t.x, -t.y) : t;
+    } else {
+#pragma unroll
+        for (int n1 = 0; n1 < NZ; n1++) lc.win[n1] = window2[C::R * n1 + lf];
+#pragma unroll
+        for (int k1 = 0; k1 < 16; k1++) lc.twa[k1] = tw_a[lf * 16 + k1];
+    }
 #pragma unroll
     for (int m = 0; m < 8; m++) lc.twp[m] = tw_p[lf + C::R * m];
 }
@@ -205,15 +226,31 @@ __device__ __forceinline__ void fft_frame_mag(const uint32_t *words, const LaneC
         }
     }
     fft16_in<NZ>(x);
-    // twiddle + exchange: S[k1][n2]
+    if (R == 32) {
+        // twiddle; keep slots j < 8 (k1 = 8 b + j), swap slots 8 + j with lane ^ 16; radix 2 over b -> S[k1 + 16 d][a]
+        float2 v[16];
 #pragma unroll
-    for (int k1 = 0; k1 < 16; k1++) {
-        float2 v = x[pos16(k1)];
-        if (k1 > 0) v = cmul(v, lc.twa[k1]);
-        scratch[k1 * RS + lf] = v;
+        for (int j = 0; j < 16; j++) v[j] = cmul(x[pos16(j)], lc.twa[j]);
+        float2 *row = scratch + (lf >> 4) * 8 * RS + (lf & 15);
+#pragma unroll
+        for (int j = 0; j < 8; j++) {
+            float2 got;
+            got.x = __shfl_xor_sync(0xffffffffu, v[8 + j].x, 16);
+            got.y = __shfl_xor_sync(0xffffffffu, v[8 + j].y, 16);
+            row[j * RS] = cadd(v[j], got);
+            row[(16 + j) * RS] = cmul(csub(v[j], got), lc.twb);
+        }
+    } else {
+        // twiddle + exchange: S[k1][n2]
+#pragma unroll
+        for (int k1 = 0; k1 < 16; k1++) {
+            float2 v = x[pos16(k1)];
+            if (k1 > 0) v = cmul(v, lc.twa[k1]);
+            scratch[k1 * RS + lf] = v;
+        }
     }
     __syncwarp();
-    if (R == 16) {
+    if (R >= 16) { // R = 32: row lf holds the 16 values over a
 #pragma unroll
         for (int n2 = 0; n2 < 16; n2++) x[n2] = scratch[lf * RS + n2];
         fft16(x);
@@ -229,7 +266,7 @@ __device__ __forceinline__ void fft_frame_mag(const uint32_t *words, const LaneC
     __syncwarp();
     // Real split without another trip through shared memory: lane lf finalises the bins k = lf + R*m, m = 0..7, and
     // their mirrors M-k. Z[k] is already in its registers; Z[M-k] lives in lane (R-lf)%R of the same frame:
-    //   R = 16: slot 15-m                          (lane 0 pairs with itself: Z[M-16m] = its own slot 16-m; Z[M] := Z[0])
+    //   R = 16, 32: slot 15-m                      (lane 0 pairs with itself: Z[M-Rm] = its own slot 16-m; Z[M] := Z[0])
     //   R =  8: the other 8-point group, slot 7-m/2 (lane 0: same group; group 0 pairs with slot 8-m/2)
     // so every lane sends 8 complex values through one shuffle each way.
     float2 za[8], zb[8];
@@ -237,7 +274,7 @@ __device__ __forceinline__ void fft_frame_mag(const uint32_t *words, const LaneC
 #pragma unroll
     for (int m = 0; m < 8; m++) {
         float2 own, send, self;
-        if (R == 16) {
+        if (R >= 16) {
             own = x[pos16(m)];
             send = x[pos16(15 - m)];
             self = m == 0 ? x[pos16(0)] : x[pos16(16 - m)];
@@ -268,7 +305,7 @@ __device__ __forceinline__ void fft_frame_mag(const uint32_t *words, const LaneC
         mr[-R * m] = SCALED ? v2 * scale : v2;
     }
     if (lf == 0) {
-        const float2 a = R == 16 ? x[pos16(8)] : x[pos8(4)]; // X[M/2] = conj(Z[M/2]): k1 = 0, k2 = M/32
+        const float2 a = R >= 16 ? x[pos16(8)] : x[pos8(4)]; // X[M/2] = conj(Z[M/2]): k1 = 0, k2 = M/32 (R = 32: c = 8)
         const float vm = mag_sqrt<FAST>(a.x * a.x + a.y * a.y);
         mag_out[M / 2] = SCALED ? vm * (1.0f / (float)N2) : vm + vm;
     }

@@ -2,15 +2,15 @@
 // -> feature rows (+ per-tile column statistics, + per-utterance normalisation): one HBM read of PCM and one HBM write
 // of features per frame.
 //
-// Work item = (utterance, tile of `nout` output frames). A CTA (8 warps, 2 CTAs per SM) computes the cepstra of its tile
+// Work item = (utterance, tile of `nout` output frames). A CTA (8 warps, 2 CTAs per SM; 1 at 1024 points) computes the cepstra of its tile
 // plus a halo of D = l1+l2 frames on each side (clamped at the utterance edges, where the reference replicates the edge
 // frame, mfcccpu.cpp:243-254) in rounds of 32 frames:
 //   stage 0  each warp stages the PCM of ITS 4 frames with one cp.async.bulk (TMA, SASS UBLKCP) into its own buffer,
 //            completion on its own mbarrier; the next round's copy is issued as soon as this round's FFTs are done
 //   phase 1  each warp: 4/FPW calls of the in-register FFT + magnitude (afe_fft.cuh, packed FP32) -> mags[32][260] (CTA
-//            shared). Frame f lives in row mag_row(f): the two adjacent frames of one call land 4 rows = 16 banks
-//            apart, and the 8 frames of a quarter warp occupy 8 consecutive rows, so phase 2's "lane = frame" 128-bit
-//            reads (row stride 65 chunks = 1 mod 8) are conflict free
+//            shared; [32][516] at 1024 points). Frame f lives in row mag_row(f): the two adjacent frames of one call land
+//            4 rows = 16 banks apart, and the 8 frames of a quarter warp occupy 8 consecutive rows, so phase 2's "lane =
+//            frame" 128-bit reads (row stride 65 or 129 chunks = 1 mod 8) are conflict free
 //   phase 2  mel + log + DCT, ONE THREAD PER FRAME, warp w owning the filters b = w (mod 8). The triangular weights and
 //            the DCT matrix are kernel parameters, i.e. constant-bank operands (LDCU.64 -> uniform-register operand of
 //            FFMA2): they cost no shared-memory bandwidth (v3/v4 re-loaded weights per lane: 116 of 245 smem wavefronts
@@ -51,19 +51,20 @@ constexpr int kTileQ1All = 2;   // every row of the tile takes its static D rows
 
 constexpr int kMaxBanks = 64;      // bank capacity of the instantiations with KF <= 8 (up to 64 banks)
 constexpr int kMaxBanksWide = 128; // bank capacity of the KF = 16 instantiations (65..128 banks)
-constexpr int kMagStride = 260; // floats per magnitude row (16-byte aligned rows)
+// floats per magnitude row (16-byte aligned rows, an odd number of 16-byte chunks): 257 bins up to 512 points, 513 at 1024
+__host__ __device__ constexpr int mag_stride(int n2) { return n2 == 1024 ? 516 : 260; }
 // row of frame f (0..31) of a round: pair k = f>>1 -> rows 8*(k>>2) + (k&3) and +4
 __host__ __device__ constexpr int mag_row(int f) { return 8 * (f >> 3) + ((f >> 1) & 3) + 4 * (f & 1); }
 
-// Mel / DCT tables for up to NB banks and NC DCT columns, passed BY VALUE as a kernel parameter (constant bank): indexed
-// with warp-uniform indices only, read with 128-bit constant loads. Weight lists are zero padded to a multiple of 4 bins;
-// DCT rows to NC columns. NB = 64: 7 KB; NB = 128: 16 KB; NB = 64 with NC = 48: 17 KB (the parameter list must stay
-// under 32 764 bytes, see below).
-template <int NB, int NC = 16>
+// Mel / DCT tables for up to NB banks, NC DCT columns and NBINS magnitude bins, passed BY VALUE as a kernel parameter
+// (constant bank): indexed with warp-uniform indices only, read with 128-bit constant loads. Weight lists are zero padded
+// to a multiple of 4 bins; DCT rows to NC columns. NB = 64: 7 KB; NB = 128: 16 KB; NB = 64 with NC = 48: 17 KB; 513 bins
+// (1024 points): 11 KB with NB = 64, 18 KB with NB = 128 (the parameter list must stay under 32 764 bytes, see below).
+template <int NB, int NC = 16, int NBINS = 257>
 struct MelConstT {
     static constexpr int kBanks = NB;
     static constexpr int kCols = NC;
-    static constexpr int kWl4 = (2 * 257 + 10 * NB + 3) / 4; // every bin feeds a rising and a falling side; lists start on
+    static constexpr int kWl4 = (2 * NBINS + 10 * NB + 3) / 4; // every bin feeds a rising and a falling side; lists start on
                                                               // a multiple of 4 bins and are padded to whole 8-bin chunks
     float4 wl4[kWl4];            // weights of filter b: 2*n8[b] float4 = bins 4*fchunk[b] + 8*i + {0..7}, i < n8[b]. The lists
                                  // of the filters of one warp class (b = w, w + 8, w + 16, ...) are CONTIGUOUS from
@@ -77,6 +78,11 @@ constexpr int kMaxCepsWide = 48; // DCT column capacity of the wide-DCT instanti
 using MelConst = MelConstT<kMaxBanks>;
 using MelConstWide = MelConstT<kMaxBanksWide>;
 using MelConstCeps = MelConstT<kMaxBanks, kMaxCepsWide>;
+using MelConst1024 = MelConstT<kMaxBanks, 16, 513>;
+using MelConstWide1024 = MelConstT<kMaxBanksWide, 16, 513>;
+// the constant-bank tables of k_fused_mfcc<N2, .., KF, .., NC>
+template <int N2, int KF, int NC>
+using MelConstFor = MelConstT<(KF <= 8 ? kMaxBanks : kMaxBanksWide), NC, (N2 == 1024 ? 513 : 257)>;
 
 struct FusedArgs {
     const int16_t *pcm;
@@ -132,16 +138,20 @@ struct FusedSmem {
         off_cep, total;
 };
 
-// CUDA 12.1+ accepts kernel parameter lists of up to 32 764 bytes; the widest ones are (FusedArgs, FusedSmem, MelConstWide)
-// and (FusedArgs, FusedSmem, MelConstCeps)
+// CUDA 12.1+ accepts kernel parameter lists of up to 32 764 bytes; the widest ones are (FusedArgs, FusedSmem, MelConstWide),
+// (FusedArgs, FusedSmem, MelConstCeps) and (FusedArgs, FusedSmem, MelConstWide1024)
 static_assert(sizeof(FusedArgs) + sizeof(FusedSmem) + sizeof(MelConstWide) + 16 <= 32764, "K1 kernel parameters too large");
 static_assert(sizeof(FusedArgs) + sizeof(FusedSmem) + sizeof(MelConstCeps) + 16 <= 32764, "K1 kernel parameters too large");
+static_assert(sizeof(FusedArgs) + sizeof(FusedSmem) + sizeof(MelConstWide1024) + 16 <= 32764, "K1 kernel parameters too large");
 
 inline int align_up(int v, int a) { return (v + a - 1) / a * a; }
 
 // dynamic shared memory of one CTA when 2 CTAs share an SM (sm_100: 228 KB per SM, 1 KB reserved per CTA, and the few
 // bytes of k_fused_mfcc's static shared variables)
 constexpr int kSmemTwoCtas = 113 * 1024 - 64;
+// the most dynamic shared memory one CTA may take: the 227 KB opt-in limit of a block holds dynamic AND static shared
+// memory, and k_fused_mfcc's static shared variables take 128 bytes (ptxas -v); 256 bytes are set aside for them
+constexpr int kSmemOneCta = 227 * 1024 - 256;
 
 template <int N2>
 FusedSmem fused_smem_layout(int kFusedWarps, int S, int cols, int tc_max, int nout_max, int l2, int nstreams)
@@ -151,7 +161,7 @@ FusedSmem fused_smem_layout(int kFusedWarps, int S, int cols, int tc_max, int no
     FusedSmem L;
     int o = 0;
     L.off_mbar = o; o += align_up(kFusedWarps * 8, 16);           // one mbarrier per warp, never aliased
-    L.off_mags = o; o += align_up((kRoundFrames * kMagStride + 16) * 4, 16); // [32][260] + pad for whole-chunk reads
+    L.off_mags = o; o += align_up((kRoundFrames * mag_stride(N2) + 16) * 4, 16); // [32][260 | 516] + pad for whole-chunk reads
     // per-warp staging [pcm]; then the FFT exchange tiles [scratch], which phase 2 reuses for the partial cepstra
     L.pcm_bytes = align_up(((kWarpFrames - 1) * S + N2) * 2, 16) + 16;
     L.w_pcm = 0;
@@ -570,13 +580,16 @@ __device__ __forceinline__ void normalise_role(const FusedArgs &a, const Tile tl
 // NC = DCT column capacity. NC = 16: every warp keeps the partial cepstra of its filter class, warps 0-3 sum them.
 // NC = 48 (ceps_len + c0 = 17..48, KF = 5 or 8): phase 2 writes log-mel values to a tile and, after barrier B, warps 0-3
 // compute the DCT split by column (12 each, lane = frame), in ascending bank order, straight into s_cep.
+// N2 = 1024: the 66 KB magnitude tile leaves room for one CTA per SM (DESIGN §4), which may use up to 255 registers.
 template <int N2, int NZ, int kFusedWarps, int KF, bool PRE, int NC = 16>
-__global__ void __launch_bounds__(32 * kFusedWarps, 2)
-k_fused_mfcc(const FusedArgs a, const FusedSmem L, const __grid_constant__ MelConstT<(KF <= 8 ? kMaxBanks : kMaxBanksWide), NC> mc)
+__global__ void __launch_bounds__(32 * kFusedWarps, N2 == 1024 ? 1 : 2)
+k_fused_mfcc(const FusedArgs a, const FusedSmem L, const __grid_constant__ MelConstFor<N2, KF, NC> mc)
 {
     constexpr bool FAST = false; // MUFU log approximation: measured in round 1, not shipped
     constexpr bool kWideDct = NC > 16;
     static_assert(!kWideDct || KF <= 8, "the wide DCT serves up to 64 banks");
+    static_assert(!kWideDct || N2 <= 512, "the wide DCT serves up to 512 points");
+    constexpr int kMagStride = mag_stride(N2);
     // warps of the wide DCT and columns per warp: with 4, warps 4-7 run ahead into the next round's FFTs (DESIGN §4)
     constexpr int kDctWarps = 4, kDctCols = NC / kDctWarps;
     using C = dev::FftCfg<N2>;

@@ -30,6 +30,8 @@ struct FusedEngine {
     MelConst mc;                 // up to 64 banks
     MelConstWide mc_wide;        // 65..128 banks (KF = 16)
     MelConstCeps mc_ceps;        // ceps_len + c0 = 17..48 (NC = 48, up to 64 banks)
+    MelConst1024 mc1024;         // 1024 points, up to 64 banks
+    MelConstWide1024 mc_wide1024; // 1024 points, 65..128 banks
     float mc_alpha = -1.f;
     bool pruned = false;         // zero-padded window tail: the first FFT layer is pruned (NZ = 13)
     bool window_set = false;
@@ -38,6 +40,7 @@ struct FusedEngine {
     int tc_max = 0, nout_max = 0;
     int kf = 0;                  // filters per warp of the instantiation: 3, 5, 8 or 16
     int nc = 16;                 // DCT column capacity of the instantiation: 16 or 48
+    int ctas_per_sm = 2;         // resident CTAs per SM the tile planning counts on: 1 at 1024 points (DESIGN §4)
 
     explicit FusedEngine(const Derived &dd, int dev);
 
@@ -46,6 +49,7 @@ struct FusedEngine {
     int launch_key() const { return fused_key(d.N2, pruned ? 13 : 16, kf, pre != 0.f, nc); }
     const void *mel_const() const
     {
+        if (d.N2 == 1024) return kf == 16 ? (const void *)&mc_wide1024 : (const void *)&mc1024;
         return nc > 16 ? (const void *)&mc_ceps : kf == 16 ? (const void *)&mc_wide : (const void *)&mc;
     }
     // the instantiation that runs, e.g. "k_fused_mfcc<512,13,8,5,false>" or, with NC = 48, "k_fused_mfcc<512,13,8,5,false,48>"

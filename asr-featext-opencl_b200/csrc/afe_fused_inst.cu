@@ -1,11 +1,11 @@
-// One instantiation of the fused kernel per translation unit: nvcc -DAFE_INST_KEY=<0..47> (see the Makefile).
+// One instantiation of the fused kernel per translation unit: nvcc -DAFE_INST_KEY=<0..63> (see the Makefile).
 #include <atomic>
 
 #include "afe_internal.h"
 #include "afe_fused_launch.h"
 
 #ifndef AFE_INST_KEY
-#error "compile with -DAFE_INST_KEY=0..47"
+#error "compile with -DAFE_INST_KEY=0..63"
 #endif
 
 namespace afe {
@@ -17,7 +17,7 @@ constexpr int kNZ = fused_key_nz(AFE_INST_KEY);
 constexpr int kKF = fused_key_kf(AFE_INST_KEY);
 constexpr int kNC = fused_key_nc(AFE_INST_KEY);
 static_assert(fused_key(kN2, kNZ, kKF, kPre, kNC) == AFE_INST_KEY, "key encoding and decoding disagree");
-using Mel = MelConstT<(kKF <= 8 ? kMaxBanks : kMaxBanksWide), kNC>;
+using Mel = MelConstFor<kN2, kKF, kNC>;
 
 void fill(cudaLaunchConfig_t &cfg, cudaLaunchAttribute &attr, const FusedLaunch &fl)
 {

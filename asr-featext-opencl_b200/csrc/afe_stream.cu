@@ -179,7 +179,8 @@ int afe_mfcc_create(const afe_params *p, int cuda_device, afe_mfcc **out)
         const size_t fc = d.frame_cap;
         // K1 covers the block when the parameter set fits it and normalisation (if any) comes after the deltas: normalising
         // BEFORE them takes statistics over the look-ahead rows of the block as well (mfcccpu.cpp:383-384), which no tile owns
-        const bool fused = fused_unsupported_reason(d).empty() && (d.p.norm == AFE_NORM_NONE || d.p.norm_after_dyn);
+        // (1024-point FFTs stay on the staged kernels here: K1 serves them in the batch extractor only)
+        const bool fused = fused_unsupported_reason(d).empty() && d.N2 <= 512 && (d.p.norm == AFE_NORM_NONE || d.p.norm_after_dyn);
         if (fused) {
             h->eng.reset(new FusedEngine(d, cuda_device));
             h->tiles_cap = fc / 32 + 2 * (size_t)h->eng->sm_count + 8;

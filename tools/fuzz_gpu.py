@@ -18,15 +18,19 @@ from common import afe, compare, run_batch, synth_utterances, to_afe_params  # n
 
 
 def random_params(rng):
-    sr = float(rng.choice([8000.0, 16000.0]))
+    sr = float(rng.choice([8000.0, 16000.0, 16000.0, 22050.0, 24000.0, 32000.0]))
     W = int(rng.choice([200, 256, 320, 400, 401, 480, 512, 150, 130]))
     if sr == 8000.0:
         W = min(W, 256) if rng.random() < 0.7 else W
+    if sr > 16000.0:  # 1024-point FFTs: 25 ms windows and the 1024 / 256 TTS shape
+        W = int(rng.choice([513, 551, 600, 800, 832, 833, 1000, 1024]))
     S = int(rng.integers(max(2, W // 5), W // 2 + 1))
     if rng.random() < 0.85:
         S -= S % 2
     nb = int(rng.choice([8, 12, 20, 23, 24, 26, 32, 40, 41, 48, 64, 72, 80, 96, 128]))
     ceps = int(rng.choice([0, 8, 12, 12, 12, 13, 15, 16, 19, 23, 29, 39, 40, 47]))
+    if W > 512:
+        ceps = min(ceps, 15)  # the batch extractor serves up to 16 columns at 1024 points
     c0 = int(rng.integers(0, 2))
     dyn = int(rng.integers(0, 3))
     cols = ceps + c0 if ceps > 0 else nb
